@@ -51,7 +51,15 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="skip the ragged-page and sustained-clock extras")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-op-profile", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed train step hands its caller (loss statistics, updated parameters, "
+                         "their gradients) to DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs is not None and (args.impl != "ours" or args.mode != "train"):
+        ap.error("--dump-outputs applies to the train step of --impl ours")
+    return args
 
 
 def peaks():
@@ -355,6 +363,30 @@ def workload_config(args, world):
     }
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def step_outputs(trainer, model):
+    """Host copies of what a caller holds after a train step: [sum w*nll, sum w, #correct], every updated parameter and
+    its gradient (the model is 105957 fp32 values, so everything is stored in full)."""
+    out = {"stats": trainer.step_stats().cpu().numpy()}
+    for name, p in model.named_parameters():
+        out["param." + name] = p.detach().cpu().numpy()
+        out["grad." + name] = p.grad.detach().cpu().numpy()
+    return out
+
+
+def write_outputs(dirname, outputs):
+    import numpy as np
+
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte dump limit")
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 # ------------------------------------------------------------- our arm -----
 def run_ours(args):
     import numpy as np
@@ -477,6 +509,8 @@ def run_ours(args):
 
     with ClockSampler(local) as clk:
         ms_res, _ = timed(resident, args.steps, args.warmup)
+        # the legs below keep training the same model: take the headline leg's results before they do
+        outputs = step_outputs(trainer, model) if args.dump_outputs and rank == 0 else None
         ms_e2e, wall_e2e = timed(e2e, args.steps, max(3, args.warmup // 2))
     loss = float(stats_host[0] / stats_host[1])
     hb = host_batches[0]
@@ -593,6 +627,8 @@ def run_ours(args):
             "cpu_baseline": cpu, "ops": ops_table, "loss": loss, "nodes_per_step_per_gpu": n_nodes,
             "edges_per_step_per_gpu": n_edges, "lib": os.path.relpath(gte.LIB_PATH, ROOT), "extras": extras,
         }
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -699,7 +735,7 @@ def run_infer(args):
     for _ in range(nw):
         pass_e2e()
     launches_per_pass = (lib.gte_launch_count() - c0) // nw
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     with ClockSampler(local) as clk:
         ms_e2e, wall_e2e = timed_passes(pass_e2e, steps)
         # resident leg: both static input sets hold a batch (the e2e leg left two of them there)

@@ -144,3 +144,31 @@ def test_bench_reference_arm_prints_the_contract_line():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2")
     out2 = subprocess.run(cmd, capture_output=True, text=True, timeout=300, cwd=root, env=env)
     assert out2.returncode == 0 and not [l for l in out2.stdout.splitlines() if l.startswith("{")]
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_are_reproducible_and_follow_steps(tmp_path):
+    """`bench.py --dump-outputs DIR`: the same arguments write the same arrays; one more timed step changes them"""
+    import json
+    import subprocess
+    import sys
+
+    def run(steps, tag):
+        d = tmp_path / tag
+        cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", "1",
+               "--pages", "8", "--no-extras", "--no-cpu-baseline", "--no-op-profile", "--dump-outputs", str(d)]
+        out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+        assert line["steps"] == steps
+        return {f.name: np.load(f) for f in sorted(d.iterdir())}
+
+    a, b, c = run(2, "a"), run(2, "b"), run(3, "c")
+    m = gte.GcnSAGE(13, 218, 9, 3, F.relu, 0)
+    names = {"stats.npy"} | {f"{kind}.{k}.npy" for kind in ("param", "grad") for k, _ in m.named_parameters()}
+    assert set(a) == set(b) == set(c) == names
+    for k in names:
+        assert a[k].dtype == np.float32 and np.isfinite(a[k]).all()
+        assert np.array_equal(a[k], b[k]), k
+    assert a["stats.npy"][1] == 8 * 300  # sum of the label weights: one per node
+    assert not np.array_equal(a["param.layers.0.linear.weight.npy"], c["param.layers.0.linear.weight.npy"])
