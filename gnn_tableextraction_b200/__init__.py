@@ -5,6 +5,7 @@ Public surface (mirrors /root/reference/src/components/graphs/models.py):
     GcnSAGELayer, GcnSAGE, WeightedMeanSAGELayer, MeanSAGE   -- drop-in nn.Modules
     PageGraphBatch, as_page_graph_batch                      -- the graph argument
     SageTrainer                                              -- fused train / inference step
+    BatchCapacity                                            -- largest batch a capacity-captured step accepts
     features.bbox_features                                   -- the 13 BBOX node features on the device
     CrossEntropyLoss, cross_entropy                          -- loss on the CUDA kernels
     ops                                                      -- tensor-level wrappers of include/gte.h
@@ -17,10 +18,10 @@ from ._lib import GteError, LIB_PATH, lib  # noqa: F401
 from .graph import PageGraphBatch, as_page_graph_batch, batch_pages_host  # noqa: F401
 from .nn import CrossEntropyLoss, GcnSAGE, GcnSAGELayer, MeanSAGE, WeightedMeanSAGELayer  # noqa: F401
 from .layers import cross_entropy  # noqa: F401
-from .engine import SageTrainer  # noqa: F401
+from .engine import BatchCapacity, SageTrainer  # noqa: F401
 from . import features, ops, synth  # noqa: F401
 
 __all__ = [
     "GcnSAGELayer", "GcnSAGE", "WeightedMeanSAGELayer", "MeanSAGE", "CrossEntropyLoss", "cross_entropy",
-    "PageGraphBatch", "as_page_graph_batch", "batch_pages_host", "SageTrainer", "ops", "synth", "GteError", "lib",
+    "PageGraphBatch", "as_page_graph_batch", "batch_pages_host", "SageTrainer", "BatchCapacity", "ops", "synth", "GteError", "lib",
 ]

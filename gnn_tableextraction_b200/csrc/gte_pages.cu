@@ -335,3 +335,84 @@ extern "C" int gte_build_page_formats(const int32_t* src, const int32_t* dst, co
   GTE_CHECK_LAUNCH("k_build_page_formats");
   return GTE_OK;
 }
+
+// ---------------------------------------------------------------------------------------------------
+// Padding of a page batch to a fixed capacity shape, on the device (the first kernel of a capacity-captured step).
+// The reference trains on shuffled batches of real pages whose node / edge totals change every step
+// (/root/reference/src/models/model_train.py:283-297) and predicts on streams ending with a short batch
+// (model_predict.py:130-154); a CUDA graph needs one shape.  The host copies only the real prefix (n nodes, e edges,
+// P pages) into buffers sized [n_cap] / [e_cap]; this kernel turns the tail into padding that is itself a legal
+// dgl.batch, so every later kernel runs on it unchanged:
+//   feat[n, n_cap) = 0, label[n, n_cap) = -1 (weight 0 in the loss, never counted correct),
+//   edges [e, e_cap): weight 0, src = dst = a padding node of the page that owns the edge (a self-loop).
+// The page table is written by the HOST: page_off / edge_off hold all p_cap + 1 entries (real pages, then padding
+// pages of at most the capacity's page sizes, then empty pages), so this kernel only reads it to find the page of a
+// padding edge (binary search over edge_off).  `word` = (n, e, P) of the batch, copied with it.  The grid is fixed by
+// the capacity; grid-stride loops are bounded by the counts read from `word`.  A word outside the capacity, or a
+// page table that gives a padding edge no padding node, raises *bad (1 / 2); the kernel then clamps, so it never
+// writes outside [0, n_cap) rows / [0, e_cap) edges (an out-of-page self-loop is left for gte_build_page_formats to
+// report).
+namespace gte {
+
+constexpr int PAD_THREADS = 256;
+
+__global__ void __launch_bounds__(PAD_THREADS)
+    k_pad_batch(const int32_t* __restrict__ word, int32_t n_cap, int32_t e_cap, int32_t p_cap,
+                const int32_t* __restrict__ page_off, const int32_t* __restrict__ edge_off, int32_t* __restrict__ src,
+                int32_t* __restrict__ dst, float* __restrict__ w, float* __restrict__ feat, int64_t ldf, int32_t f,
+                float* __restrict__ label, int* __restrict__ bad) {
+  int32_t n = word[0], e = word[1];
+  const int32_t p = word[2];
+  if (n < 0 || n > n_cap || e < 0 || e > e_cap || p < 0 || p > p_cap) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) atomicOr(bad, 1);
+    n = min(max(n, 0), n_cap);
+    e = min(max(e, 0), e_cap);
+  }
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  const int64_t t0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t nf = (int64_t)(n_cap - n) * f;
+  for (int64_t k = t0; k < nf; k += stride) feat[(n + k / f) * ldf + k % f] = 0.0f;
+  for (int64_t i = n + t0; i < n_cap; i += stride) label[i] = -1.0f;
+  for (int64_t i = e + t0; i < e_cap; i += stride) {
+    // page of edge i: the last page whose first edge is <= i
+    int32_t lo = 0, hi = p_cap - 1;
+    while (lo < hi) {
+      const int32_t mid = (lo + hi + 1) >> 1;
+      if (edge_off[mid] <= i) lo = mid; else hi = mid - 1;
+    }
+    const int32_t n0 = page_off[lo], cnt = page_off[lo + 1] - n0;
+    const int64_t j = i - edge_off[lo];
+    int32_t v;
+    if (cnt > 0 && n0 >= n && n0 + cnt <= n_cap && j >= 0) {
+      v = n0 + (int32_t)(j % cnt);
+    } else {
+      atomicOr(bad, 2);
+      v = n_cap - 1;
+    }
+    src[i] = v;
+    dst[i] = v;
+    w[i] = 0.0f;
+  }
+}
+
+}  // namespace gte
+
+extern "C" int gte_pad_batch(const int32_t* word, int32_t n_cap, int64_t e_cap, int32_t p_cap, const int32_t* page_off,
+                             const int32_t* edge_off, int32_t* src, int32_t* dst, float* weight, float* feat, int64_t ldf,
+                             int32_t f, float* label, int32_t* bad, gte_stream_t stream) {
+  GTE_CHECK_ARG(n_cap > 0 && e_cap >= 0 && e_cap < ((int64_t)1 << 31) && p_cap > 0 && f > 0 && ldf >= f,
+                "gte_pad_batch: bad capacity");
+  GTE_CHECK_ARG(word && page_off && edge_off && feat && label && bad, "gte_pad_batch: null argument");
+  GTE_CHECK_ARG(e_cap == 0 || (src && dst && weight), "gte_pad_batch: null edge argument");
+  cudaStream_t st = as_stream(stream);
+  GTE_CHECK_CUDA(cudaMemsetAsync(bad, 0, 4, st), "gte_pad_batch(memset bad)");
+  const int64_t work = (int64_t)n_cap * f > e_cap ? (int64_t)n_cap * f : e_cap;
+  const int64_t cap_blocks = 4 * (int64_t)sm_count();
+  int64_t blocks = ceil_div64(work, PAD_THREADS);
+  if (blocks > cap_blocks) blocks = cap_blocks;
+  if (blocks < 1) blocks = 1;
+  k_pad_batch<<<(unsigned)blocks, PAD_THREADS, 0, st>>>(word, n_cap, (int32_t)e_cap, p_cap, page_off, edge_off, src, dst, weight,
+                                              feat, ldf, f, label, bad);
+  GTE_CHECK_LAUNCH("k_pad_batch");
+  return GTE_OK;
+}

@@ -11,8 +11,9 @@ Restates the train-step envelope of the reference
                                                              one flat gradient buffer, one
                                                              (optional) all-reduce, fused Adam
 
-without autograd bookkeeping, without the per-step ``.item()`` sync, and -- for
-fixed-shape batches -- replayed from a CUDA graph.  Data parallel by graph
+without autograd bookkeeping, without the per-step ``.item()`` sync, and replayed
+from a CUDA graph -- for fixed-shape batches, or for every batch up to a
+``BatchCapacity`` (padded on the device inside the graph).  Data parallel by graph
 (pages are independent): every rank runs the same step on its own pages; the
 loss statistics ride in the tail of the flat gradient buffer, so ONE SUM
 all-reduce per step carries gradients and statistics; Adam divides by the
@@ -22,8 +23,10 @@ of per-rank means).
 from __future__ import annotations
 
 import os
-from typing import Dict, List, Optional
+from dataclasses import dataclass
+from typing import Dict, List, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 import torch.nn as nn
 
@@ -37,6 +40,98 @@ from .nn import GcnSAGE, _is_relu
 def _dropout_p(d) -> float:
     """dropout attribute of the reference modules: nn.Dropout or the float 0. (models.py:30-33)"""
     return float(d.p) if isinstance(d, nn.Dropout) else float(d or 0.0)
+
+
+@dataclass(frozen=True)
+class BatchCapacity:
+    """The largest page batch a capacity-captured step accepts: total nodes, total edges, page count, and the largest
+    page in nodes and in edges.  The reference batches shuffled real pages (model_train.py:283-297) and streams pages
+    for prediction (model_predict.py:130-154), so the totals change from batch to batch; a step captured for a
+    capacity replays one CUDA graph for every batch that fits, padded on the device to the shape ``shape``."""
+
+    nodes: int
+    edges: int
+    pages: int
+    page_nodes: int
+    page_edges: int
+
+    def __post_init__(self):
+        for k in ("nodes", "edges", "pages", "page_nodes", "page_edges"):
+            v = getattr(self, k)
+            if not isinstance(v, (int, np.integer)) or isinstance(v, bool):
+                raise GteError(f"BatchCapacity: {k} must be an int, got {v!r}")
+            object.__setattr__(self, k, int(v))
+        if self.nodes < 1 or self.pages < 1 or self.edges < 0 or self.page_edges < 1:
+            raise GteError(f"BatchCapacity: need nodes >= 1, pages >= 1, edges >= 0, page_edges >= 1 (got {self})")
+        if self.page_nodes < 2:  # every padding page needs room for more than one node (see shape)
+            raise GteError(f"BatchCapacity: page_nodes={self.page_nodes} < 2")
+        if self.page_nodes > PAGE_NODES_MAX:
+            raise GteError(f"BatchCapacity: page_nodes={self.page_nodes} > {PAGE_NODES_MAX}, the largest page the page "
+                           "kernels stage")
+        n_cap, e_cap, _ = self.shape
+        if e_cap >= 2 ** 31 or n_cap >= 2 ** 31:
+            raise GteError(f"BatchCapacity: {n_cap} nodes / {e_cap} edges after padding exceed int32 ids")
+
+    @property
+    def shape(self) -> Tuple[int, int, int]:
+        """(N_cap, E_cap, P_cap) of the captured batch.  K = max(ceil(nodes / (page_nodes - 1)), ceil(edges /
+        page_edges)) padding slots: any fitting batch leaves at least K free page slots and K padding nodes, and
+        K slots carry all padding nodes and edges without exceeding the page caps."""
+        k = max(-(-self.nodes // (self.page_nodes - 1)), -(-self.edges // self.page_edges))
+        return self.nodes + k, self.edges, self.pages + k
+
+    def check(self, batch_num_nodes: Sequence[int], batch_num_edges: Sequence[int]) -> None:
+        """Raise a GteError naming the limit a batch with these page sizes breaks."""
+        bn, be = list(batch_num_nodes), list(batch_num_edges)
+        if len(bn) != len(be):
+            raise GteError(f"batch: {len(bn)} page node counts but {len(be)} page edge counts")
+        if not bn:
+            raise GteError("batch: no pages")
+        if min(bn) < 0 or min(be) < 0:
+            raise GteError("batch: negative page size")
+        pre = "batch does not fit the captured capacity:"
+        if len(bn) > self.pages:
+            raise GteError(f"{pre} {len(bn)} pages > pages={self.pages}")
+        if sum(bn) > self.nodes:
+            raise GteError(f"{pre} {sum(bn)} nodes > nodes={self.nodes}")
+        if sum(be) > self.edges:
+            raise GteError(f"{pre} {sum(be)} edges > edges={self.edges}")
+        if max(bn) > self.page_nodes:
+            raise GteError(f"{pre} a page of {max(bn)} nodes > page_nodes={self.page_nodes}")
+        if max(be) > self.page_edges:
+            raise GteError(f"{pre} a page of {max(be)} edges > page_edges={self.page_edges}")
+
+    def fits(self, batch_num_nodes: Sequence[int], batch_num_edges: Sequence[int]) -> bool:
+        try:
+            self.check(batch_num_nodes, batch_num_edges)
+        except GteError:
+            return False
+        return True
+
+
+PAGE_NODES_MAX = 1600  # graph.page_table: larger pages get no page table (generic kernels)
+
+
+def padded_page_table(capacity: BatchCapacity, batch_num_nodes: Sequence[int], batch_num_edges: Sequence[int]):
+    """Page table (node offsets, edge offsets: int32 [P_cap + 1] each) of a batch padded to ``capacity.shape``: the
+    real pages as given, then s = min(P_cap - P, N_cap - n) padding pages sharing the N_cap - n padding nodes and the
+    E_cap - e padding edges evenly (each gets at least one node and at most page_nodes / page_edges), then empty
+    pages.  gte_pad_batch makes every padding edge a weight-0 self-loop on a node of its own padding page."""
+    capacity.check(batch_num_nodes, batch_num_edges)
+    n_cap, e_cap, p_cap = capacity.shape
+    bn = np.asarray(list(batch_num_nodes), dtype=np.int64)
+    be = np.asarray(list(batch_num_edges), dtype=np.int64)
+    p, n, e = len(bn), int(bn.sum()), int(be.sum())
+    s = min(p_cap - p, n_cap - n)  # >= K >= 1
+    j = np.arange(1, s + 1, dtype=np.int64)
+    po = np.full(p_cap + 1, n_cap, dtype=np.int64)
+    eo = np.full(p_cap + 1, e_cap, dtype=np.int64)
+    po[0] = eo[0] = 0
+    np.cumsum(bn, out=po[1:p + 1])
+    np.cumsum(be, out=eo[1:p + 1])
+    po[p + 1:p + 1 + s] = n + j * (n_cap - n) // s
+    eo[p + 1:p + 1 + s] = e + j * (e_cap - e) // s
+    return po.astype(np.int32), eo.astype(np.int32)
 
 
 class SageTrainer:
@@ -112,6 +207,7 @@ class SageTrainer:
                                             group=self.pg)
         self._graph = None
         self._static: Optional[Dict[str, torch.Tensor]] = None
+        self._capacity: Optional[BatchCapacity] = None
 
     # ----------------------------------------------------------- pieces ----
     def _layer_args(self, layer):
@@ -300,46 +396,69 @@ class SageTrainer:
         return preds, acc
 
     # ----------------------------------------------------- CUDA graphs -----
-    def capture_predict(self, host_batch: Dict[str, torch.Tensor]):
+    def capture_predict(self, host_batch: Dict[str, torch.Tensor], capacity: Optional[BatchCapacity] = None):
         """Capture the batched predict pass of model_predict.py:130-154 (format build + forward without saved
-        activations + argmax + per-page correct counts) for batches of this shape.  Feed batches with ``load_batch`` /
-        ``prefetch_batch``; ``replay()`` / ``replay_prefetched()`` then return ``(preds int32 [N], page_correct int32 [P])``
-        -- static device tensors of the input set that ran, valid until that set runs again."""
-        return self.capture(host_batch, split=False, mode="predict")
+        activations + argmax + per-page correct counts) for batches of this shape, or for every batch that fits
+        ``capacity`` (see ``capture``).  Feed batches with ``load_batch`` / ``prefetch_batch``; ``replay()`` /
+        ``replay_prefetched()`` then return ``(preds int32 [N], page_correct int32 [P])`` -- views of static device
+        tensors of the input set that ran, sized for the batch in it, valid until that set runs again."""
+        return self.capture(host_batch, capacity=capacity, split=False, mode="predict")
 
-    def capture(self, host_batch: Dict[str, torch.Tensor], split: Optional[bool] = None, mode: str = "train"):
+    def capture(self, host_batch: Dict[str, torch.Tensor], capacity: Optional[BatchCapacity] = None,
+                split: Optional[bool] = None, mode: str = "train"):
         """Capture the whole step (format build + forward + loss + backward +
         optimiser) for batches with exactly this node / edge count.  Later
         batches are fed with ``load_batch`` + ``replay``.  ``split`` (default: data-parallel
-        runs) captures the kernels in one graph and leaves the all-reduce and Adam outside it."""
+        runs) captures the kernels in one graph and leaves the all-reduce and Adam outside it.
+
+        ``capacity``: capture once for every batch that fits it (``fits()``), e.g. the shuffled batches of real pages
+        of model_train.py:283-297.  The static inputs have the capacity's padded shape; a batch is copied as it is and
+        ``gte_pad_batch``, the first kernel of the graph, pads it on the device with zero-feature, label -1 nodes and
+        weight-0 self-loops in pages of their own, which change no loss statistic and no gradient.  ``host_batch``
+        must fit; it gives the feature width and the warm-up contents."""
         if split is None:
             split = self.world > 1 and self._dp_peer is None  # the peer-memory exchange is an ordinary kernel: one graph
         if mode not in ("train", "predict"):
             raise GteError(f"capture: unknown mode {mode}")
+        if capacity is not None:
+            self._check_capacity(capacity, host_batch)
         self._mode = mode
+        self._capacity = capacity
         dev = self.device
-        n, e = int(host_batch["num_nodes"]), int(host_batch["src"].numel())
-        f = int(host_batch["feat"].shape[1])
-        st = {
-            "src": torch.empty(e, dtype=torch.int32, device=dev),
-            "dst": torch.empty(e, dtype=torch.int32, device=dev),
-            "weight": torch.empty(e, dtype=torch.float32, device=dev),
-            "feat": torch.empty((n, f), dtype=torch.float32, device=dev),
-            "label": torch.empty(n, dtype=torch.float32, device=dev),
-        }
-        self._static = st
-        bn, be = list(host_batch["batch_num_nodes"]), list(host_batch["batch_num_edges"])
-        self._static_meta = (n, e, bn, be)
-        # The page table (node / edge offsets of the pages) is part of the INPUT: a later batch with the same totals
-        # may order or size its pages differently, so every static input set owns device copies of the two offset
-        # arrays and load_batch / prefetch_batch refresh them.  Only the maxima (shared-memory sizing of the page
-        # kernels) and the page count are fixed at capture time.
-        pages = page_table(bn, be, n, dev)
-        if pages is not None:
-            st["page_off"], st["edge_off"] = pages[0], pages[4]
-            self._static_caps = (pages[1], pages[2], pages[3])  # page count, max page nodes, max page edges
+        if capacity is None:
+            n, e = int(host_batch["num_nodes"]), int(host_batch["src"].numel())
+            f = int(host_batch["feat"].shape[1])
+            st = {
+                "src": torch.empty(e, dtype=torch.int32, device=dev),
+                "dst": torch.empty(e, dtype=torch.int32, device=dev),
+                "weight": torch.empty(e, dtype=torch.float32, device=dev),
+                "feat": torch.empty((n, f), dtype=torch.float32, device=dev),
+                "label": torch.empty(n, dtype=torch.float32, device=dev),
+            }
+            self._static = st
+            bn, be = list(host_batch["batch_num_nodes"]), list(host_batch["batch_num_edges"])
+            self._static_meta = (n, e, bn, be)
+            # The page table (node / edge offsets of the pages) is part of the INPUT: a later batch with the same totals
+            # may order or size its pages differently, so every static input set owns device copies of the two offset
+            # arrays and load_batch / prefetch_batch refresh them.  Only the maxima (shared-memory sizing of the page
+            # kernels) and the page count are fixed at capture time.
+            pages = page_table(bn, be, n, dev)
+            if pages is not None:
+                st["page_off"], st["edge_off"] = pages[0], pages[4]
+                self._static_caps = (pages[1], pages[2], pages[3])  # page count, max page nodes, max page edges
+            else:
+                self._static_caps = None
         else:
-            self._static_caps = None
+            n_cap, e_cap, p_cap = capacity.shape
+            self._feat_width = int(host_batch["feat"].shape[1])
+            st = self._capacity_set()
+            self._static = st
+            # the structure the captured kernels see: P_cap pages, none larger than the capacity's page caps (the
+            # page lists only size the batch; the offsets come from st["page_off"] / st["edge_off"] every replay)
+            po, eo = padded_page_table(capacity, host_batch["batch_num_nodes"], host_batch["batch_num_edges"])
+            self._static_meta = (n_cap, e_cap, np.diff(po).tolist(), np.diff(eo).tolist())
+            self._static_caps = (p_cap, capacity.page_nodes, capacity.page_edges)
+            self._set_rows = [None, None]  # (n, P) of the batch in each input set: predict outputs are cut to it
         self._loaded_layout = [None, None]
         self.load_batch(host_batch)
 
@@ -350,6 +469,7 @@ class SageTrainer:
         s.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(s):
             for _ in range(2):
+                self._pad(st)
                 if mode == "train":
                     self._step_impl(self._static_graph(st), st["label"])
                 else:
@@ -381,10 +501,73 @@ class SageTrainer:
         g = self._static_graph(st)
         if g.prepare(st["weight"]):
             g.check_page_structure()
+        if "pad_bad" in st and int(st["pad_bad"].item()) != 0:
+            raise GteError("capture: gte_pad_batch flagged the padded batch (word outside the capacity or bad page table)")
+
+    # -- capacity capture: one graph for every batch that fits a BatchCapacity ------------------------------------
+    def _check_capacity(self, capacity: BatchCapacity, host_batch):
+        if not isinstance(capacity, BatchCapacity):
+            raise GteError(f"capture: capacity must be a BatchCapacity, got {type(capacity).__name__}")
+        _, _, p_cap = capacity.shape
+        if not ops.page_formats_supported((None, p_cap, capacity.page_nodes, capacity.page_edges)):
+            raise GteError(f"capture: pages of {capacity.page_nodes} nodes / {capacity.page_edges} edges do not fit the "
+                           "one-kernel batch assembly (shared memory); lower page_nodes / page_edges")
+        self._check_fit(capacity, host_batch, int(host_batch["feat"].shape[1]))
+
+    @staticmethod
+    def _check_fit(capacity: BatchCapacity, host_batch, f: int):
+        bn, be = list(host_batch["batch_num_nodes"]), list(host_batch["batch_num_edges"])
+        capacity.check(bn, be)
+        n, e = int(host_batch["num_nodes"]), int(host_batch["src"].numel())
+        if sum(bn) != n or sum(be) != e:
+            raise GteError("captured step: page sizes do not add up to the batch's node / edge totals")
+        feat = host_batch["feat"]
+        if feat.dim() != 2 or int(feat.shape[0]) != n or int(feat.shape[1]) != f:
+            raise GteError(f"captured step: features {tuple(feat.shape)}, expected [{n}, {f}]")
+        if host_batch["label"].numel() != n or host_batch["dst"].numel() != e or host_batch["weight"].numel() != e:
+            raise GteError("captured step: label / dst / weight sizes do not match the batch totals")
+
+    def _capacity_set(self) -> Dict[str, torch.Tensor]:
+        """One static input set of the capacity shape.  ``meta`` = [n, e, P, 0 | page_off (P_cap + 1) | edge_off
+        (P_cap + 1)] travels in ONE copy; ``word``, ``page_off`` and ``edge_off`` are views of it."""
+        dev = self.device
+        n_cap, e_cap, p_cap = self._capacity.shape
+        meta = torch.zeros(4 + 2 * (p_cap + 1), dtype=torch.int32, device=dev)
+        return {
+            "src": torch.zeros(e_cap, dtype=torch.int32, device=dev),
+            "dst": torch.zeros(e_cap, dtype=torch.int32, device=dev),
+            "weight": torch.zeros(e_cap, dtype=torch.float32, device=dev),
+            "feat": torch.zeros((n_cap, self._feat_width), dtype=torch.float32, device=dev),
+            "label": torch.zeros(n_cap, dtype=torch.float32, device=dev),
+            "meta": meta, "word": meta[:4], "page_off": meta[4:5 + p_cap], "edge_off": meta[5 + p_cap:],
+            "pad_bad": torch.zeros(1, dtype=torch.int32, device=dev),
+        }
+
+    def _pad(self, st):
+        """first kernel of a capacity-captured step: pad the batch in ``st`` to the capacity shape"""
+        if self._capacity is not None:
+            ops.pad_batch(st["word"], st["page_off"], st["edge_off"], st["src"], st["dst"], st["weight"], st["feat"],
+                          st["label"], bad=st["pad_bad"])
+
+    def fits(self, host_batch: Dict[str, torch.Tensor]) -> bool:
+        """True when ``host_batch`` can run through the captured step (``load_batch`` / ``prefetch_batch`` accept it).
+        Route a batch that does not fit to ``train_step`` / ``predict_pages``."""
+        if self._static is None:
+            raise GteError("fits: call capture() first")
+        try:
+            self._page_layout(host_batch)
+        except GteError:
+            return False
+        return True
 
     def _page_layout(self, host_batch):
         """Validated (page_off, edge_off) host int32 tensors of a batch fed to a captured step, or None when the
-        captured step has no page table.  Raises when the batch cannot run through the captured kernels."""
+        captured step has no page table.  Raises when the batch cannot run through the captured kernels.  Capacity
+        capture: (n, e, P, key) of the batch, the padded page table is built when it is copied."""
+        if self._capacity is not None:
+            self._check_fit(self._capacity, host_batch, self._feat_width)
+            bn, be = tuple(host_batch["batch_num_nodes"]), tuple(host_batch["batch_num_edges"])
+            return int(host_batch["num_nodes"]), int(host_batch["src"].numel()), len(bn), (bn, be)
         n, e, bn0, be0 = self._static_meta
         if int(host_batch["num_nodes"]) != n or int(host_batch["src"].numel()) != e:
             raise GteError("captured step: batch node / edge totals differ from the captured ones")
@@ -407,6 +590,24 @@ class SageTrainer:
         return torch.from_numpy(po), torch.from_numpy(eo), (bn, be)
 
     def _copy_inputs(self, st, which: int, host_batch, layout):
+        if self._capacity is not None:
+            # the real prefix only: H2D bytes and host work follow the batch, not the capacity (the graph pads)
+            n, e, p, key = layout
+            for k, m in (("src", e), ("dst", e), ("weight", e), ("feat", n), ("label", n)):
+                st[k][:m].copy_(host_batch[k], non_blocking=True)
+            if self._loaded_layout[which] != key:
+                # a fresh pinned staging tensor per load: torch's caching host allocator keeps it until its
+                # non-blocking copy has run, so a queued copy never reads a rewritten buffer
+                po, eo = padded_page_table(self._capacity, key[0], key[1])
+                meta = torch.empty(st["meta"].numel(), dtype=torch.int32, pin_memory=True)
+                m = meta.numpy()
+                m[:4] = (n, e, p, 0)
+                m[4:4 + po.size] = po
+                m[4 + po.size:] = eo
+                st["meta"].copy_(meta, non_blocking=True)
+                self._loaded_layout[which] = key
+            self._set_rows[which] = (n, p)
+            return
         for k in ("src", "dst", "weight", "feat", "label"):
             st[k].copy_(host_batch[k], non_blocking=True)
         if layout is not None:
@@ -423,6 +624,7 @@ class SageTrainer:
         graph = torch.cuda.CUDAGraph()
         kw = {} if pool is None else {"pool": pool}
         with torch.cuda.graph(graph, **kw):
+            self._pad(st)
             if getattr(self, "_mode", "train") == "predict":
                 st["preds"], st["correct"] = self._predict_impl(self._static_graph(st), st["label"])
             elif self._split:
@@ -436,7 +638,8 @@ class SageTrainer:
     def load_batch(self, host_batch: Dict[str, torch.Tensor]):
         """Copy a host batch into static input set 0.  The batch must have the captured node / edge totals and page
         count and no page larger than the captured maxima; page ORDER and SIZES may differ (the page table is
-        refreshed with the batch)."""
+        refreshed with the batch).  Capacity capture: any batch that fits the capacity; one that does not is refused
+        with a GteError before anything is copied."""
         st = self._static
         if st is None:
             raise GteError("load_batch: call capture() first")
@@ -453,6 +656,9 @@ class SageTrainer:
     def _outputs(self, which: int):
         if getattr(self, "_mode", "train") == "predict":
             st = self._statics[which]
+            if self._capacity is not None:  # the batch that ran, without its padding
+                n, p = self._set_rows[which]
+                return st["preds"][:n], st["correct"][:p]
             return st["preds"], st["correct"]
         return self._result()
 
@@ -471,10 +677,16 @@ class SageTrainer:
         if getattr(self, "_stage_sets", None) is None:
             torch.cuda.synchronize(self.device)
             self._copy_stream = torch.cuda.Stream(device=self.device)
-            inputs = {k: v for k, v in self._static.items() if k not in ("preds", "correct")}
-            second = {k: torch.empty_like(v) for k, v in inputs.items()}
-            for k, v in inputs.items():
-                second[k].copy_(v)  # valid contents for the capture below (capturing runs nothing)
+            if self._capacity is None:
+                inputs = {k: v for k, v in self._static.items() if k not in ("preds", "correct")}
+                second = {k: torch.empty_like(v) for k, v in inputs.items()}
+                for k, v in inputs.items():
+                    second[k].copy_(v)  # valid contents for the capture below (capturing runs nothing)
+            else:
+                second = self._capacity_set()  # word / page_off / edge_off are views of meta: allocate, do not clone
+                for k in ("src", "dst", "weight", "feat", "label", "meta"):
+                    second[k].copy_(self._static[k])
+                self._set_rows[1] = self._set_rows[0]
             self._loaded_layout[1] = self._loaded_layout[0]
             pool = (self._graph[0] if isinstance(self._graph, tuple) else self._graph).pool()
             self._statics = [self._static, second]

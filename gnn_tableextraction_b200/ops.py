@@ -946,6 +946,27 @@ def build_page_formats(src, dst, w, page_off, edge_off, num_pages: int, n: int, 
     return csc, csr, norm, pk_csc, pk_csr, bad
 
 
+def pad_batch(word, page_off, edge_off, src, dst, weight, feat, label, bad: Optional[torch.Tensor] = None):
+    """Pad a page batch in place to the capacity shape its buffers have (gte_pad_batch): ``word`` = device int32
+    (n, e, P) of the real prefix, ``page_off`` / ``edge_off`` the full int32 page table [p_cap + 1] (real pages,
+    padding pages, empty pages), ``src`` / ``dst`` int32 and ``weight`` fp32 [e_cap], ``feat`` [n_cap, f],
+    ``label`` fp32 [n_cap].  Returns the device int32 flag (bit 0: word outside the capacity, bit 1: page table
+    inconsistent)."""
+    i32 = torch.int32
+    _req_cuda(word, page_off, edge_off, src, dst, weight, feat, label, bad)
+    fp, ldf, f = _mat(feat, "pad_batch.feat")
+    n_cap, e_cap, p_cap = int(feat.shape[0]), int(src.numel()), int(page_off.numel()) - 1
+    if dst.numel() != e_cap or weight.numel() != e_cap or label.numel() != n_cap or edge_off.numel() != p_cap + 1:
+        raise GteError("pad_batch: src / dst / weight need e_cap, label n_cap, edge_off p_cap + 1 entries")
+    if bad is None:
+        bad = torch.empty(1, dtype=i32, device=feat.device)
+    check(lib().gte_pad_batch(_vec(word, "word", i32, 3), n_cap, e_cap, p_cap, _vec(page_off, "page_off", i32),
+                              _vec(edge_off, "edge_off", i32), _vec(src, "src", i32), _vec(dst, "dst", i32),
+                              _vec(weight, "weight"), fp, ldf, f, _vec(label, "label"), _vec(bad, "bad", i32, 1),
+                              _stream()), "gte_pad_batch")
+    return bad
+
+
 def bbox_features(boxes: torch.Tensor, counts: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """13 BBOX features per text box (bbox.py:49-111) from int32 boxes [n,4] and character-class counts [n,3]."""
     _req_cuda(boxes, counts)

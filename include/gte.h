@@ -529,6 +529,23 @@ int gte_build_page_formats(const int32_t* src, const int32_t* dst, const float* 
                            float* norm, int32_t* page_flag, int32_t* bad, gte_stream_t stream);
 
 /*
+ * Pads a page batch to a capacity shape in place, so that one captured CUDA graph serves batches of any size up to
+ * the capacity: the shuffled training batches of model_train.py:283-297 and the streamed predict batches of
+ * model_predict.py:130-154 (whose last batch is short) change their node / edge totals from batch to batch.
+ * The caller fills the real prefix of src / dst / weight [e_cap], feat [n_cap, f] (row stride ldf) and label [n_cap],
+ * the device word `word` = (n, e, P) of that prefix, and the whole page table page_off / edge_off [p_cap + 1]:
+ * the P real pages, then padding pages, then empty pages (0 nodes, 0 edges) up to p_cap.  The kernel writes
+ *   feat rows [n, n_cap) = 0, label [n, n_cap) = -1, weight [e, e_cap) = 0,
+ *   src = dst over [e, e_cap) = a node of the padding page that owns the edge (a weight-0 self-loop),
+ * which makes the padded batch a valid dgl.batch whose padding adds nothing to the loss statistics or any
+ * gradient.  *bad (device int, cleared first): bit 0 = the word lies outside the capacity, bit 1 = the page table
+ * leaves a padding edge without a padding node; the kernel then clamps and writes nothing outside the buffers.
+ */
+int gte_pad_batch(const int32_t* word, int32_t n_cap, int64_t e_cap, int32_t p_cap, const int32_t* page_off,
+                  const int32_t* edge_off, int32_t* src, int32_t* dst, float* weight, float* feat, int64_t ldf,
+                  int32_t f, float* label, int32_t* bad, gte_stream_t stream);
+
+/*
  * BBOX node features on the device (src/components/nlp/bbox.py:49-54 get_shape, :57-111 get_histogram, called
  * per batch at model_train.py:293): boxes [n, 4] int32 = [x0, y0, x1, y1]; counts [n, 3] int32 = (letters,
  * digits, other symbols) of the box text with blanks removed (str.isalpha / str.isdigit are host string
