@@ -328,7 +328,8 @@ static int launch_spmm_paged(const int32_t* indptr, const int32_t* indices, cons
 //     (k_paged_pack_edges, once per graph and direction instead of once per CTA and slice),
 //   * runs one persistent CTA per SM over a contiguous range of (page, column slice) items with two
 //     shared-memory stages filled by the TMA unit (x slice: 2-D tensor boxes; packed edges: one bulk
-//     copy; row pointers / normalisers: 4-byte cp.async) while the previous item is reduced,
+//     copy; row pointers / normalisers: 4-byte cp.async tracked by the stage's mbarrier, so the producer
+//     never waits for them) while the previous item is reduced,
 //   * gives each lane V 128-bit column chunks of TWO rows at a time (G lanes per row) with the next
 //     group's metadata loaded ahead, so 8 independent 128-bit shared loads are in flight per lane,
 //   * prefetches the addend rows of the next item into L2 when it stages that item.
@@ -373,6 +374,16 @@ __device__ __forceinline__ void bulk_load_1d(uint32_t dst, const void* src, uint
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
                "r"(bytes), "r"(bar)
                : "memory");
+}
+
+// 4-byte asynchronous copy global -> shared (no register round trip: every copy of a lane is in flight at once)
+__device__ __forceinline__ void cp_async_4(uint32_t dst, const void* src) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory");
+}
+// the mbarrier's current phase also waits for every cp.async this thread issued so far (pending count +1, then an
+// arrive when they have landed: the expected arrival count is unchanged)
+__device__ __forceinline__ void cp_async_mbar_arrive(uint32_t bar) {
+  asm volatile("cp.async.mbarrier.arrive.shared.b64 [%0];" ::"r"(bar) : "memory");
 }
 
 struct PkStageLayout {
@@ -654,15 +665,17 @@ __global__ void __launch_bounds__(PK_THREADS, 1)
           mbar_arrive(bar);  // nothing in flight: the page runs from global memory
         }
       }
-      if (it.staged) {  // row pointers and normalisers: plain loads + shared stores by the 32 producer lanes
-        int32_t* sptr = reinterpret_cast<int32_t*>(sbase + off_ptr);
-        float* snrm = reinterpret_cast<float*>(sbase + off_nrm);
+      if (it.staged) {
+        // row pointers and normalisers: 4-byte cp.async by the 32 producer lanes, completion tracked by full[s].
+        // (Plain loads + shared stores cost the producer one global round trip per 4 entries and lane -- about six
+        // per 300-row page -- and that chain, not the ring depth, set the time of the narrow slices.)
         const int32_t* ip = indptr + it.n0;
-        for (int i = pl; i <= it.np; i += 32) sptr[i] = __ldg(ip + i);
+        for (int i = pl; i <= it.np; i += 32) cp_async_4(sx + off_ptr + 4u * i, ip + i);
         if (mode == GTE_AGG_SUM_NORM) {
           const float* nr = row_norm + it.n0;
-          for (int i = pl; i < it.np; i += 32) snrm[i] = __ldg(nr + i);
+          for (int i = pl; i < it.np; i += 32) cp_async_4(sx + off_nrm + 4u * i, nr + i);
         }
+        cp_async_mbar_arrive(bar);
       }
       if (addend) {  // pull the addend rows of this slice into L2 ahead of the consumers
         for (int i = pl; i < it.np * 2; i += 32) {

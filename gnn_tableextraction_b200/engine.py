@@ -264,7 +264,8 @@ class SageTrainer:
                 g, ctxs[i], dy, W, gamma, beta, gv[id(layer.linear.weight)],
                 None if layer.linear.bias is None else gv[id(layer.linear.bias)],
                 gv[id(layer.lynorm.weight)] if has_ln else None, gv[id(layer.lynorm.bias)] if has_ln else None,
-                need_dh=(i > 0), accumulate=False, dy_comb=dy_comb if i == len(layers) - 1 else None)
+                need_dh=(i > 0), accumulate=False, dy_comb=dy_comb if i == len(layers) - 1 else None,
+                dh_agg_first=True)
 
     def _all_reduce(self, t: torch.Tensor):
         if self.world > 1:

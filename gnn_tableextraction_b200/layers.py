@@ -145,6 +145,9 @@ def aggregate_backward(g: PageGraphBatch, d_out: torch.Tensor, w_edge: torch.Ten
 
 
 COMB = os.environ.get("GTE_COMB", "1") != "0"  # combined [n, 32] operands for the narrow layers (0: two operands, A/B runs)
+# input gradient of an aggregate-first layer when the caller allows it: "agg" = (A_hat^T dz) first, then one projection
+# [dz | A_hat^T dz] W; "layer" = [dz Ws | dz Wn] first, then A_hat^T (dz Wn) + dz Ws (A/B runs)
+DH_ORDER = os.environ.get("GTE_DH_ORDER", "agg")
 
 
 def _comb_rows(n: int) -> bool:
@@ -259,9 +262,12 @@ def sage_layer_backward(g: Optional[PageGraphBatch], ctx: LayerCtx, dy: torch.Te
                         gamma: Optional[torch.Tensor], beta: Optional[torch.Tensor], dW: torch.Tensor,
                         db: Optional[torch.Tensor], dgamma: Optional[torch.Tensor], dbeta: Optional[torch.Tensor],
                         *, need_dh: bool, accumulate: bool = False,
-                        dy_comb: Optional[torch.Tensor] = None) -> Optional[torch.Tensor]:
+                        dy_comb: Optional[torch.Tensor] = None, dh_agg_first: bool = False) -> Optional[torch.Tensor]:
     """Writes dW/db/dgamma/dbeta (overwrite or accumulate) and returns dh (or None).  ``dy_comb``: the buffer from
-    class_grad_buffer() whose self block IS ``dy`` (saves one copy of the class-layer gradient)."""
+    class_grad_buffer() whose self block IS ``dy`` (saves one copy of the class-layer gradient).  ``dh_agg_first``: an
+    aggregate-first tensor-core layer with fout <= fin and no dropout may build dh as [dz | A_hat^T dz] W (one SpMM of
+    the narrower dz without an addend, one two-segment projection) instead of A_hat^T (dz Wn) + dz Ws; the sums then run
+    in a different order, so callers that compare against the per-layer order leave it off."""
     fin, fout = ctx.fin, ctx.fout
     if ctx.ln:
         # the linear-bias gradient (column sums of dz) falls out of the same pass
@@ -294,6 +300,11 @@ def sage_layer_backward(g: Optional[PageGraphBatch], ctx: LayerCtx, dy: torch.Te
             ops.linear_bwd_weight(dz, ctx.h, ctx.ah, dW, db, accumulate)
         if not need_dh:
             return None
+        if (dh_agg_first and DH_ORDER == "agg" and drop is None and fout <= fin and ctx.pack is not None
+                and ops._aligned_mat(dz)):
+            # dh = dz Ws + A_hat^T (dz Wn) = [dz | A_hat^T dz] W: 5 instead of 6 passes over an [n, fin] matrix
+            # (the mask of [h | ah] sits between the projection and A_hat^T, hence no dropout)
+            return ops.umma_linear_bwd_data2(dz, aggregate_backward(g, dz, ctx.w_edge), ctx.pack, fin)
         if ctx.pack is not None and ops._aligned_mat(dz):
             d_self, d_ah = ops.umma_linear_bwd_data(dz, ctx.pack, fin, 2)
         else:
