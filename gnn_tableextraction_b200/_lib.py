@@ -80,6 +80,8 @@ SIGNATURES = {
     "gte_cross_entropy_fwd": (ci, [vp, i64, vp, ci, vp, i32, i32, vp, vp, sz, vp]),
     "gte_cross_entropy_bwd": (ci, [vp, i64, vp, ci, vp, i32, i32, vp, vp, i64, vp]),
     "gte_cross_entropy_bwd_padded": (ci, [vp, i64, vp, ci, vp, i32, i32, vp, vp, i64, i32, vp]),
+    "gte_eval_workspace_bytes": (sz, [i32]),
+    "gte_eval_accumulate": (ci, [vp, i64, vp, ci, vp, i32, i32, vp, vp, sz, vp]),
     "gte_comb_fill": (ci, [vp, i64, i32, vp, i64, i64, vp]),
     "gte_page_predictions": (ci, [vp, i64, i32, i32, vp, ci, vp, i32, vp, vp, vp]),
     "gte_build_page_formats_smem_bytes": (sz, [i32, i32]),

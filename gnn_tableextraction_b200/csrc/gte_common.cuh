@@ -84,6 +84,24 @@ __device__ __forceinline__ float reduce_partials_block(const float* __restrict__
     for (int k = 0; k < RED_SLICES; ++k) t += smem[k * 32 + ox];
   return t;
 }
+
+// torch.argmax of one row of c >= 1 values: the first maximal index, a NaN counting as maximal (the first NaN wins)
+__device__ __forceinline__ int row_argmax(const float* __restrict__ lr, int c) {
+  float mx = lr[0];
+  int arg = 0;
+  bool nan = mx != mx;
+  for (int j = 1; j < c && !nan; ++j) {
+    const float v = lr[j];
+    if (v != v) {
+      arg = j;
+      nan = true;
+    } else if (v > mx) {
+      mx = v;
+      arg = j;
+    }
+  }
+  return arg;
+}
 #endif
 
 }  // namespace gte

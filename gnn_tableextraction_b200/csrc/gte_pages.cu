@@ -30,20 +30,7 @@ __global__ void __launch_bounds__(256)
   const int32_t n0 = page_off[page], n1 = page_off[page + 1];
   int correct = 0;
   for (int32_t i = n0 + threadIdx.x; i < n1; i += blockDim.x) {
-    const float* lr = logits + (int64_t)i * ld;
-    float mx = lr[0];
-    int arg = 0;
-    bool nan = mx != mx;  // torch.argmax treats NaN as the maximum (first NaN wins)
-    for (int j = 1; j < c && !nan; ++j) {
-      const float v = lr[j];
-      if (v != v) {
-        arg = j;
-        nan = true;
-      } else if (v > mx) {
-        mx = v;
-        arg = j;
-      }
-    }
+    const int arg = row_argmax(logits + (int64_t)i * ld, c);
     preds[i] = arg;
     if (labels && page_label(labels, label_dtype, i) == arg) ++correct;
   }

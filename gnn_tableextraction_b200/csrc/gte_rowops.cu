@@ -243,17 +243,19 @@ __global__ void __launch_bounds__(ROW_THREADS)
   }
 }
 
-// out[i] (+)= sum_b partial[b*stride + i] in a fixed order; 32 outputs per block
+// out[i] (+)= sum_b partial[b*stride + i] in a fixed order; 32 outputs per block (T = double: added in double)
+template <typename T>
 __global__ void __launch_bounds__(RED_THREADS)
-    k_reduce_partials(const float* __restrict__ partial, int nb, int64_t stride, int32_t count, float* __restrict__ out,
+    k_reduce_partials(const float* __restrict__ partial, int nb, int64_t stride, int32_t count, T* __restrict__ out,
                       int accumulate) {
   __shared__ float red[RED_THREADS];
   const int i = blockIdx.x * 32 + (threadIdx.x & 31);
   const bool valid = i < count;
-  float s = reduce_partials_block(partial, nb, stride, i, valid, red);
+  const float s = reduce_partials_block(partial, nb, stride, i, valid, red);
   if ((threadIdx.x >> 5) != 0 || !valid) return;
-  if (accumulate) s += out[i];
-  out[i] = s;
+  T r = s;
+  if (accumulate) r += out[i];
+  out[i] = r;
 }
 
 // three reductions over one partial matrix [nb][3 * f] in one launch: out_k[i] (+)= sum_b partial[b * 3f + k * f + i]
@@ -374,11 +376,21 @@ __device__ __forceinline__ int64_t load_label(const void* labels, int dtype, int
 
 constexpr int CE_THREADS = 256;
 
-// per-block partials: [block][3] = {sum w*nll, sum w, #correct}
+// per-block partials: [block][3] = {sum w*nll, sum w, #correct}.
+// EVAL (gte_eval_accumulate): no #correct (its partial is 0); the block counts (label, torch.argmax) pairs of the rows
+// with a label in [0, c) in a c x c int32 histogram in dynamic shared memory and adds it to cm[c * c] (float64) at
+// the end: integral sums below 2^53 are exact in any order.
+template <bool EVAL>
 __global__ void __launch_bounds__(CE_THREADS)
     k_ce_fwd(const float* __restrict__ logits, int64_t ld, const void* __restrict__ labels, int label_dtype,
-             const float* __restrict__ class_w, int32_t n, int32_t c, float* __restrict__ partial) {
+             const float* __restrict__ class_w, int32_t n, int32_t c, float* __restrict__ partial,
+             double* __restrict__ cm) {
   __shared__ float red[3][CE_THREADS / 32];
+  extern __shared__ int hist[];
+  if constexpr (EVAL) {
+    for (int k = threadIdx.x; k < c * c; k += CE_THREADS) hist[k] = 0;
+    __syncthreads();
+  }
   float loss = 0.f, wsum = 0.f, correct = 0.f;
   for (int64_t i = (int64_t)blockIdx.x * CE_THREADS + threadIdx.x; i < n; i += (int64_t)gridDim.x * CE_THREADS) {
     const float* lr = logits + i * ld;
@@ -399,8 +411,9 @@ __global__ void __launch_bounds__(CE_THREADS)
       const float nll = (mx + logf(se)) - lr[yv];
       loss = fmaf(wv, nll, loss);
       wsum += wv;
+      if constexpr (EVAL) atomicAdd(&hist[(int)yv * c + row_argmax(lr, c)], 1);
     }
-    correct += (arg == (int)yv) ? 1.f : 0.f;
+    if constexpr (!EVAL) correct += (arg == (int)yv) ? 1.f : 0.f;
   }
   loss = warp_sum(loss);
   wsum = warp_sum(wsum);
@@ -415,6 +428,10 @@ __global__ void __launch_bounds__(CE_THREADS)
     float s = 0.f;
     for (int w = 0; w < CE_THREADS / 32; ++w) s += red[threadIdx.x][w];
     partial[(int64_t)blockIdx.x * 3 + threadIdx.x] = s;
+  }
+  if constexpr (EVAL) {
+    for (int k = threadIdx.x; k < c * c; k += CE_THREADS)  // after the __syncthreads above: the histogram is complete
+      if (hist[k] != 0) atomicAdd(cm + k, (double)hist[k]);
   }
 }
 
@@ -797,11 +814,34 @@ int gte_cross_entropy_fwd(const float* logits, int64_t ld, const void* labels, i
   float* partial = static_cast<float*>(ws);
   const int grid = ce_grid(n);
   if (n > 0) {
-    k_ce_fwd<<<grid, CE_THREADS, 0, st>>>(logits, ld, labels, label_dtype, class_w, n, c, partial);
+    k_ce_fwd<false><<<grid, CE_THREADS, 0, st>>>(logits, ld, labels, label_dtype, class_w, n, c, partial, nullptr);
     GTE_CHECK_LAUNCH("k_ce_fwd");
   }
-  k_reduce_partials<<<1, RED_THREADS, 0, st>>>(partial, n > 0 ? grid : 0, 3, 3, stats, 0);
+  k_reduce_partials<float><<<1, RED_THREADS, 0, st>>>(partial, n > 0 ? grid : 0, 3, 3, stats, 0);
   GTE_CHECK_LAUNCH("k_reduce_partials(ce)");
+  return GTE_OK;
+}
+
+size_t gte_eval_workspace_bytes(int32_t n) { return gte_cross_entropy_workspace_bytes(n); }
+
+int gte_eval_accumulate(const float* logits, int64_t ld, const void* labels, int label_dtype, const float* class_w,
+                        int32_t n, int32_t c, double* totals, void* ws, size_t ws_bytes, gte_stream_t stream) {
+  GTE_CHECK_ARG(n >= 0 && c > 0 && c <= GTE_EVAL_MAX_CLASSES, "gte_eval_accumulate: need 0 < c <= %d classes (got %d)",
+                GTE_EVAL_MAX_CLASSES, c);
+  GTE_CHECK_ARG(label_dtype >= GTE_LABEL_I64 && label_dtype <= GTE_LABEL_F32, "gte_eval_accumulate: bad label dtype");
+  if (n == 0) return GTE_OK;
+  GTE_CHECK_ARG(logits && labels && totals && ld >= c, "gte_eval_accumulate: bad argument");
+  const size_t need = gte_eval_workspace_bytes(n);
+  if (ws == nullptr || ws_bytes < need)
+    return fail(GTE_ERR_WORKSPACE, "gte_eval_accumulate: workspace %zu < required %zu", ws_bytes, need);
+  cudaStream_t st = as_stream(stream);
+  float* partial = static_cast<float*>(ws);
+  const int grid = ce_grid(n);
+  k_ce_fwd<true><<<grid, CE_THREADS, (size_t)c * c * sizeof(int), st>>>(logits, ld, labels, label_dtype, class_w, n, c,
+                                                                       partial, totals + 2);
+  GTE_CHECK_LAUNCH("k_ce_fwd(eval)");
+  k_reduce_partials<double><<<1, RED_THREADS, 0, st>>>(partial, grid, 3, 2, totals, 1);
+  GTE_CHECK_LAUNCH("k_reduce_partials(eval)");
   return GTE_OK;
 }
 

@@ -205,9 +205,9 @@ class SageTrainer:
             for t in (self.flat_param, self.exp_avg, self.exp_avg_sq, self.step_dev):
                 torch.distributed.broadcast(t, src=torch.distributed.get_global_rank(self.pg, 0) if self.pg is not None else 0,
                                             group=self.pg)
-        self._graph = None
-        self._static: Optional[Dict[str, torch.Tensor]] = None
-        self._capacity: Optional[BatchCapacity] = None
+        self.num_classes = int(model.layers[-1].linear.weight.shape[0])
+        self._train: Optional[_CapturedPass] = None  # the captured train or predict step
+        self._mode = "train"
 
     # ----------------------------------------------------------- pieces ----
     def _layer_args(self, layer):
@@ -341,9 +341,14 @@ class SageTrainer:
         """device tensor [sum w*nll, sum w, #correct] of the last step (global over ranks)"""
         return self._result()
 
-    def _step_impl(self, g: PageGraphBatch, labels: torch.Tensor):
+    def _stage_local(self, g: PageGraphBatch, labels: torch.Tensor):
+        """the step up to the gradient exchange: forward + loss + backward"""
         logits, ctxs = self._stage_forward(g, labels)
         self._stage_backward(g, labels, logits, ctxs)
+        return logits
+
+    def _step_impl(self, g: PageGraphBatch, labels: torch.Tensor):
+        logits = self._stage_local(g, labels)
         self._stage_exchange_update()
         return logits
 
@@ -396,7 +401,54 @@ class SageTrainer:
             acc = correct.to(torch.float64) / sizes
         return preds, acc
 
+    # ------------------------------------------------------- evaluation -----
+    def _eval_impl(self, g: PageGraphBatch, labels: torch.Tensor, totals: torch.Tensor):
+        """forward without dropout and without saved activations + gte_eval_accumulate into ``totals``: reads the
+        parameters, writes nothing the train step reads (not rng_dev, not self.stats / the flat-gradient tail)"""
+        logits, _ = self.forward(g, keep_ctx=False)
+        ops.eval_accumulate(logits, labels, self.class_w, totals)
+
+    def eval_totals(self) -> torch.Tensor:
+        """A zeroed float64 device buffer [2 + C*C] for ``evaluate``: [sum w*nll, sum w, confusion counts C x C]."""
+        return torch.zeros(2 + self.num_classes ** 2, dtype=torch.float64, device=self.device)
+
+    @torch.no_grad()
+    def evaluate(self, g: PageGraphBatch, labels: Optional[torch.Tensor] = None,
+                 totals: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The validation step of model_train.py:349-364 on the device: forward (always without dropout, nothing saved
+        for a backward pass), then the weighted CE statistics and the confusion matrix of ``torch.argmax`` ADDED to
+        ``totals`` (a fresh ``eval_totals()`` when None), which is returned.  Rows with a label outside [0, C) are
+        skipped.  ``EvalCapture.result`` shows how to read the totals.  No host synchronisation happens here."""
+        if labels is None:
+            labels = g.ndata["label"]
+        if totals is None:
+            totals = self.eval_totals()
+        with torch.cuda.device(self.device):
+            self._eval_impl(g, labels, totals)
+        return totals
+
+    def capture_eval(self, host_batch: Dict[str, torch.Tensor], capacity: Optional[BatchCapacity] = None) -> "EvalCapture":
+        """Capture ``evaluate`` as a pass of its own, beside the captured train step (which stays): without a capacity
+        for batches of this shape -- ``host_batch`` stays resident and ``replay()`` copies nothing, the fixed
+        validation batch of model_train.py:242-249 --, with one for every batch that fits it (see ``capture``).  The
+        pass has its own memory pool and totals buffer and reads the live parameters, so after a train replay it sees
+        the updated weights."""
+        return EvalCapture(self, host_batch, capacity)
+
     # ----------------------------------------------------- CUDA graphs -----
+    @property
+    def _static(self) -> Optional[Dict[str, torch.Tensor]]:
+        """static input set 0 of the captured train / predict step"""
+        return None if self._train is None else self._train.statics[0]
+
+    @property
+    def _statics(self) -> Optional[List[Dict[str, torch.Tensor]]]:
+        return None if self._train is None else self._train.statics
+
+    @property
+    def _graph(self):
+        return None if self._train is None else self._train.graphs[0]
+
     def capture_predict(self, host_batch: Dict[str, torch.Tensor], capacity: Optional[BatchCapacity] = None):
         """Capture the batched predict pass of model_predict.py:130-154 (format build + forward without saved
         activations + argmax + per-page correct counts) for batches of this shape, or for every batch that fits
@@ -416,19 +468,94 @@ class SageTrainer:
         of model_train.py:283-297.  The static inputs have the capacity's padded shape; a batch is copied as it is and
         ``gte_pad_batch``, the first kernel of the graph, pads it on the device with zero-feature, label -1 nodes and
         weight-0 self-loops in pages of their own, which change no loss statistic and no gradient.  ``host_batch``
-        must fit; it gives the feature width and the warm-up contents."""
+        must fit; it gives the feature width and the warm-up contents.
+
+        A trainer holds one captured step: a new capture replaces the previous one.  A pass captured by
+        ``capture_eval`` is separate and stays."""
         if split is None:
             split = self.world > 1 and self._dp_peer is None  # the peer-memory exchange is an ordinary kernel: one graph
         if mode not in ("train", "predict"):
             raise GteError(f"capture: unknown mode {mode}")
+        if mode == "predict":
+            body, tail = self._predict_impl, None
+        elif split:  # [graph: batch assembly + forward + CE + backward] -> ONE all-reduce -> Adam (eager, 2 launches)
+            body, tail = self._stage_local, self._stage_exchange_update
+        else:
+            body, tail = self._step_impl, None
+        # the warm-up steps train: restore the optimiser state afterwards
+        snap = (self.flat_param.clone(), self.exp_avg.clone(), self.exp_avg_sq.clone(), self.step_dev.clone())
+        self._train = _CapturedPass(self.device, host_batch, capacity, body, tail)
+        self._mode = mode
+        self.flat_param.copy_(snap[0])
+        self.exp_avg.copy_(snap[1])
+        self.exp_avg_sq.copy_(snap[2])
+        self.step_dev.copy_(snap[3])
+        return self._graph
+
+    def _captured(self, what: str) -> "_CapturedPass":
+        if self._train is None:
+            raise GteError(f"{what}: call capture() first")
+        return self._train
+
+    def fits(self, host_batch: Dict[str, torch.Tensor]) -> bool:
+        """True when ``host_batch`` can run through the captured step (``load_batch`` / ``prefetch_batch`` accept it).
+        Route a batch that does not fit to ``train_step`` / ``predict_pages``."""
+        return self._captured("fits").fits(host_batch)
+
+    def load_batch(self, host_batch: Dict[str, torch.Tensor]):
+        """Copy a host batch into static input set 0.  The batch must have the captured node / edge totals and page
+        count and no page larger than the captured maxima; page ORDER and SIZES may differ (the page table is
+        refreshed with the batch).  Capacity capture: any batch that fits the capacity; one that does not is refused
+        with a GteError before anything is copied."""
+        self._captured("load_batch").load_batch(host_batch)
+
+    def _outputs(self, which: int):
+        if self._mode == "predict":
+            preds, correct = self._train.outs[which]
+            if self._train.capacity is not None:  # the batch that ran, without its padding
+                n, p = self._train.rows[which]
+                return preds[:n], correct[:p]
+            return preds, correct
+        return self._result()
+
+    def replay(self):
+        self._captured("replay").replay(0)
+        return self._outputs(0)
+
+    def prefetch_batch(self, host_batch: Dict[str, torch.Tensor]):
+        """Start the H2D copy of the NEXT batch on a side stream.  Two static input sets alternate, each with its own
+        captured graph (sharing one memory pool), so the step reads the batch where the copy engine put it: no
+        device-to-device staging copy.  ``replay_prefetched()`` consumes the sets in order."""
+        self._captured("prefetch_batch").prefetch_batch(host_batch)
+
+    def replay_set(self, which: int) -> torch.Tensor:
+        """Run one captured step on static input set ``which`` (0 or 1) as it is: inputs resident in HBM, no copy.
+        The sets are filled by ``prefetch_batch`` / ``load_batch``; the caller keeps track of what is in them."""
+        self._captured("replay_set").replay_set(which)
+        return self._outputs(which)
+
+    def replay_prefetched(self):
+        """Run one captured step on the oldest prefetched batch."""
+        if self._train is None:
+            raise GteError("replay_prefetched: no prefetched batch")
+        return self._outputs(self._train.replay_prefetched())
+
+
+class _CapturedPass:
+    """One captured pass: the CUDA graph of ``body(g, labels)`` over static input sets, and everything that feeds it --
+    the static inputs of the batch shape or of a ``BatchCapacity`` (padded on the device by gte_pad_batch, the first
+    kernel of the graph), the validation and page layout of a fed batch, its host->device copies and the two-set
+    prefetch pipeline.  ``outs[i]`` keeps what ``body`` returned while capturing over input set i.  ``tail`` (may be
+    None) runs eagerly after every replay: the data-parallel all-reduce + Adam of a split train step."""
+
+    def __init__(self, device, host_batch: Dict[str, torch.Tensor], capacity: Optional[BatchCapacity], body, tail=None):
         if capacity is not None:
             self._check_capacity(capacity, host_batch)
-        self._mode = mode
-        self._capacity = capacity
-        dev = self.device
+        self.device, self.capacity, self.body, self.tail = device, capacity, body, tail
+        dev = device
         if capacity is None:
             n, e = int(host_batch["num_nodes"]), int(host_batch["src"].numel())
-            f = int(host_batch["feat"].shape[1])
+            f = self.feat_width = int(host_batch["feat"].shape[1])
             st = {
                 "src": torch.empty(e, dtype=torch.int32, device=dev),
                 "dst": torch.empty(e, dtype=torch.int32, device=dev),
@@ -436,9 +563,8 @@ class SageTrainer:
                 "feat": torch.empty((n, f), dtype=torch.float32, device=dev),
                 "label": torch.empty(n, dtype=torch.float32, device=dev),
             }
-            self._static = st
             bn, be = list(host_batch["batch_num_nodes"]), list(host_batch["batch_num_edges"])
-            self._static_meta = (n, e, bn, be)
+            self.meta = (n, e, bn, be)
             # The page table (node / edge offsets of the pages) is part of the INPUT: a later batch with the same totals
             # may order or size its pages differently, so every static input set owns device copies of the two offset
             # arrays and load_batch / prefetch_batch refresh them.  Only the maxima (shared-memory sizing of the page
@@ -446,51 +572,43 @@ class SageTrainer:
             pages = page_table(bn, be, n, dev)
             if pages is not None:
                 st["page_off"], st["edge_off"] = pages[0], pages[4]
-                self._static_caps = (pages[1], pages[2], pages[3])  # page count, max page nodes, max page edges
+                self.caps = (pages[1], pages[2], pages[3])  # page count, max page nodes, max page edges
             else:
-                self._static_caps = None
+                self.caps = None
         else:
             n_cap, e_cap, p_cap = capacity.shape
-            self._feat_width = int(host_batch["feat"].shape[1])
+            self.feat_width = int(host_batch["feat"].shape[1])
             st = self._capacity_set()
-            self._static = st
             # the structure the captured kernels see: P_cap pages, none larger than the capacity's page caps (the
             # page lists only size the batch; the offsets come from st["page_off"] / st["edge_off"] every replay)
             po, eo = padded_page_table(capacity, host_batch["batch_num_nodes"], host_batch["batch_num_edges"])
-            self._static_meta = (n_cap, e_cap, np.diff(po).tolist(), np.diff(eo).tolist())
-            self._static_caps = (p_cap, capacity.page_nodes, capacity.page_edges)
-            self._set_rows = [None, None]  # (n, P) of the batch in each input set: predict outputs are cut to it
-        self._loaded_layout = [None, None]
+            self.meta = (n_cap, e_cap, np.diff(po).tolist(), np.diff(eo).tolist())
+            self.caps = (p_cap, capacity.page_nodes, capacity.page_edges)
+        self.rows = [None, None]  # capacity capture: (n, P) of the batch in each input set
+        self.loaded_layout = [None, None]
+        self.statics = [st]
+        self.stage_sets = None
         self.load_batch(host_batch)
 
-        self._split = split
-        # warm-up on a side stream (allocator + lazy module state), restoring the optimiser state afterwards
-        snap = (self.flat_param.clone(), self.exp_avg.clone(), self.exp_avg_sq.clone(), self.step_dev.clone())
+        # warm-up on a side stream (allocator + lazy module state)
         s = torch.cuda.Stream(device=dev)
         s.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(s):
             for _ in range(2):
                 self._pad(st)
-                if mode == "train":
-                    self._step_impl(self._static_graph(st), st["label"])
-                else:
-                    self._predict_impl(self._static_graph(st), st["label"])
+                body(self.graph_of(st), st["label"])
+                if tail is not None:
+                    tail()
         torch.cuda.current_stream(dev).wait_stream(s)
         torch.cuda.synchronize(dev)
         self._check_static_structure(st)
-        self._graph = self._capture_over(st)
-        self._statics, self._graphs = [st], [self._graph]
-        self._stage_sets = None
-        self.flat_param.copy_(snap[0])
-        self.exp_avg.copy_(snap[1])
-        self.exp_avg_sq.copy_(snap[2])
-        self.step_dev.copy_(snap[3])
-        return self._graph
+        self.outs = [None, None]
+        self.graphs = [self._capture_over(0)]
 
-    def _static_graph(self, st) -> PageGraphBatch:
-        n = self._static_meta[0]
-        g = PageGraphBatch(st["src"], st["dst"], n, self._static_meta[2], self._static_meta[3])
-        caps = self._static_caps
+    def graph_of(self, st) -> PageGraphBatch:
+        n = self.meta[0]
+        g = PageGraphBatch(st["src"], st["dst"], n, self.meta[2], self.meta[3])
+        caps = self.caps
         g._cache["pages"] = None if caps is None else (st["page_off"], caps[0], caps[1], caps[2], st["edge_off"])
         g.edata["feat"] = st["weight"]
         g.ndata["feat"] = st["feat"]
@@ -499,21 +617,22 @@ class SageTrainer:
     def _check_static_structure(self, st):
         """Host check (one synchronisation, capture time only) that the batch in ``st`` honours its page table: the
         one-kernel batch assembly raises a device flag when an edge leaves its page (results would be undefined)."""
-        g = self._static_graph(st)
+        g = self.graph_of(st)
         if g.prepare(st["weight"]):
             g.check_page_structure()
         if "pad_bad" in st and int(st["pad_bad"].item()) != 0:
             raise GteError("capture: gte_pad_batch flagged the padded batch (word outside the capacity or bad page table)")
 
     # -- capacity capture: one graph for every batch that fits a BatchCapacity ------------------------------------
-    def _check_capacity(self, capacity: BatchCapacity, host_batch):
+    @classmethod
+    def _check_capacity(cls, capacity: BatchCapacity, host_batch):
         if not isinstance(capacity, BatchCapacity):
             raise GteError(f"capture: capacity must be a BatchCapacity, got {type(capacity).__name__}")
         _, _, p_cap = capacity.shape
         if not ops.page_formats_supported((None, p_cap, capacity.page_nodes, capacity.page_edges)):
             raise GteError(f"capture: pages of {capacity.page_nodes} nodes / {capacity.page_edges} edges do not fit the "
                            "one-kernel batch assembly (shared memory); lower page_nodes / page_edges")
-        self._check_fit(capacity, host_batch, int(host_batch["feat"].shape[1]))
+        cls._check_fit(capacity, host_batch, int(host_batch["feat"].shape[1]))
 
     @staticmethod
     def _check_fit(capacity: BatchCapacity, host_batch, f: int):
@@ -532,29 +651,25 @@ class SageTrainer:
         """One static input set of the capacity shape.  ``meta`` = [n, e, P, 0 | page_off (P_cap + 1) | edge_off
         (P_cap + 1)] travels in ONE copy; ``word``, ``page_off`` and ``edge_off`` are views of it."""
         dev = self.device
-        n_cap, e_cap, p_cap = self._capacity.shape
+        n_cap, e_cap, p_cap = self.capacity.shape
         meta = torch.zeros(4 + 2 * (p_cap + 1), dtype=torch.int32, device=dev)
         return {
             "src": torch.zeros(e_cap, dtype=torch.int32, device=dev),
             "dst": torch.zeros(e_cap, dtype=torch.int32, device=dev),
             "weight": torch.zeros(e_cap, dtype=torch.float32, device=dev),
-            "feat": torch.zeros((n_cap, self._feat_width), dtype=torch.float32, device=dev),
+            "feat": torch.zeros((n_cap, self.feat_width), dtype=torch.float32, device=dev),
             "label": torch.zeros(n_cap, dtype=torch.float32, device=dev),
             "meta": meta, "word": meta[:4], "page_off": meta[4:5 + p_cap], "edge_off": meta[5 + p_cap:],
             "pad_bad": torch.zeros(1, dtype=torch.int32, device=dev),
         }
 
     def _pad(self, st):
-        """first kernel of a capacity-captured step: pad the batch in ``st`` to the capacity shape"""
-        if self._capacity is not None:
+        """first kernel of a capacity-captured pass: pad the batch in ``st`` to the capacity shape"""
+        if self.capacity is not None:
             ops.pad_batch(st["word"], st["page_off"], st["edge_off"], st["src"], st["dst"], st["weight"], st["feat"],
                           st["label"], bad=st["pad_bad"])
 
     def fits(self, host_batch: Dict[str, torch.Tensor]) -> bool:
-        """True when ``host_batch`` can run through the captured step (``load_batch`` / ``prefetch_batch`` accept it).
-        Route a batch that does not fit to ``train_step`` / ``predict_pages``."""
-        if self._static is None:
-            raise GteError("fits: call capture() first")
         try:
             self._page_layout(host_batch)
         except GteError:
@@ -562,20 +677,23 @@ class SageTrainer:
         return True
 
     def _page_layout(self, host_batch):
-        """Validated (page_off, edge_off) host int32 tensors of a batch fed to a captured step, or None when the
-        captured step has no page table.  Raises when the batch cannot run through the captured kernels.  Capacity
+        """Validated (page_off, edge_off) host int32 tensors of a batch fed to a captured pass, or None when the
+        captured pass has no page table.  Raises when the batch cannot run through the captured kernels.  Capacity
         capture: (n, e, P, key) of the batch, the padded page table is built when it is copied."""
-        if self._capacity is not None:
-            self._check_fit(self._capacity, host_batch, self._feat_width)
+        if self.capacity is not None:
+            self._check_fit(self.capacity, host_batch, self.feat_width)
             bn, be = tuple(host_batch["batch_num_nodes"]), tuple(host_batch["batch_num_edges"])
             return int(host_batch["num_nodes"]), int(host_batch["src"].numel()), len(bn), (bn, be)
-        n, e, bn0, be0 = self._static_meta
+        n, e, bn0, be0 = self.meta
         if int(host_batch["num_nodes"]) != n or int(host_batch["src"].numel()) != e:
             raise GteError("captured step: batch node / edge totals differ from the captured ones")
-        if self._static_caps is None:
+        feat = host_batch["feat"]
+        if feat.dim() != 2 or int(feat.shape[1]) != self.feat_width:
+            raise GteError(f"captured step: features {tuple(feat.shape)}, expected [{n}, {self.feat_width}]")
+        if self.caps is None:
             return None
         bn, be = list(host_batch["batch_num_nodes"]), list(host_batch["batch_num_edges"])
-        p, max_n, max_e = self._static_caps
+        p, max_n, max_e = self.caps
         if len(bn) != p or len(be) != p or sum(bn) != n or sum(be) != e:
             raise GteError("captured step: page count / page sizes do not add up to the captured batch shape")
         if max(bn) > max_n or max(be) > max_e:
@@ -583,116 +701,83 @@ class SageTrainer:
                            f"({max_n}, {max_e}) the page kernels were sized for; capture with the largest batch first")
         if "page_off" in host_batch and "edge_off" in host_batch:
             return host_batch["page_off"], host_batch["edge_off"], (bn, be)
-        import numpy as np
         po = np.zeros(p + 1, dtype=np.int32)
         eo = np.zeros(p + 1, dtype=np.int32)
         np.cumsum(np.asarray(bn, dtype=np.int64), out=po[1:])
         np.cumsum(np.asarray(be, dtype=np.int64), out=eo[1:])
         return torch.from_numpy(po), torch.from_numpy(eo), (bn, be)
 
-    def _copy_inputs(self, st, which: int, host_batch, layout):
-        if self._capacity is not None:
+    def _copy_inputs(self, which: int, host_batch, layout):
+        st = self.statics[which]
+        if self.capacity is not None:
             # the real prefix only: H2D bytes and host work follow the batch, not the capacity (the graph pads)
             n, e, p, key = layout
             for k, m in (("src", e), ("dst", e), ("weight", e), ("feat", n), ("label", n)):
                 st[k][:m].copy_(host_batch[k], non_blocking=True)
-            if self._loaded_layout[which] != key:
+            if self.loaded_layout[which] != key:
                 # a fresh pinned staging tensor per load: torch's caching host allocator keeps it until its
                 # non-blocking copy has run, so a queued copy never reads a rewritten buffer
-                po, eo = padded_page_table(self._capacity, key[0], key[1])
+                po, eo = padded_page_table(self.capacity, key[0], key[1])
                 meta = torch.empty(st["meta"].numel(), dtype=torch.int32, pin_memory=True)
                 m = meta.numpy()
                 m[:4] = (n, e, p, 0)
                 m[4:4 + po.size] = po
                 m[4 + po.size:] = eo
                 st["meta"].copy_(meta, non_blocking=True)
-                self._loaded_layout[which] = key
-            self._set_rows[which] = (n, p)
+                self.loaded_layout[which] = key
+            self.rows[which] = (n, p)
             return
         for k in ("src", "dst", "weight", "feat", "label"):
             st[k].copy_(host_batch[k], non_blocking=True)
         if layout is not None:
             po, eo, key = layout
-            if self._loaded_layout[which] != key:  # fixed-size pages: the offsets never change, skip the copies
+            if self.loaded_layout[which] != key:  # fixed-size pages: the offsets never change, skip the copies
                 st["page_off"].copy_(po, non_blocking=True)
                 st["edge_off"].copy_(eo, non_blocking=True)
-                self._loaded_layout[which] = key
+                self.loaded_layout[which] = key
 
-    def _capture_over(self, st, pool=None):
-        """Capture the step reading the static input set ``st`` (capturing launches nothing).  Under data parallelism
-        the collective stays outside: [graph: batch assembly + forward + CE + backward] -> ONE all-reduce (flat
-        gradient + loss statistics) -> Adam (eager, 2 launches)."""
+    def _capture_over(self, which: int, pool=None):
+        """Capture the pass reading static input set ``which`` (capturing launches nothing)."""
+        st = self.statics[which]
         graph = torch.cuda.CUDAGraph()
         kw = {} if pool is None else {"pool": pool}
         with torch.cuda.graph(graph, **kw):
             self._pad(st)
-            if getattr(self, "_mode", "train") == "predict":
-                st["preds"], st["correct"] = self._predict_impl(self._static_graph(st), st["label"])
-            elif self._split:
-                g = self._static_graph(st)
-                logits, ctxs = self._stage_forward(g, st["label"])
-                self._stage_backward(g, st["label"], logits, ctxs)
-            else:
-                self._step_impl(self._static_graph(st), st["label"])
-        return (graph,) if self._split else graph
+            self.outs[which] = self.body(self.graph_of(st), st["label"])
+        return (graph,) if self.tail is not None else graph
 
     def load_batch(self, host_batch: Dict[str, torch.Tensor]):
-        """Copy a host batch into static input set 0.  The batch must have the captured node / edge totals and page
-        count and no page larger than the captured maxima; page ORDER and SIZES may differ (the page table is
-        refreshed with the batch).  Capacity capture: any batch that fits the capacity; one that does not is refused
-        with a GteError before anything is copied."""
-        st = self._static
-        if st is None:
-            raise GteError("load_batch: call capture() first")
-        self._copy_inputs(st, 0, host_batch, self._page_layout(host_batch))
+        self._copy_inputs(0, host_batch, self._page_layout(host_batch))
 
-    def _replay_graphs(self, which: int = 0):
-        graph = self._graphs[which] if getattr(self, "_graphs", None) else self._graph
+    def replay(self, which: int = 0):
+        graph = self.graphs[which]
         if isinstance(graph, tuple):
             graph[0].replay()
-            self._stage_exchange_update()
+            self.tail()
         else:
             graph.replay()
 
-    def _outputs(self, which: int):
-        if getattr(self, "_mode", "train") == "predict":
-            st = self._statics[which]
-            if self._capacity is not None:  # the batch that ran, without its padding
-                n, p = self._set_rows[which]
-                return st["preds"][:n], st["correct"][:p]
-            return st["preds"], st["correct"]
-        return self._result()
-
-    def replay(self):
-        self._replay_graphs()
-        return self._outputs(0)
-
-    # -- pipelined input: the host->device copy of batch i+1 overlaps the step of batch i ----------------------
+    # -- pipelined input: the host->device copy of batch i+1 overlaps the pass over batch i ----------------------
     def prefetch_batch(self, host_batch: Dict[str, torch.Tensor]):
-        """Start the H2D copy of the NEXT batch on a side stream.  Two static input sets alternate, each with its own
-        captured graph (sharing one memory pool), so the step reads the batch where the copy engine put it: no
-        device-to-device staging copy.  ``replay_prefetched()`` consumes the sets in order."""
-        if self._static is None:
-            raise GteError("prefetch_batch: call capture() first")
         layout = self._page_layout(host_batch)
-        if getattr(self, "_stage_sets", None) is None:
+        if self.stage_sets is None:
             torch.cuda.synchronize(self.device)
             self._copy_stream = torch.cuda.Stream(device=self.device)
-            if self._capacity is None:
-                inputs = {k: v for k, v in self._static.items() if k not in ("preds", "correct")}
-                second = {k: torch.empty_like(v) for k, v in inputs.items()}
-                for k, v in inputs.items():
+            first = self.statics[0]
+            if self.capacity is None:
+                second = {k: torch.empty_like(v) for k, v in first.items()}
+                for k, v in first.items():
                     second[k].copy_(v)  # valid contents for the capture below (capturing runs nothing)
             else:
                 second = self._capacity_set()  # word / page_off / edge_off are views of meta: allocate, do not clone
                 for k in ("src", "dst", "weight", "feat", "label", "meta"):
-                    second[k].copy_(self._static[k])
-                self._set_rows[1] = self._set_rows[0]
-            self._loaded_layout[1] = self._loaded_layout[0]
-            pool = (self._graph[0] if isinstance(self._graph, tuple) else self._graph).pool()
-            self._statics = [self._static, second]
-            self._graphs = [self._graph, self._capture_over(second, pool=pool)]
-            self._stage_sets = self._statics
+                    second[k].copy_(first[k])
+                self.rows[1] = self.rows[0]
+            self.loaded_layout[1] = self.loaded_layout[0]
+            pool = (self.graphs[0][0] if isinstance(self.graphs[0], tuple) else self.graphs[0]).pool()
+            self.statics.append(second)
+            self.graphs.append(self._capture_over(1, pool=pool))
+            self.stage_sets = self.statics
             self._stage_ready = [torch.cuda.Event(), torch.cuda.Event()]
             self._stage_free = [torch.cuda.Event(), torch.cuda.Event()]
             self._stage_w = self._stage_r = 0
@@ -703,28 +788,83 @@ class SageTrainer:
             raise GteError("prefetch_batch: both input sets hold unconsumed batches; call replay_prefetched() first")
         i = self._stage_w % 2
         cs = self._copy_stream
-        cs.wait_event(self._stage_free[i])  # the step that last read input set i has finished
+        cs.wait_event(self._stage_free[i])  # the pass that last read input set i has finished
         with torch.cuda.stream(cs):
-            self._copy_inputs(self._statics[i], i, host_batch, layout)
+            self._copy_inputs(i, host_batch, layout)
             self._stage_ready[i].record(cs)
         self._stage_w += 1
 
-    def replay_set(self, which: int) -> torch.Tensor:
-        """Run one captured step on static input set ``which`` (0 or 1) as it is: inputs resident in HBM, no copy.
-        The sets are filled by ``prefetch_batch`` / ``load_batch``; the caller keeps track of what is in them."""
-        if getattr(self, "_stage_sets", None) is None and which != 0:
+    def replay_set(self, which: int):
+        if self.stage_sets is None and which != 0:
             raise GteError("replay_set: the second input set exists after the first prefetch_batch()")
-        self._replay_graphs(which)
-        return self._outputs(which)
+        self.replay(which)
 
-    def replay_prefetched(self):
-        """Run one captured step on the oldest prefetched batch."""
-        if getattr(self, "_stage_sets", None) is None or self._stage_r >= self._stage_w:
+    def replay_prefetched(self) -> int:
+        """Run the pass on the oldest prefetched batch; returns the input set it read."""
+        if self.stage_sets is None or self._stage_r >= self._stage_w:
             raise GteError("replay_prefetched: no prefetched batch")
         i = self._stage_r % 2
         cur = torch.cuda.current_stream(self.device)
         cur.wait_event(self._stage_ready[i])
-        self._replay_graphs(i)
+        self.replay(i)
         self._stage_free[i].record(cur)
         self._stage_r += 1
-        return self._outputs(i)
+        return i
+
+
+class EvalCapture:
+    """A captured evaluation pass (``SageTrainer.capture_eval``): forward without dropout + gte_eval_accumulate into
+    one float64 device buffer ``totals`` = [sum w*nll, sum w, confusion counts C x C (rows: true class, columns:
+    prediction)].  Replays ADD to the totals, so one ``reset()`` per epoch followed by replays over the validation
+    batches sums the epoch; ``result()`` reads it.  Feed batches as for the captured train step: ``load_batch`` +
+    ``replay()`` or ``prefetch_batch`` + ``replay_prefetched()``; a batch that does not ``fits()`` goes to ``run(g)``.
+
+    Data parallel: every rank evaluates its own shard; ``all_reduce(totals, SUM)`` once per epoch before
+    ``result()`` gives the global numbers."""
+
+    def __init__(self, trainer: SageTrainer, host_batch: Dict[str, torch.Tensor], capacity: Optional[BatchCapacity]):
+        self._trainer = trainer
+        self.num_classes = trainer.num_classes
+        self.totals = trainer.eval_totals()
+        totals = self.totals
+        self._pass = _CapturedPass(trainer.device, host_batch, capacity,
+                                   lambda g, labels: trainer._eval_impl(g, labels, totals))
+        self.reset()  # the warm-up passes accumulated into the totals
+
+    def fits(self, host_batch: Dict[str, torch.Tensor]) -> bool:
+        """True when ``host_batch`` can run through the captured pass; route one that does not to ``run``."""
+        return self._pass.fits(host_batch)
+
+    def load_batch(self, host_batch: Dict[str, torch.Tensor]):
+        """Copy a host batch into the pass's static input set 0 (refused with a GteError before anything is copied
+        when it does not fit)."""
+        self._pass.load_batch(host_batch)
+
+    def prefetch_batch(self, host_batch: Dict[str, torch.Tensor]):
+        """Start the H2D copy of the next batch on a side stream (two input sets alternate, as for the train step)."""
+        self._pass.prefetch_batch(host_batch)
+
+    def replay(self) -> torch.Tensor:
+        """Evaluate the batch in input set 0 (a resident batch needs no copy); returns ``totals``."""
+        self._pass.replay(0)
+        return self.totals
+
+    def replay_prefetched(self) -> torch.Tensor:
+        """Evaluate the oldest prefetched batch; returns ``totals``."""
+        self._pass.replay_prefetched()
+        return self.totals
+
+    def run(self, g: PageGraphBatch, labels: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Eager evaluation of a batch into the same totals (for batches that do not fit the capture)."""
+        return self._trainer.evaluate(g, labels, totals=self.totals)
+
+    def reset(self):
+        """Zero the totals (once per epoch)."""
+        self.totals.zero_()
+
+    def result(self) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """Device tensors (loss = sum w*nll / sum w, accuracy = trace / sum of counts, cm int64 [C, C]) of the
+        totals.  ``metrics.precision_recall_f1(cm)`` gives the per-class scores."""
+        t = self.totals
+        cm = t[2:].view(self.num_classes, self.num_classes).to(torch.int64)
+        return t[0] / t[1], cm.trace().to(torch.float64) / cm.sum(), cm

@@ -835,6 +835,24 @@ def cross_entropy_fwd(logits, labels, class_w=None, stats=None):
     return stats
 
 
+def eval_accumulate(logits, labels, class_w, totals):
+    """Add one batch's validation statistics to ``totals`` (float64 [2 + C*C], device; gte_eval_accumulate):
+    [0] += sum w[y]*nll, [1] += sum w[y], [2 + y*C + argmax] += 1 over the rows with a label in [0, C)."""
+    lp, ld, c = _mat(logits, "eval.logits")
+    n = logits.shape[0]
+    yp, ydt = _labels(labels)
+    if labels.numel() != n:
+        raise GteError("eval_accumulate: labels/logits row mismatch")
+    tp = _vec(totals, "eval.totals", torch.float64)
+    if totals.numel() != 2 + c * c:
+        raise GteError(f"eval_accumulate: totals has {totals.numel()} elements, expected 2 + {c}*{c}")
+    l = lib()
+    ws = workspace(l.gte_eval_workspace_bytes(n), logits.device)
+    check(l.gte_eval_accumulate(lp, ld, yp, ydt, _vec(class_w, "class_w", n=c), n, c, tp, ws.data_ptr(), ws.numel(),
+                                _stream()), "gte_eval_accumulate")
+    return totals
+
+
 def cross_entropy_bwd_comb(logits, labels, class_w, denominator, width: int = COMB_LD):
     """d logits written in place as the self block of a fresh combined [n, 32] operand (other columns zero).
     ``width`` (tests): any multiple of 4 >= c gives an [n, width] matrix with columns [c, width) zeroed."""

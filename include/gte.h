@@ -459,6 +459,21 @@ int gte_cross_entropy_bwd(const float* logits, int64_t ld, const void* labels, i
 int gte_cross_entropy_bwd_padded(const float* logits, int64_t ld, const void* labels, int label_dtype,
                                  const float* class_w, int32_t n, int32_t c, const float* denominator,
                                  float* dlogits, int64_t lddl, int32_t zero_to, gte_stream_t stream);
+/*
+ * Validation statistics of one batch, ADDED to a float64 buffer totals[2 + c*c] (the validation step of
+ * model_train.py:349-364 and the confusion matrix of model_predict.py:159-169):
+ *   totals[0] += sum_i w[y_i] * nll_i and totals[1] += sum_i w[y_i]  (log-sum-exp and class weights of
+ *                gte_cross_entropy_fwd; the validation loss is totals[0] / totals[1]),
+ *   totals[2 + y_i*c + p_i] += 1  (confusion matrix: rows are true classes, columns predictions), p_i = torch.argmax
+ *                of row i: the first maximal index, NaN counting as maximal (as gte_page_predictions).
+ * Rows whose label lies outside [0, c) -- the -1 padding of gte_pad_batch -- are skipped.  c <= GTE_EVAL_MAX_CLASSES.
+ * Deterministic: the counts are exact integer sums, the loss partials are reduced in a fixed order and added in
+ * double.  n == 0 is a no-op.  Two launches.
+ */
+#define GTE_EVAL_MAX_CLASSES 64
+size_t gte_eval_workspace_bytes(int32_t n);
+int gte_eval_accumulate(const float* logits, int64_t ld, const void* labels, int label_dtype, const float* class_w,
+                        int32_t n, int32_t c, double* totals, void* ws, size_t ws_bytes, gte_stream_t stream);
 /* Self block of a combined [n, 32] operand (see the *_comb entries): out[r, 0:w] = x[r, 0:w] (x rows may be
  * unaligned, e.g. the raw [N, 13] BBOX features), every other column of the 32 zero; w <= 16. */
 int gte_comb_fill(const float* x, int64_t ldx, int32_t w, float* out, int64_t ldo, int64_t n,
