@@ -6,6 +6,8 @@ Public surface (mirrors /root/reference/src/components/graphs/models.py):
     PageGraphBatch, as_page_graph_batch                      -- the graph argument
     SageTrainer                                              -- fused train / inference step
     BatchCapacity                                            -- largest batch a capacity-captured step accepts
+    PagePool                                                 -- a dataset's pages resident on the device; captured
+                                                                passes gather their batches from it (plan_epoch)
     features.bbox_features                                   -- the 13 BBOX node features on the device
     CrossEntropyLoss, cross_entropy                          -- loss on the CUDA kernels
     metrics.precision_recall_f1                              -- per-class scores of an evaluation's confusion matrix
@@ -20,11 +22,12 @@ from .graph import PageGraphBatch, as_page_graph_batch, batch_pages_host  # noqa
 from .nn import CrossEntropyLoss, GcnSAGE, GcnSAGELayer, MeanSAGE, WeightedMeanSAGELayer  # noqa: F401
 from .layers import cross_entropy  # noqa: F401
 from .engine import BatchCapacity, EvalCapture, SageTrainer  # noqa: F401
+from .pool import PagePool  # noqa: F401
 from . import features, metrics, ops, synth  # noqa: F401
 from .metrics import precision_recall_f1  # noqa: F401
 
 __all__ = [
     "GcnSAGELayer", "GcnSAGE", "WeightedMeanSAGELayer", "MeanSAGE", "CrossEntropyLoss", "cross_entropy",
-    "PageGraphBatch", "as_page_graph_batch", "batch_pages_host", "SageTrainer", "BatchCapacity", "EvalCapture", "ops",
-    "synth", "metrics", "precision_recall_f1", "GteError", "lib",
+    "PageGraphBatch", "as_page_graph_batch", "batch_pages_host", "SageTrainer", "BatchCapacity", "EvalCapture",
+    "PagePool", "ops", "synth", "metrics", "precision_recall_f1", "GteError", "lib",
 ]

@@ -87,6 +87,8 @@ SIGNATURES = {
     "gte_build_page_formats_smem_bytes": (sz, [i32, i32]),
     "gte_build_page_formats": (ci, [vp, vp, vp, vp, vp, i32, i32, i64, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
     "gte_pad_batch": (ci, [vp, i32, i64, i32, vp, vp, vp, vp, vp, vp, i64, i32, vp, vp, vp]),
+    "gte_gather_plan": (ci, [vp, vp, vp, i32, i32, i64, i32, i32, i32, i32, i64, i32, vp, vp]),
+    "gte_gather_pages": (ci, [vp, vp, i32, i64, i32, i32, vp, vp, i32, vp, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp, vp]),
     "gte_bbox_features": (ci, [vp, vp, i32, vp, i64, vp]),
     "gte_adam_step": (ci, [vp, vp, vp, vp, i64, f32, f32, f32, f32, f32, i64, vp, f32, vp, vp]),
     "gte_dp_allreduce_adam": (ci, [vp, vp, i32, i32, i64, i64, vp, vp, vp, vp, f32, f32, f32, f32, f32, vp, vp, vp]),

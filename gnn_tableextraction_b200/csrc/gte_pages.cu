@@ -403,3 +403,286 @@ extern "C" int gte_pad_batch(const int32_t* word, int32_t n_cap, int64_t e_cap, 
   GTE_CHECK_LAUNCH("k_pad_batch");
   return GTE_OK;
 }
+
+// ---------------------------------------------------------------------------------------------------
+// Batches gathered from a device-resident page pool (the first kernels of a resident capacity-captured pass).
+// The reference builds every training batch on the host (`dgl.batch(train_batch).to(device)`,
+// /root/reference/src/models/model_train.py:279-297) and every predict batch the same way (model_predict.py:130-154);
+// here the pages stay in HBM (PagePool) and the captured pass itself assembles the next batch of an epoch plan:
+//   k_gather_plan   : one CTA; reads the plan cursor, checks the batch against the capacity and writes the static
+//                     set's `meta` = (n, e, P, start | padded page table) -- what the host uploads for a host-fed batch;
+//   k_gather_pages  : copies the batch's pages (features, labels, weights, page-local src / dst + node offset) into the
+//                     real prefix of the static set; gte_pad_batch then pads it as for a host-fed batch.
+// Plan layout (int32): [cursor, flag, nfit, B, L, 0, 0, 0 | ids[L] | starts[nfit]]: slice k of the plan is
+// ids[starts[k], min(starts[k] + B, L)).
+namespace gte {
+
+constexpr int PLAN_HDR = 8;
+constexpr int PLAN_THREADS = 1024;
+constexpr int GATHER_THREADS = 256;
+
+struct GatherCap {
+  int32_t nodes, pages, page_nodes, page_edges;
+  int64_t edges;
+  int32_t n_cap, e_cap, p_cap;
+};
+
+// inclusive block scan of two int32 values (PLAN_THREADS threads); returns the block totals in tot[2]
+__device__ __forceinline__ void block_scan2(int32_t& a, int32_t& b, int32_t* warp_a, int32_t* warp_b, int32_t* tot) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int32_t ta = __shfl_up_sync(0xffffffffu, a, o), tb = __shfl_up_sync(0xffffffffu, b, o);
+    if (lane >= o) {
+      a += ta;
+      b += tb;
+    }
+  }
+  if (lane == 31) {
+    warp_a[w] = a;
+    warp_b[w] = b;
+  }
+  __syncthreads();
+  if (w == 0) {
+    int32_t xa = lane < PLAN_THREADS / 32 ? warp_a[lane] : 0, xb = lane < PLAN_THREADS / 32 ? warp_b[lane] : 0;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int32_t ta = __shfl_up_sync(0xffffffffu, xa, o), tb = __shfl_up_sync(0xffffffffu, xb, o);
+      if (lane >= o) {
+        xa += ta;
+        xb += tb;
+      }
+    }
+    warp_a[lane] = xa;  // inclusive warp prefixes
+    warp_b[lane] = xb;
+    if (lane == 31) {
+      tot[0] = xa;
+      tot[1] = xb;
+    }
+  }
+  __syncthreads();
+  if (w > 0) {
+    a += warp_a[w - 1];
+    b += warp_b[w - 1];
+  }
+  __syncthreads();
+}
+
+__global__ void __launch_bounds__(PLAN_THREADS)
+    k_gather_plan(int32_t* __restrict__ plan, const int32_t* __restrict__ pool_n, const int32_t* __restrict__ pool_e,
+                  int32_t pool_pages, GatherCap cap, int32_t* __restrict__ meta) {
+  __shared__ int32_t hdr[3];  // start, P, status
+  __shared__ unsigned long long s_n, s_e;
+  __shared__ int32_t s_mn, s_me, s_badid;
+  __shared__ int32_t warp_a[PLAN_THREADS / 32], warp_b[PLAN_THREADS / 32], tot[2];
+  const int tid = threadIdx.x;
+  if (tid == 0) {
+    const int32_t cur = plan[0], nfit = plan[2], b = plan[3], l = plan[4];
+    int32_t status = 0, start = 0, p = 0;
+    if (cur < 0 || cur >= nfit || b < 1 || l < 1 || l > pool_pages || nfit > l) {  // reads stay in 8 + 2 * pool_pages words
+      status = 1;
+    } else {
+      start = plan[PLAN_HDR + l + cur];
+      if (start < 0 || start >= l) status = 1;
+      else p = min(b, l - start);
+    }
+    if (status == 0 && p > cap.pages) status = 2;
+    hdr[0] = start;
+    hdr[1] = p;
+    hdr[2] = status;
+    s_n = s_e = 0ull;
+    s_mn = s_me = 0;
+    s_badid = 0;
+    plan[0] = cur + 1;  // one planned batch per launch
+    if (status) atomicOr(plan + 1, status);
+  }
+  __syncthreads();
+  if (hdr[2]) return;
+  const int32_t start = hdr[0], p = hdr[1];
+  const int32_t* ids = plan + PLAN_HDR + start;
+  // 1. totals and largest page of the batch: nothing is written before it is known to fit
+  unsigned long long ln = 0, le = 0;
+  int32_t mn = 0, me = 0;
+  for (int j = tid; j < p; j += PLAN_THREADS) {
+    const int32_t id = ids[j];
+    if (id < 0 || id >= pool_pages) {
+      s_badid = 1;
+      continue;
+    }
+    const int32_t a = pool_n[id], b = pool_e[id];
+    ln += (unsigned long long)max(a, 0);
+    le += (unsigned long long)max(b, 0);
+    mn = max(mn, a);
+    me = max(me, b);
+  }
+  atomicAdd(&s_n, ln);
+  atomicAdd(&s_e, le);
+  atomicMax(&s_mn, mn);
+  atomicMax(&s_me, me);
+  __syncthreads();
+  const int64_t n64 = (int64_t)s_n, e64 = (int64_t)s_e;
+  // BatchCapacity.check: pages, nodes, edges, largest page
+  if (s_badid || n64 > cap.nodes || e64 > cap.edges || s_mn > cap.page_nodes || s_me > cap.page_edges) {
+    if (tid == 0) atomicOr(plan + 1, 2);
+    return;
+  }
+  const int32_t n = (int32_t)n64, e = (int32_t)e64;
+  int32_t* po = meta + 4;
+  int32_t* eo = meta + 5 + cap.p_cap;
+  // 2. offsets of the real pages
+  int32_t carry_n = 0, carry_e = 0;
+  for (int base = 0; base < p; base += PLAN_THREADS) {
+    const int j = base + tid;
+    int32_t a = 0, b = 0;
+    if (j < p) {
+      const int32_t id = ids[j];
+      a = pool_n[id];
+      b = pool_e[id];
+    }
+    block_scan2(a, b, warp_a, warp_b, tot);
+    if (j < p) {
+      po[j + 1] = carry_n + a;
+      eo[j + 1] = carry_e + b;
+    }
+    carry_n += tot[0];
+    carry_e += tot[1];
+    __syncthreads();
+  }
+  // 3. padding pages and empty pages, as engine.padded_page_table
+  const int32_t s = min(cap.p_cap - p, cap.n_cap - n);
+  for (int j = p + 1 + tid; j <= cap.p_cap; j += PLAN_THREADS) {
+    const int64_t k = j - p;  // 1-based padding slot
+    if (k <= s) {
+      po[j] = (int32_t)(n + k * (int64_t)(cap.n_cap - n) / s);
+      eo[j] = (int32_t)(e + k * (int64_t)(cap.e_cap - e) / s);
+    } else {
+      po[j] = cap.n_cap;
+      eo[j] = cap.e_cap;
+    }
+  }
+  if (tid == 0) {
+    po[0] = 0;
+    eo[0] = 0;
+    meta[0] = n;
+    meta[1] = e;
+    meta[2] = p;
+    meta[3] = start;
+  }
+}
+
+// dst[i] = src[i] + add over `count` 32-bit words; float4 / int4 accesses where both sides share their 16-byte phase
+template <typename T>
+__device__ __forceinline__ void copy_words(T* __restrict__ dst, const T* __restrict__ src, int64_t count, int32_t add) {
+  static_assert(sizeof(T) == 4, "32-bit words");
+  int64_t head = 0;
+  const bool vec = ((reinterpret_cast<uintptr_t>(dst) ^ reinterpret_cast<uintptr_t>(src)) & 15u) == 0;
+  if (vec) {
+    head = (int64_t)(((16u - (reinterpret_cast<uintptr_t>(dst) & 15u)) & 15u) >> 2);
+    if (head > count) head = count;
+    const int64_t nv = (count - head) >> 2;
+    const int4* s4 = reinterpret_cast<const int4*>(src + head);
+    int4* d4 = reinterpret_cast<int4*>(dst + head);
+    for (int64_t k = threadIdx.x; k < nv; k += blockDim.x) {
+      int4 v = __ldg(s4 + k);
+      if (add) {
+        v.x += add;
+        v.y += add;
+        v.z += add;
+        v.w += add;
+      }
+      d4[k] = v;
+    }
+    for (int64_t k = head + 4 * nv + threadIdx.x; k < count; k += blockDim.x) {
+      if (add) dst[k] = (T)(__ldg(src + k) + add);
+      else dst[k] = __ldg(src + k);
+    }
+    if (threadIdx.x < head) {
+      if (add) dst[threadIdx.x] = (T)(__ldg(src + threadIdx.x) + add);
+      else dst[threadIdx.x] = __ldg(src + threadIdx.x);
+    }
+    return;
+  }
+  for (int64_t k = threadIdx.x; k < count; k += blockDim.x) {
+    if (add) dst[k] = (T)(__ldg(src + k) + add);
+    else dst[k] = __ldg(src + k);
+  }
+}
+
+__global__ void __launch_bounds__(GATHER_THREADS)
+    k_gather_pages(int32_t* __restrict__ plan, const int32_t* __restrict__ meta, int32_t n_cap, int32_t e_cap,
+                   int32_t p_cap, const int64_t* __restrict__ pool_node_off, const int64_t* __restrict__ pool_edge_off,
+                   int32_t pool_pages, const int32_t* __restrict__ pool_src, const int32_t* __restrict__ pool_dst,
+                   const float* __restrict__ pool_w, const float* __restrict__ pool_feat,
+                   const float* __restrict__ pool_label, int32_t f, int32_t* __restrict__ src, int32_t* __restrict__ dst,
+                   float* __restrict__ w, float* __restrict__ feat, float* __restrict__ label) {
+  // a flagged plan (the plan kernel refused this batch, so meta still describes an earlier one): copy nothing
+  if (plan[1] != 0) return;
+  const int32_t p = meta[2], start = meta[3], l = plan[4];
+  if (p < 0 || p > p_cap || start < 0 || l > pool_pages || (int64_t)start + p > l) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) atomicOr(plan + 1, 4);
+    return;
+  }
+  const int32_t* ids = plan + PLAN_HDR + start;
+  const int32_t* po = meta + 4;
+  const int32_t* eo = meta + 5 + p_cap;
+  for (int32_t j = blockIdx.x; j < p; j += gridDim.x) {
+    const int32_t id = ids[j];
+    const int32_t nb = po[j], ni = po[j + 1] - nb, eb = eo[j], ei = eo[j + 1] - eb;
+    // the page table must describe exactly these pool pages (it does unless the plan buffer was rewritten after
+    // k_gather_plan ran): otherwise skip the page and flag, never copy out of bounds
+    bool ok = id >= 0 && id < pool_pages && nb >= 0 && ni >= 0 && (int64_t)nb + ni <= n_cap && eb >= 0 && ei >= 0 &&
+              (int64_t)eb + ei <= e_cap;
+    int64_t pn = 0, pe = 0;
+    if (ok) {
+      pn = pool_node_off[id];
+      pe = pool_edge_off[id];
+      ok = pool_node_off[id + 1] - pn == ni && pool_edge_off[id + 1] - pe == ei;
+    }
+    if (!ok) {
+      if (threadIdx.x == 0) atomicOr(plan + 1, 4);
+      continue;
+    }
+    copy_words(feat + (int64_t)nb * f, pool_feat + pn * f, (int64_t)ni * f, 0);
+    copy_words(label + nb, pool_label + pn, ni, 0);
+    copy_words(w + eb, pool_w + pe, ei, 0);
+    copy_words(src + eb, pool_src + pe, ei, nb);
+    copy_words(dst + eb, pool_dst + pe, ei, nb);
+  }
+}
+
+}  // namespace gte
+
+extern "C" int gte_gather_plan(int32_t* plan, const int32_t* pool_num_nodes, const int32_t* pool_num_edges,
+                               int32_t pool_pages, int32_t cap_nodes, int64_t cap_edges, int32_t cap_pages,
+                               int32_t cap_page_nodes, int32_t cap_page_edges, int32_t n_cap, int64_t e_cap, int32_t p_cap,
+                               int32_t* meta, gte_stream_t stream) {
+  GTE_CHECK_ARG(plan && pool_num_nodes && pool_num_edges && meta, "gte_gather_plan: null argument");
+  GTE_CHECK_ARG(pool_pages > 0 && cap_nodes > 0 && cap_edges >= 0 && cap_pages > 0 && cap_page_nodes > 0 &&
+                    cap_page_edges > 0, "gte_gather_plan: bad pool or capacity");
+  GTE_CHECK_ARG(n_cap > cap_nodes && e_cap >= cap_edges && e_cap < ((int64_t)1 << 31) && p_cap > cap_pages,
+                "gte_gather_plan: padded shape below the capacity");
+  GatherCap cap{cap_nodes, cap_pages, cap_page_nodes, cap_page_edges, cap_edges, n_cap, (int32_t)e_cap, p_cap};
+  k_gather_plan<<<1, PLAN_THREADS, 0, as_stream(stream)>>>(plan, pool_num_nodes, pool_num_edges, pool_pages, cap, meta);
+  GTE_CHECK_LAUNCH("k_gather_plan");
+  return GTE_OK;
+}
+
+extern "C" int gte_gather_pages(int32_t* plan, const int32_t* meta, int32_t n_cap, int64_t e_cap, int32_t p_cap,
+                                int32_t max_pages, const int64_t* pool_node_off, const int64_t* pool_edge_off,
+                                int32_t pool_pages, const int32_t* pool_src, const int32_t* pool_dst,
+                                const float* pool_weight, const float* pool_feat, const float* pool_label, int32_t f,
+                                int32_t* src, int32_t* dst, float* weight, float* feat, float* label,
+                                gte_stream_t stream) {
+  GTE_CHECK_ARG(plan && meta && pool_node_off && pool_edge_off && pool_feat && pool_label && feat && label,
+                "gte_gather_pages: null argument");
+  GTE_CHECK_ARG(e_cap == 0 || (src && dst && weight), "gte_gather_pages: null edge argument");
+  GTE_CHECK_ARG(pool_pages > 0 && f > 0 && n_cap > 0 && e_cap >= 0 && e_cap < ((int64_t)1 << 31) && p_cap > 0 &&
+                    max_pages > 0 && max_pages <= p_cap, "gte_gather_pages: bad size");
+  int64_t blocks = 4 * (int64_t)sm_count();
+  if (blocks > max_pages) blocks = max_pages;
+  k_gather_pages<<<(unsigned)blocks, GATHER_THREADS, 0, as_stream(stream)>>>(
+      plan, meta, n_cap, (int32_t)e_cap, p_cap, pool_node_off, pool_edge_off, pool_pages, pool_src, pool_dst, pool_weight,
+      pool_feat, pool_label, f, src, dst, weight, feat, label);
+  GTE_CHECK_LAUNCH("k_gather_pages");
+  return GTE_OK;
+}

@@ -22,6 +22,7 @@ of per-rank means).
 """
 from __future__ import annotations
 
+import gc
 import os
 from dataclasses import dataclass
 from typing import Dict, List, Optional, Sequence, Tuple
@@ -35,6 +36,7 @@ from . import ops
 from ._lib import GteError
 from .graph import PageGraphBatch, page_table
 from .nn import GcnSAGE, _is_relu
+from .pool import PagePool
 
 
 def _dropout_p(d) -> float:
@@ -132,6 +134,77 @@ def padded_page_table(capacity: BatchCapacity, batch_num_nodes: Sequence[int], b
     po[p + 1:p + 1 + s] = n + j * (n_cap - n) // s
     eo[p + 1:p + 1 + s] = e + j * (e_cap - e) // s
     return po.astype(np.int32), eo.astype(np.int32)
+
+
+# ------------------------------------------------------------------ resident passes: epochs planned over a PagePool --
+@dataclass(frozen=True)
+class PlannedBatch:
+    """One slice of an epoch plan (``plan_epoch``): its page ids, whether it fits the captured capacity -- then the
+    next ``replay()`` runs it; otherwise run it eagerly on ``pool.batch(ids)`` --, and its node and page counts."""
+
+    ids: np.ndarray
+    fits: bool
+    nodes: int
+    pages: int
+
+
+def _plan_words(ids: np.ndarray, starts: np.ndarray, batch_pages: int) -> np.ndarray:
+    """int32 plan buffer contents (gte.h): [cursor 0, flag 0, nfit, B, L, 0, 0, 0 | ids | starts]"""
+    words = np.zeros(ops.PLAN_HEADER + ids.size + starts.size, dtype=np.int32)
+    words[2:5] = (starts.size, min(batch_pages, ids.size), ids.size)
+    words[ops.PLAN_HEADER:ops.PLAN_HEADER + ids.size] = ids
+    words[ops.PLAN_HEADER + ids.size:] = starts
+    return words
+
+
+def plan_slices(capacity: BatchCapacity, n_i: np.ndarray, e_i: np.ndarray, page_ids, batch_pages: int):
+    """Host side of ``plan_epoch`` over a pool with per-page node / edge counts ``n_i`` / ``e_i``: ``page_ids`` cut
+    into consecutive slices of ``batch_pages`` (the last may be short), each decided against ``capacity`` exactly as
+    ``capacity.fits`` decides (vectorised over the slices).  Returns (list of PlannedBatch, int32 plan words)."""
+    num_pages = len(n_i)
+    if isinstance(batch_pages, bool) or not isinstance(batch_pages, (int, np.integer)) or batch_pages < 1:
+        raise GteError(f"plan_epoch: batch_pages must be a positive int, got {batch_pages!r}")
+    ids = np.asarray(page_ids)
+    if ids.ndim != 1 or ids.size == 0 or not np.issubdtype(ids.dtype, np.integer):
+        raise GteError(f"plan_epoch: page_ids must be a non-empty 1-D integer sequence, got {ids.dtype} {ids.shape}")
+    if ids.size > num_pages:
+        raise GteError(f"plan_epoch: {ids.size} page ids > the pool's {num_pages} pages (the device plan holds at most "
+                       "one epoch over the pool)")
+    if int(ids.min()) < 0 or int(ids.max()) >= num_pages:
+        raise GteError(f"plan_epoch: page ids must lie in [0, {num_pages}), got [{int(ids.min())}, {int(ids.max())}]")
+    ids = ids.astype(np.int64)
+    b = int(batch_pages)
+    starts = np.arange(0, ids.size, b, dtype=np.int64)
+    pn, pe = n_i[ids], e_i[ids]
+    nodes, edges = np.add.reduceat(pn, starts), np.add.reduceat(pe, starts)
+    pages = np.minimum(b, ids.size - starts)
+    fits = ((pages <= capacity.pages) & (nodes <= capacity.nodes) & (edges <= capacity.edges)
+            & (np.maximum.reduceat(pn, starts) <= capacity.page_nodes)
+            & (np.maximum.reduceat(pe, starts) <= capacity.page_edges))
+    batches = [PlannedBatch(ids[s:s + p], bool(f), int(n), int(p)) for s, p, f, n in zip(starts, pages, fits, nodes)]
+    return batches, _plan_words(ids, starts[fits], b)
+
+
+def check_resident_capture(pool, capacity: Optional[BatchCapacity], world: int, in_feats: int) -> None:
+    """Refuse a pass captured on a PagePool that cannot run: no capacity, data parallel, a feature width other than
+    the model's input."""
+    if capacity is None:
+        raise GteError("capture: a pass on a PagePool needs a capacity (capacity=BatchCapacity(...))")
+    if world > 1:
+        raise GteError("capture: data parallel with a resident PagePool is not supported (each rank would need its own "
+                       "pool shard); feed host batches on every rank")
+    if pool.feat_width != in_feats:
+        raise GteError(f"capture: the pool's features are {pool.feat_width} wide, the model takes {in_feats}")
+
+
+def resident_warmup_ids(pool, capacity: BatchCapacity) -> np.ndarray:
+    """The pool's first pages that fit ``capacity`` together (the capture's warm-up batch): pages no larger than the
+    page caps, in pool order, as many as the page / node / edge totals allow."""
+    ok = np.flatnonzero((pool.n_i <= capacity.page_nodes) & (pool.e_i <= capacity.page_edges))[:capacity.pages]
+    k = int(np.count_nonzero((np.cumsum(pool.n_i[ok]) <= capacity.nodes) & (np.cumsum(pool.e_i[ok]) <= capacity.edges)))
+    if k == 0:
+        raise GteError("capture: no page of the pool fits the capacity")
+    return ok[:k]
 
 
 class SageTrainer:
@@ -427,13 +500,16 @@ class SageTrainer:
             self._eval_impl(g, labels, totals)
         return totals
 
-    def capture_eval(self, host_batch: Dict[str, torch.Tensor], capacity: Optional[BatchCapacity] = None) -> "EvalCapture":
+    def capture_eval(self, host_batch, capacity: Optional[BatchCapacity] = None) -> "EvalCapture":
         """Capture ``evaluate`` as a pass of its own, beside the captured train step (which stays): without a capacity
         for batches of this shape -- ``host_batch`` stays resident and ``replay()`` copies nothing, the fixed
-        validation batch of model_train.py:242-249 --, with one for every batch that fits it (see ``capture``).  The
-        pass has its own memory pool and totals buffer and reads the live parameters, so after a train replay it sees
-        the updated weights."""
+        validation batch of model_train.py:242-249 --, with one for every batch that fits it (see ``capture``), or on
+        a ``PagePool`` with a capacity (``plan_epoch`` + ``replay``, see ``capture``).  The pass has its own memory
+        pool and totals buffer and reads the live parameters, so after a train replay it sees the updated weights."""
         return EvalCapture(self, host_batch, capacity)
+
+    def _check_resident(self, pool: PagePool, capacity: Optional[BatchCapacity]):
+        check_resident_capture(pool, capacity, self.world, int(self.model.layers[0].linear.weight.shape[1]) // 2)
 
     # ----------------------------------------------------- CUDA graphs -----
     @property
@@ -449,16 +525,17 @@ class SageTrainer:
     def _graph(self):
         return None if self._train is None else self._train.graphs[0]
 
-    def capture_predict(self, host_batch: Dict[str, torch.Tensor], capacity: Optional[BatchCapacity] = None):
+    def capture_predict(self, host_batch, capacity: Optional[BatchCapacity] = None):
         """Capture the batched predict pass of model_predict.py:130-154 (format build + forward without saved
         activations + argmax + per-page correct counts) for batches of this shape, or for every batch that fits
-        ``capacity`` (see ``capture``).  Feed batches with ``load_batch`` / ``prefetch_batch``; ``replay()`` /
-        ``replay_prefetched()`` then return ``(preds int32 [N], page_correct int32 [P])`` -- views of static device
-        tensors of the input set that ran, sized for the batch in it, valid until that set runs again."""
+        ``capacity`` (see ``capture``).  Feed batches with ``load_batch`` / ``prefetch_batch`` (on a ``PagePool``:
+        ``plan_epoch``); ``replay()`` / ``replay_prefetched()`` then return ``(preds int32 [N], page_correct int32
+        [P])`` -- views of static device tensors of the input set that ran, sized for the batch in it, valid until
+        that set runs again."""
         return self.capture(host_batch, capacity=capacity, split=False, mode="predict")
 
-    def capture(self, host_batch: Dict[str, torch.Tensor], capacity: Optional[BatchCapacity] = None,
-                split: Optional[bool] = None, mode: str = "train"):
+    def capture(self, host_batch, capacity: Optional[BatchCapacity] = None, split: Optional[bool] = None,
+                mode: str = "train"):
         """Capture the whole step (format build + forward + loss + backward +
         optimiser) for batches with exactly this node / edge count.  Later
         batches are fed with ``load_batch`` + ``replay``.  ``split`` (default: data-parallel
@@ -470,12 +547,20 @@ class SageTrainer:
         weight-0 self-loops in pages of their own, which change no loss statistic and no gradient.  ``host_batch``
         must fit; it gives the feature width and the warm-up contents.
 
+        ``host_batch`` may be a ``PagePool`` instead (``capacity`` required, one GPU): the pass then gathers its
+        batches from the pool on the device -- its first kernels plan the next batch of an epoch plan and copy its
+        pages into the static inputs --, so an epoch costs one upload of page ids (``plan_epoch``) and one
+        ``replay()`` per fitting batch, with no host batching and no per-batch copy.  The warm-up runs on the pool's
+        first pages that fit.
+
         A trainer holds one captured step: a new capture replaces the previous one.  A pass captured by
         ``capture_eval`` is separate and stays."""
         if split is None:
             split = self.world > 1 and self._dp_peer is None  # the peer-memory exchange is an ordinary kernel: one graph
         if mode not in ("train", "predict"):
             raise GteError(f"capture: unknown mode {mode}")
+        if isinstance(host_batch, PagePool):
+            self._check_resident(host_batch, capacity)
         if mode == "predict":
             body, tail = self._predict_impl, None
         elif split:  # [graph: batch assembly + forward + CE + backward] -> ONE all-reduce -> Adam (eager, 2 launches)
@@ -502,6 +587,14 @@ class SageTrainer:
         Route a batch that does not fit to ``train_step`` / ``predict_pages``."""
         return self._captured("fits").fits(host_batch)
 
+    def plan_epoch(self, page_ids, batch_pages: int) -> List[PlannedBatch]:
+        """Plan an epoch of a step captured on a ``PagePool``: ``page_ids`` (at most ``pool.num_pages`` ids, in the
+        caller's order -- e.g. a permutation, trimmed by a loop that drops the last short batch) is cut into
+        consecutive batches of ``batch_pages`` pages, the last possibly short.  One copy uploads the ids and the
+        batches that fit the capacity; every later ``replay()`` runs the next of them.  Returns the batches in
+        order; run one that does not fit eagerly: ``train_step(pool.batch(b.ids))`` / ``predict_pages(...)``."""
+        return self._captured("plan_epoch").plan_epoch(page_ids, batch_pages)
+
     def load_batch(self, host_batch: Dict[str, torch.Tensor]):
         """Copy a host batch into static input set 0.  The batch must have the captured node / edge totals and page
         count and no page larger than the captured maxima; page ORDER and SIZES may differ (the page table is
@@ -519,7 +612,9 @@ class SageTrainer:
         return self._result()
 
     def replay(self):
-        self._captured("replay").replay(0)
+        """Run the captured step on input set 0 -- on a ``PagePool``: on the next planned batch that fits --; returns
+        the statistics (train) or ``(preds, page_correct)`` of the batch (predict)."""
+        self._captured("replay").replay_next()
         return self._outputs(0)
 
     def prefetch_batch(self, host_batch: Dict[str, torch.Tensor]):
@@ -546,10 +641,19 @@ class _CapturedPass:
     the static inputs of the batch shape or of a ``BatchCapacity`` (padded on the device by gte_pad_batch, the first
     kernel of the graph), the validation and page layout of a fed batch, its host->device copies and the two-set
     prefetch pipeline.  ``outs[i]`` keeps what ``body`` returned while capturing over input set i.  ``tail`` (may be
-    None) runs eagerly after every replay: the data-parallel all-reduce + Adam of a split train step."""
+    None) runs eagerly after every replay: the data-parallel all-reduce + Adam of a split train step.
 
-    def __init__(self, device, host_batch: Dict[str, torch.Tensor], capacity: Optional[BatchCapacity], body, tail=None):
-        if capacity is not None:
+    Captured on a ``PagePool`` (a resident pass; capacity capture with one input set), the graph starts with
+    gte_gather_plan + gte_gather_pages, which assemble the next batch of the device epoch plan ``plan`` from the pool;
+    the host keeps the same plan's (n, P) per fitting batch to cut the outputs and to refuse a replay past it."""
+
+    def __init__(self, device, source, capacity: Optional[BatchCapacity], body, tail=None):
+        self.pool = source if isinstance(source, PagePool) else None
+        host_batch = None if self.pool is not None else source
+        if self.pool is not None:
+            self._check_capacity(capacity, None)
+            warm = resident_warmup_ids(self.pool, capacity)
+        elif capacity is not None:
             self._check_capacity(capacity, host_batch)
         self.device, self.capacity, self.body, self.tail = device, capacity, body, tail
         dev = device
@@ -577,33 +681,53 @@ class _CapturedPass:
                 self.caps = None
         else:
             n_cap, e_cap, p_cap = capacity.shape
-            self.feat_width = int(host_batch["feat"].shape[1])
+            if self.pool is not None:
+                self.feat_width = self.pool.feat_width
+                bn, be = self.pool.n_i[warm], self.pool.e_i[warm]
+            else:
+                self.feat_width = int(host_batch["feat"].shape[1])
+                bn, be = host_batch["batch_num_nodes"], host_batch["batch_num_edges"]
             st = self._capacity_set()
             # the structure the captured kernels see: P_cap pages, none larger than the capacity's page caps (the
             # page lists only size the batch; the offsets come from st["page_off"] / st["edge_off"] every replay)
-            po, eo = padded_page_table(capacity, host_batch["batch_num_nodes"], host_batch["batch_num_edges"])
+            po, eo = padded_page_table(capacity, bn, be)
             self.meta = (n_cap, e_cap, np.diff(po).tolist(), np.diff(eo).tolist())
             self.caps = (p_cap, capacity.page_nodes, capacity.page_edges)
         self.rows = [None, None]  # capacity capture: (n, P) of the batch in each input set
         self.loaded_layout = [None, None]
         self.statics = [st]
         self.stage_sets = None
-        self.load_batch(host_batch)
+        if self.pool is None:
+            self.load_batch(host_batch)
+        else:
+            # the device plan holds one epoch over the pool: its pointer is captured, so it is sized once, here
+            self.plan = torch.zeros(ops.PLAN_HEADER + 2 * self.pool.num_pages, dtype=torch.int32, device=dev)
+            # a plan of the one warm-up batch (nfit = 1 <= L = len(warm) for any warm-up, as the plan kernel requires),
+            # uploaded again before each warm-up run
+            warm_words = _plan_words(warm, np.zeros(1, dtype=np.int64), len(warm))
 
         # warm-up on a side stream (allocator + lazy module state)
         s = torch.cuda.Stream(device=dev)
         s.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(s):
             for _ in range(2):
-                self._pad(st)
-                body(self.graph_of(st), st["label"])
-                if tail is not None:
-                    tail()
+                if self.pool is not None:
+                    self._upload_plan(warm_words)
+                self.run_eager(st)
         torch.cuda.current_stream(dev).wait_stream(s)
         torch.cuda.synchronize(dev)
         self._check_static_structure(st)
         self.outs = [None, None]
         self.graphs = [self._capture_over(0)]
+        self._plan_rows, self._plan_next, self._plan_checked = [], 0, True  # no epoch planned yet
+
+    def run_eager(self, st):
+        """the captured pass over static input set ``st``, launched eagerly (warm-up)"""
+        self._pad(st)
+        out = self.body(self.graph_of(st), st["label"])
+        if self.tail is not None:
+            self.tail()
+        return out
 
     def graph_of(self, st) -> PageGraphBatch:
         n = self.meta[0]
@@ -622,6 +746,8 @@ class _CapturedPass:
             g.check_page_structure()
         if "pad_bad" in st and int(st["pad_bad"].item()) != 0:
             raise GteError("capture: gte_pad_batch flagged the padded batch (word outside the capacity or bad page table)")
+        if self.pool is not None:
+            self._check_plan_flag("capture")
 
     # -- capacity capture: one graph for every batch that fits a BatchCapacity ------------------------------------
     @classmethod
@@ -632,7 +758,8 @@ class _CapturedPass:
         if not ops.page_formats_supported((None, p_cap, capacity.page_nodes, capacity.page_edges)):
             raise GteError(f"capture: pages of {capacity.page_nodes} nodes / {capacity.page_edges} edges do not fit the "
                            "one-kernel batch assembly (shared memory); lower page_nodes / page_edges")
-        cls._check_fit(capacity, host_batch, int(host_batch["feat"].shape[1]))
+        if host_batch is not None:
+            cls._check_fit(capacity, host_batch, int(host_batch["feat"].shape[1]))
 
     @staticmethod
     def _check_fit(capacity: BatchCapacity, host_batch, f: int):
@@ -664,12 +791,60 @@ class _CapturedPass:
         }
 
     def _pad(self, st):
-        """first kernel of a capacity-captured pass: pad the batch in ``st`` to the capacity shape"""
+        """first kernels of a capacity-captured pass: (resident: plan the next batch and gather it from the pool,) pad
+        the batch in ``st`` to the capacity shape"""
+        if self.pool is not None:
+            pool = self.pool
+            ops.gather_plan(self.plan, pool.n_dev, pool.e_dev, self.capacity, st["meta"])
+            ops.gather_pages(self.plan, st["meta"], self.capacity, pool.node_off, pool.edge_off, pool.coo[0], pool.coo[1],
+                             pool.w_coo, pool.feat, pool.label, st["src"], st["dst"], st["weight"], st["feat"],
+                             st["label"])
         if self.capacity is not None:
             ops.pad_batch(st["word"], st["page_off"], st["edge_off"], st["src"], st["dst"], st["weight"], st["feat"],
                           st["label"], bad=st["pad_bad"])
 
+    # -- resident pass: batches planned over the pool, gathered on the device ------------------------------------
+    def _host_fed(self, what: str):
+        if self.pool is not None:
+            raise GteError(f"{what}: this pass gathers its batches from a PagePool; use plan_epoch() + replay()")
+
+    def _upload_plan(self, words: np.ndarray):
+        # a fresh pinned staging tensor per upload, as in _copy_inputs: a queued copy never reads a rewritten buffer
+        staging = torch.empty(words.size, dtype=torch.int32, pin_memory=True)
+        staging.numpy()[:] = words
+        self.plan[:words.size].copy_(staging, non_blocking=True)
+
+    def _check_plan_flag(self, what: str):
+        flag = int(self.plan[1].item())
+        if flag:
+            raise GteError(f"{what}: the resident pass's gather kernels flagged the plan ({flag}: 1 = past the plan, "
+                           "2 = a batch did not fit or named a page outside the pool, 4 = page table and pool disagree)")
+
+    def plan_epoch(self, page_ids, batch_pages: int) -> List[PlannedBatch]:
+        if self.pool is None:
+            raise GteError("plan_epoch: the pass was captured on a host batch; capture it on a PagePool")
+        batches, words = plan_slices(self.capacity, self.pool.n_i, self.pool.e_i, page_ids, batch_pages)
+        self._upload_plan(words)
+        self._plan_rows = [(b.nodes, b.pages) for b in batches if b.fits]
+        self._plan_next, self._plan_checked = 0, False
+        return batches
+
+    def replay_next(self):
+        """``replay()`` of the public API: input set 0, or the next planned batch of a resident pass"""
+        if self.pool is None:
+            self.replay(0)
+            return
+        if self._plan_next >= len(self._plan_rows):
+            raise GteError(f"replay: all {len(self._plan_rows)} fitting batches of the plan have run; call plan_epoch()")
+        self.rows[0] = self._plan_rows[self._plan_next]
+        self._plan_next += 1
+        self.replay(0)
+        if not self._plan_checked:  # once per plan: one host read
+            self._plan_checked = True
+            self._check_plan_flag("replay")
+
     def fits(self, host_batch: Dict[str, torch.Tensor]) -> bool:
+        self._host_fed("fits")
         try:
             self._page_layout(host_batch)
         except GteError:
@@ -741,12 +916,25 @@ class _CapturedPass:
         st = self.statics[which]
         graph = torch.cuda.CUDAGraph()
         kw = {} if pool is None else {"pool": pool}
-        with torch.cuda.graph(graph, **kw):
-            self._pad(st)
-            self.outs[which] = self.body(self.graph_of(st), st["label"])
+        # No cyclic garbage collection while capturing.  Trainers and their passes reference each other, so a discarded
+        # trainer's CUDA graphs are freed by the cyclic collector, whenever it happens to run; destroying a graph while
+        # a stream captures invalidates the capture.  torch.cuda.graph no longer runs gc.collect() before capturing
+        # (torch 2.11), and this showed up as a capture failing with cudaErrorStreamCaptureInvalidated after
+        # "operation not permitted when stream is capturing (function reset)" warnings, in a test that ran after
+        # others had dropped captured trainers.
+        gc_was_on = gc.isenabled()
+        gc.disable()
+        try:
+            with torch.cuda.graph(graph, **kw):
+                self._pad(st)
+                self.outs[which] = self.body(self.graph_of(st), st["label"])
+        finally:
+            if gc_was_on:
+                gc.enable()
         return (graph,) if self.tail is not None else graph
 
     def load_batch(self, host_batch: Dict[str, torch.Tensor]):
+        self._host_fed("load_batch")
         self._copy_inputs(0, host_batch, self._page_layout(host_batch))
 
     def replay(self, which: int = 0):
@@ -759,6 +947,7 @@ class _CapturedPass:
 
     # -- pipelined input: the host->device copy of batch i+1 overlaps the pass over batch i ----------------------
     def prefetch_batch(self, host_batch: Dict[str, torch.Tensor]):
+        self._host_fed("prefetch_batch")
         layout = self._page_layout(host_batch)
         if self.stage_sets is None:
             torch.cuda.synchronize(self.device)
@@ -795,12 +984,14 @@ class _CapturedPass:
         self._stage_w += 1
 
     def replay_set(self, which: int):
+        self._host_fed("replay_set")
         if self.stage_sets is None and which != 0:
             raise GteError("replay_set: the second input set exists after the first prefetch_batch()")
         self.replay(which)
 
     def replay_prefetched(self) -> int:
         """Run the pass on the oldest prefetched batch; returns the input set it read."""
+        self._host_fed("replay_prefetched")
         if self.stage_sets is None or self._stage_r >= self._stage_w:
             raise GteError("replay_prefetched: no prefetched batch")
         i = self._stage_r % 2
@@ -819,10 +1010,15 @@ class EvalCapture:
     batches sums the epoch; ``result()`` reads it.  Feed batches as for the captured train step: ``load_batch`` +
     ``replay()`` or ``prefetch_batch`` + ``replay_prefetched()``; a batch that does not ``fits()`` goes to ``run(g)``.
 
+    Captured on a ``PagePool`` (with a capacity): ``plan_epoch(ids, B)`` once per epoch, then ``replay()`` per
+    planned batch that fits and ``run(pool.batch(b.ids))`` for the others.
+
     Data parallel: every rank evaluates its own shard; ``all_reduce(totals, SUM)`` once per epoch before
     ``result()`` gives the global numbers."""
 
-    def __init__(self, trainer: SageTrainer, host_batch: Dict[str, torch.Tensor], capacity: Optional[BatchCapacity]):
+    def __init__(self, trainer: SageTrainer, host_batch, capacity: Optional[BatchCapacity]):
+        if isinstance(host_batch, PagePool):
+            trainer._check_resident(host_batch, capacity)
         self._trainer = trainer
         self.num_classes = trainer.num_classes
         self.totals = trainer.eval_totals()
@@ -844,9 +1040,14 @@ class EvalCapture:
         """Start the H2D copy of the next batch on a side stream (two input sets alternate, as for the train step)."""
         self._pass.prefetch_batch(host_batch)
 
+    def plan_epoch(self, page_ids, batch_pages: int) -> List[PlannedBatch]:
+        """Plan the validation batches of a pass captured on a ``PagePool`` (see ``SageTrainer.plan_epoch``)."""
+        return self._pass.plan_epoch(page_ids, batch_pages)
+
     def replay(self) -> torch.Tensor:
-        """Evaluate the batch in input set 0 (a resident batch needs no copy); returns ``totals``."""
-        self._pass.replay(0)
+        """Evaluate the batch in input set 0 (a resident batch needs no copy) -- on a ``PagePool``: the next planned
+        batch that fits --; returns ``totals``."""
+        self._pass.replay_next()
         return self.totals
 
     def replay_prefetched(self) -> torch.Tensor:

@@ -985,6 +985,51 @@ def pad_batch(word, page_off, edge_off, src, dst, weight, feat, label, bad: Opti
     return bad
 
 
+PLAN_HEADER = 8  # [cursor, flag, nfit, B, L, 0, 0, 0] ahead of the ids and slice starts of an epoch plan
+
+
+def gather_plan(plan, pool_num_nodes, pool_num_edges, capacity, meta):
+    """Plan the next batch of an epoch plan on the device (gte_gather_plan): ``plan`` int32 [8 + 2 * pool pages]
+    (layout in gte.h), ``pool_num_nodes`` / ``pool_num_edges`` int32 per pool page, ``capacity`` a BatchCapacity,
+    ``meta`` the static set's int32 [4 + 2 * (P_cap + 1)] = (n, e, P, start | padded page table), written when the
+    batch fits.  Raises plan[1] bits on the device: 1 = cursor past the plan, 2 = batch refused."""
+    i32 = torch.int32
+    pages = int(pool_num_nodes.numel())
+    n_cap, e_cap, p_cap = capacity.shape
+    if pool_num_edges.numel() != pages or pages < 1:
+        raise GteError("gather_plan: need one node and one edge count per pool page")
+    check(lib().gte_gather_plan(_vec(plan, "plan", i32, PLAN_HEADER + 2 * pages), _vec(pool_num_nodes, "pool_num_nodes", i32),
+                                _vec(pool_num_edges, "pool_num_edges", i32), pages, capacity.nodes, capacity.edges,
+                                capacity.pages, capacity.page_nodes, capacity.page_edges, n_cap, e_cap, p_cap,
+                                _vec(meta, "meta", i32, 4 + 2 * (p_cap + 1)), _stream()), "gte_gather_plan")
+
+
+def gather_pages(plan, meta, capacity, pool_node_off, pool_edge_off, pool_src, pool_dst, pool_weight, pool_feat,
+                 pool_label, src, dst, weight, feat, label):
+    """Copy the batch ``meta`` describes (gather_plan) from the pool into the real prefix of a capacity static set
+    (gte_gather_pages): ``pool_*`` = page-local COO, weights, features [N_pool, f], labels and int64 node / edge
+    offsets [pool pages + 1]; ``src`` / ``dst`` / ``weight`` [E_cap], ``feat`` [N_cap, f] contiguous, ``label``
+    [N_cap].  Copies nothing while plan[1] is non-zero (the plan kernel refused the batch); a page the page table
+    does not describe raises plan[1] bit 4 and is skipped."""
+    i32, i64 = torch.int32, torch.int64
+    n_cap, e_cap, p_cap = capacity.shape
+    pages = int(pool_node_off.numel()) - 1
+    f = int(feat.shape[1]) if feat.dim() == 2 else -1
+    if pool_feat.dim() != 2 or int(pool_feat.shape[1]) != f or not feat.is_contiguous() or not pool_feat.is_contiguous():
+        raise GteError(f"gather_pages: pool features {tuple(pool_feat.shape)} and batch features {tuple(feat.shape)} "
+                       "must be contiguous with the same width")
+    if feat.shape[0] != n_cap or label.numel() != n_cap or src.numel() != e_cap or dst.numel() != e_cap \
+            or weight.numel() != e_cap or pool_edge_off.numel() != pages + 1:
+        raise GteError("gather_pages: static set or pool offsets of the wrong size")
+    check(lib().gte_gather_pages(_vec(plan, "plan", i32, PLAN_HEADER + 2 * pages), _vec(meta, "meta", i32, 4 + 2 * (p_cap + 1)),
+                                 n_cap, e_cap, p_cap, capacity.pages, _vec(pool_node_off, "pool_node_off", i64),
+                                 _vec(pool_edge_off, "pool_edge_off", i64), pages, _vec(pool_src, "pool_src", i32),
+                                 _vec(pool_dst, "pool_dst", i32), _vec(pool_weight, "pool_weight"),
+                                 _vec(pool_feat, "pool_feat"), _vec(pool_label, "pool_label"), f, _vec(src, "src", i32),
+                                 _vec(dst, "dst", i32), _vec(weight, "weight"), _vec(feat, "feat"),
+                                 _vec(label, "label"), _stream()), "gte_gather_pages")
+
+
 def bbox_features(boxes: torch.Tensor, counts: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """13 BBOX features per text box (bbox.py:49-111) from int32 boxes [n,4] and character-class counts [n,3]."""
     _req_cuda(boxes, counts)

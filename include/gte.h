@@ -561,6 +561,40 @@ int gte_pad_batch(const int32_t* word, int32_t n_cap, int64_t e_cap, int32_t p_c
                   int32_t f, float* label, int32_t* bad, gte_stream_t stream);
 
 /*
+ * Batches gathered from a device-resident page pool, so that a captured pass assembles its own next batch: the
+ * host-side `dgl.batch(train_batch).to(device)` of model_train.py:279-297 and the per-page batches of
+ * model_predict.py:130-154 become one small upload of page ids per epoch.  Both entries are graph-capturable.
+ *
+ * The pool (PagePool) holds every page with page-local ids: COO src / dst [E_pool] int32, weights [E_pool], features
+ * [N_pool, f] (row-major, stride f), labels [N_pool] fp32, node / edge offsets [pool_pages + 1] int64 and the per-page
+ * node / edge counts [pool_pages] int32.  `plan` is an int32 device buffer of 8 + 2 * pool_pages words:
+ *   [cursor, flag, nfit, B, L, 0, 0, 0 | ids[L] | starts[nfit]],
+ * the epoch's page ids and the start offsets of its slices that fit; slice k is ids[starts[k], min(starts[k] + B, L)).
+ *
+ * gte_gather_plan (one CTA) runs slice `cursor` and advances the cursor by one.  It writes the capacity static set's
+ * `meta` = [n, e, P, start | page_off (p_cap + 1) | edge_off (p_cap + 1)]: the batch's totals, its start offset in
+ * ids, and the padded page table of gte_pad_batch -- the real pages, then s = min(p_cap - P, n_cap - n) padding
+ * pages at n + j (n_cap - n) / s nodes (64-bit; edges likewise), then empty pages.  The batch must fit the capacity
+ * (cap_*: total nodes, total edges, pages, largest page in nodes / edges, as BatchCapacity.check) with n_cap >
+ * cap_nodes, p_cap > cap_pages.  Otherwise `flag` gains bit 0 (cursor past the plan, or a malformed header) or bit 1
+ * (the batch does not fit, or an id lies outside the pool) and `meta` is left as it was.
+ * gte_gather_pages copies the pages of the batch in `meta` into the real prefix of src / dst / weight [e_cap], feat
+ * [n_cap, f] (contiguous) and label [n_cap]: features, labels and weights as they are, src / dst plus the page's node
+ * offset in the batch.  It copies nothing while `flag` is non-zero (the plan kernel refused the batch, so `meta`
+ * still describes an earlier one); a page the page table does not describe sets flag bit 2 and is skipped.  Its grid is
+ * min(4 * SMs, max_pages) CTAs (max_pages = the capacity's page count), looping over the pages.
+ */
+int gte_gather_plan(int32_t* plan, const int32_t* pool_num_nodes, const int32_t* pool_num_edges, int32_t pool_pages,
+                    int32_t cap_nodes, int64_t cap_edges, int32_t cap_pages, int32_t cap_page_nodes,
+                    int32_t cap_page_edges, int32_t n_cap, int64_t e_cap, int32_t p_cap, int32_t* meta,
+                    gte_stream_t stream);
+int gte_gather_pages(int32_t* plan, const int32_t* meta, int32_t n_cap, int64_t e_cap, int32_t p_cap,
+                     int32_t max_pages, const int64_t* pool_node_off, const int64_t* pool_edge_off,
+                     int32_t pool_pages, const int32_t* pool_src, const int32_t* pool_dst, const float* pool_weight,
+                     const float* pool_feat, const float* pool_label, int32_t f, int32_t* src, int32_t* dst,
+                     float* weight, float* feat, float* label, gte_stream_t stream);
+
+/*
  * BBOX node features on the device (src/components/nlp/bbox.py:49-54 get_shape, :57-111 get_histogram, called
  * per batch at model_train.py:293): boxes [n, 4] int32 = [x0, y0, x1, y1]; counts [n, 3] int32 = (letters,
  * digits, other symbols) of the box text with blanks removed (str.isalpha / str.isdigit are host string
