@@ -92,6 +92,8 @@ SIGNATURES = {
     "gte_bbox_features": (ci, [vp, vp, i32, vp, i64, vp]),
     "gte_adam_step": (ci, [vp, vp, vp, vp, i64, f32, f32, f32, f32, f32, i64, vp, f32, vp, vp]),
     "gte_dp_allreduce_adam": (ci, [vp, vp, i32, i32, i64, i64, vp, vp, vp, vp, f32, f32, f32, f32, f32, vp, vp, vp]),
+    "gte_adam_step_dev": (ci, [vp, vp, vp, vp, i64, vp, i64, vp, f32, vp, vp]),
+    "gte_dp_allreduce_adam_dev": (ci, [vp, vp, i32, i32, i64, i64, vp, vp, vp, vp, vp, vp, vp, vp]),
 }
 
 PACK_BATCH_MAX = 8

@@ -62,6 +62,7 @@ struct DpArgs {
   float* exp_avg_sq;
   float* stats_out;                // [4] global statistics
   float lr, b1, b2, eps, wd;
+  const float* hparams;            // NULL, or device [lr, b1, b2, eps, wd] read in place of the five values above
   int64_t* step_dev;               // optimiser step counter (incremented here)
   uint32_t* local;                 // [4] device words: 0 = sequence number of the last finished call, 1 = "peers ready" flag,
                                    //     2 = finished-blocks counter
@@ -69,6 +70,7 @@ struct DpArgs {
 
 __global__ void __launch_bounds__(DP_THREADS) k_dp_allreduce_adam(const DpArgs A) {
   __shared__ float s_den;
+  __shared__ float s_hp[5];
   const int tid = threadIdx.x;
   const uint32_t seq = A.local[0] + 1;  // written only by the LAST block of the previous call: every block reads the same value
   const int64_t t = *A.step_dev + 1;    // likewise
@@ -118,14 +120,17 @@ __global__ void __launch_bounds__(DP_THREADS) k_dp_allreduce_adam(const DpArgs A
       (void)w3;
     }
   }
+  if (A.hparams && tid < 5) s_hp[tid] = A.hparams[tid];
   __syncthreads();
   const float den = s_den;
+  const float lr = A.hparams ? s_hp[0] : A.lr, b1 = A.hparams ? s_hp[1] : A.b1, b2 = A.hparams ? s_hp[2] : A.b2;
+  const float eps = A.hparams ? s_hp[3] : A.eps, wd = A.hparams ? s_hp[4] : A.wd;
   if (den > 0.f) {  // a step without any weighted label has no defined gradient: leave the replica untouched
     const float gscale = 1.0f / den;
     // bias corrections exactly as torch.optim.Adam's single-tensor path (double maths, then fp32 use)
-    const double bc1 = 1.0 - pow((double)A.b1, (double)t);
-    const double bc2 = 1.0 - pow((double)A.b2, (double)t);
-    const float step_size = (float)((double)A.lr / bc1);
+    const double bc1 = 1.0 - pow((double)b1, (double)t);
+    const double bc2 = 1.0 - pow((double)b2, (double)t);
+    const float step_size = (float)((double)lr / bc1);
     const float bc2_sqrt = (float)sqrt(bc2);
     const int64_t n4 = A.count >> 2;
     for (int64_t i = (int64_t)blockIdx.x * DP_THREADS + tid; i < n4; i += (int64_t)gridDim.x * DP_THREADS) {
@@ -143,12 +148,12 @@ __global__ void __launch_bounds__(DP_THREADS) k_dp_allreduce_adam(const DpArgs A
       float* gp = &g.x; float* pp = &p.x; float* mp = &m.x; float* vp = &v.x;
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
-        const float gi = fmaf(A.wd, pp[e], gp[e] * gscale);      // grad = grad + weight_decay * param
-        const float mi = mp[e] + (gi - mp[e]) * (1.0f - A.b1);   // exp_avg.lerp_(grad, 1 - beta1)
-        const float vi = vp[e] * A.b2 + (1.0f - A.b2) * gi * gi;
+        const float gi = fmaf(wd, pp[e], gp[e] * gscale);      // grad = grad + weight_decay * param
+        const float mi = mp[e] + (gi - mp[e]) * (1.0f - b1);   // exp_avg.lerp_(grad, 1 - beta1)
+        const float vi = vp[e] * b2 + (1.0f - b2) * gi * gi;
         mp[e] = mi;
         vp[e] = vi;
-        pp[e] = pp[e] - step_size * (mi / (sqrtf(vi) / bc2_sqrt + A.eps));
+        pp[e] = pp[e] - step_size * (mi / (sqrtf(vi) / bc2_sqrt + eps));
       }
       reinterpret_cast<float4*>(A.param)[i] = p;
       reinterpret_cast<float4*>(A.exp_avg)[i] = m;
@@ -177,10 +182,10 @@ __global__ void __launch_bounds__(DP_THREADS) k_dp_allreduce_adam(const DpArgs A
 
 using namespace gte;
 
-extern "C" int gte_dp_allreduce_adam(const void* peer_grad_ptrs_dev, const void* peer_signal_ptrs_dev, int32_t rank,
-                                     int32_t world, int64_t count, int64_t stats_off, float* param, float* exp_avg,
-                                     float* exp_avg_sq, float* stats_out, float lr, float beta1, float beta2, float eps,
-                                     float weight_decay, int64_t* step_dev, uint32_t* local_words, gte_stream_t stream) {
+static int dp_allreduce_adam(const void* peer_grad_ptrs_dev, const void* peer_signal_ptrs_dev, int32_t rank, int32_t world,
+                             int64_t count, int64_t stats_off, float* param, float* exp_avg, float* exp_avg_sq,
+                             float* stats_out, float lr, float beta1, float beta2, float eps, float weight_decay,
+                             const float* hparams, int64_t* step_dev, uint32_t* local_words, gte_stream_t stream) {
   GTE_CHECK_ARG(world >= 1 && world <= DP_MAX_WORLD && rank >= 0 && rank < world, "gte_dp_allreduce_adam: bad rank/world");
   GTE_CHECK_ARG(count >= 0 && count % 4 == 0 && stats_off >= count, "gte_dp_allreduce_adam: count must be a multiple of 4 and the statistics behind the parameters");
   GTE_CHECK_ARG(peer_grad_ptrs_dev && peer_signal_ptrs_dev && param && exp_avg && exp_avg_sq && stats_out && step_dev && local_words,
@@ -190,7 +195,7 @@ extern "C" int gte_dp_allreduce_adam(const void* peer_grad_ptrs_dev, const void*
   a.peer_signal = static_cast<uint32_t* const*>(peer_signal_ptrs_dev);
   a.rank = rank; a.world = world; a.count = count; a.stats_off = stats_off;
   a.param = param; a.exp_avg = exp_avg; a.exp_avg_sq = exp_avg_sq; a.stats_out = stats_out;
-  a.lr = lr; a.b1 = beta1; a.b2 = beta2; a.eps = eps; a.wd = weight_decay;
+  a.lr = lr; a.b1 = beta1; a.b2 = beta2; a.eps = eps; a.wd = weight_decay; a.hparams = hparams;
   a.step_dev = step_dev; a.local = local_words;
   // all blocks must be resident at once (they wait for block 0): a fraction of the SMs is plenty for <= tens of MB
   int grid = sm_count() / 2;
@@ -200,4 +205,22 @@ extern "C" int gte_dp_allreduce_adam(const void* peer_grad_ptrs_dev, const void*
   k_dp_allreduce_adam<<<grid, DP_THREADS, 0, as_stream(stream)>>>(a);
   GTE_CHECK_LAUNCH("k_dp_allreduce_adam");
   return GTE_OK;
+}
+
+extern "C" int gte_dp_allreduce_adam(const void* peer_grad_ptrs_dev, const void* peer_signal_ptrs_dev, int32_t rank,
+                                     int32_t world, int64_t count, int64_t stats_off, float* param, float* exp_avg,
+                                     float* exp_avg_sq, float* stats_out, float lr, float beta1, float beta2, float eps,
+                                     float weight_decay, int64_t* step_dev, uint32_t* local_words, gte_stream_t stream) {
+  return dp_allreduce_adam(peer_grad_ptrs_dev, peer_signal_ptrs_dev, rank, world, count, stats_off, param, exp_avg,
+                           exp_avg_sq, stats_out, lr, beta1, beta2, eps, weight_decay, nullptr, step_dev, local_words,
+                           stream);
+}
+
+extern "C" int gte_dp_allreduce_adam_dev(const void* peer_grad_ptrs_dev, const void* peer_signal_ptrs_dev, int32_t rank,
+                                         int32_t world, int64_t count, int64_t stats_off, float* param, float* exp_avg,
+                                         float* exp_avg_sq, float* stats_out, const float* hparams, int64_t* step_dev,
+                                         uint32_t* local_words, gte_stream_t stream) {
+  GTE_CHECK_ARG(hparams != nullptr, "gte_dp_allreduce_adam_dev: null hparams");
+  return dp_allreduce_adam(peer_grad_ptrs_dev, peer_signal_ptrs_dev, rank, world, count, stats_off, param, exp_avg,
+                           exp_avg_sq, stats_out, 0.f, 0.f, 0.f, 0.f, 0.f, hparams, step_dev, local_words, stream);
 }

@@ -629,10 +629,17 @@ __global__ void k_rng_advance(int64_t* rng, int64_t by) { rng[1] += by; }
 
 __global__ void k_step_inc(int64_t* step) { *step += 1; }
 
+// hp (may be NULL): device [lr, beta1, beta2, eps, weight_decay], read once per CTA in place of the by-value arguments
 __global__ void k_adam(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                        float* __restrict__ v, int64_t count, float lr, float b1, float b2, float eps, float wd,
-                       int64_t step_host, const int64_t* __restrict__ step_dev, float grad_scale,
-                       const float* __restrict__ grad_den) {
+                       const float* __restrict__ hp, int64_t step_host, const int64_t* __restrict__ step_dev,
+                       float grad_scale, const float* __restrict__ grad_den) {
+  if (hp) {
+    __shared__ float s_hp[5];
+    if (threadIdx.x < 5) s_hp[threadIdx.x] = hp[threadIdx.x];
+    __syncthreads();
+    lr = s_hp[0]; b1 = s_hp[1]; b2 = s_hp[2]; eps = s_hp[3]; wd = s_hp[4];
+  }
   const int64_t t = step_dev ? *step_dev : step_host;
   if (grad_den) {
     // data parallel: gradients were summed un-normalised.  A step without any weighted label (every label out of
@@ -888,9 +895,9 @@ int gte_comb_fill(const float* x, int64_t ldx, int32_t w, float* out, int64_t ld
   return GTE_OK;
 }
 
-int gte_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t count, float lr,
-                  float beta1, float beta2, float eps, float weight_decay, int64_t step_host, int64_t* step_dev,
-                  float grad_scale, const float* grad_den, gte_stream_t stream) {
+static int adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t count, float lr,
+                     float beta1, float beta2, float eps, float weight_decay, const float* hparams, int64_t step_host,
+                     int64_t* step_dev, float grad_scale, const float* grad_den, gte_stream_t stream) {
   GTE_CHECK_ARG(count >= 0, "gte_adam_step: negative count");
   GTE_CHECK_ARG(step_dev != nullptr || step_host >= 1, "gte_adam_step: step must be >= 1");
   if (count == 0) return GTE_OK;
@@ -901,9 +908,24 @@ int gte_adam_step(float* param, const float* grad, float* exp_avg, float* exp_av
     GTE_CHECK_LAUNCH("k_step_inc");
   }
   k_adam<<<ew_grid(count), 256, 0, st>>>(param, grad, exp_avg, exp_avg_sq, count, lr, beta1, beta2, eps, weight_decay,
-                                        step_host, step_dev, grad_scale, grad_den);
+                                        hparams, step_host, step_dev, grad_scale, grad_den);
   GTE_CHECK_LAUNCH("k_adam");
   return GTE_OK;
+}
+
+int gte_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t count, float lr,
+                  float beta1, float beta2, float eps, float weight_decay, int64_t step_host, int64_t* step_dev,
+                  float grad_scale, const float* grad_den, gte_stream_t stream) {
+  return adam_step(param, grad, exp_avg, exp_avg_sq, count, lr, beta1, beta2, eps, weight_decay, nullptr, step_host,
+                   step_dev, grad_scale, grad_den, stream);
+}
+
+int gte_adam_step_dev(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t count,
+                      const float* hparams, int64_t step_host, int64_t* step_dev, float grad_scale, const float* grad_den,
+                      gte_stream_t stream) {
+  GTE_CHECK_ARG(hparams != nullptr, "gte_adam_step_dev: null hparams");
+  return adam_step(param, grad, exp_avg, exp_avg_sq, count, 0.f, 0.f, 0.f, 0.f, 0.f, hparams, step_host, step_dev,
+                   grad_scale, grad_den, stream);
 }
 
 int gte_dropout_concat(const float* x1, int64_t ldx1, int32_t f1, const float* x2, int64_t ldx2, int32_t f2, int32_t n,

@@ -207,6 +207,134 @@ def resident_warmup_ids(pool, capacity: BatchCapacity) -> np.ndarray:
     return ok[:k]
 
 
+# ---------------------------------------------------------------------- the trainer's optimizer as torch.optim.Adam --
+def check_adam_group(group: dict, where: str) -> Tuple[float, float, float, float, float]:
+    """(lr, beta1, beta2, eps, weight_decay) of an Adam param group the trainer's kernels can run, validated by
+    torch.optim.Adam's rules; a GteError names what they cannot run (a tensor value, AMSGrad, maximize, AdamW)."""
+    for k in ("amsgrad", "maximize", "decoupled_weight_decay"):
+        if group.get(k, False):
+            raise GteError(f"{where}: {k}=True is not supported (plain Adam with L2 weight decay only)")
+    lr, betas, eps, wd = group["lr"], group["betas"], group["eps"], group["weight_decay"]
+    if not isinstance(betas, (tuple, list)) or len(betas) != 2:
+        raise GteError(f"{where}: betas must be a pair, got {betas!r}")
+    vals = (lr, betas[0], betas[1], eps, wd)
+    for name, v in zip(("lr", "beta1", "beta2", "eps", "weight_decay"), vals):
+        if isinstance(v, torch.Tensor):
+            raise GteError(f"{where}: {name} as a tensor is not supported; assign a Python number")
+        if isinstance(v, bool) or not isinstance(v, (int, float, np.integer, np.floating)):
+            raise GteError(f"{where}: {name} must be a number, got {v!r}")
+    lr, b1, b2, eps, wd = (float(v) for v in vals)
+    # torch.optim.Adam.__init__'s checks (written so that NaN fails them)
+    if not 0.0 <= lr:
+        raise GteError(f"{where}: invalid learning rate: {lr}")
+    if not 0.0 <= eps:
+        raise GteError(f"{where}: invalid epsilon value: {eps}")
+    if not 0.0 <= b1 < 1.0 or not 0.0 <= b2 < 1.0:
+        raise GteError(f"{where}: invalid beta parameters: {(b1, b2)}")
+    if not 0.0 <= wd:
+        raise GteError(f"{where}: invalid weight_decay value: {wd}")
+    return lr, b1, b2, eps, wd
+
+
+def loaded_adam_step(state_dict: dict, shapes: Sequence[torch.Size]) -> int:
+    """The step count of an Adam state dict for parameters of these shapes, in flat-buffer order (0: no state yet).
+    Raises a GteError when the trainer cannot load it: other than one param group, a parameter count or shape other
+    than the model's, per-parameter steps that differ, or a group the kernels cannot run (``check_adam_group``)."""
+    groups = state_dict.get("param_groups")
+    if not isinstance(groups, list) or len(groups) != 1:
+        raise GteError(f"optimizer.load_state_dict: expected one param group, got "
+                       f"{len(groups) if isinstance(groups, list) else groups!r}")
+    group = groups[0]
+    check_adam_group(group, "optimizer.load_state_dict")
+    ids = list(group["params"])
+    if len(ids) != len(shapes):
+        raise GteError(f"optimizer.load_state_dict: {len(ids)} parameters, the model has {len(shapes)}")
+    state = state_dict.get("state", {})
+    if not any(i in state for i in ids):
+        return 0
+    steps = set()
+    for j, (i, shape) in enumerate(zip(ids, shapes)):
+        st = state.get(i)
+        if not st:
+            raise GteError(f"optimizer.load_state_dict: parameter {j} has no state while others have")
+        for k in ("exp_avg", "exp_avg_sq"):
+            t = st.get(k)
+            if not isinstance(t, torch.Tensor) or tuple(t.shape) != tuple(shape):
+                raise GteError(f"optimizer.load_state_dict: parameter {j}: {k} of shape "
+                               f"{tuple(t.shape) if isinstance(t, torch.Tensor) else t!r}, expected {tuple(shape)}")
+        step = st.get("step")  # a tensor since torch 1.12, an int before
+        steps.add(float(step.item() if isinstance(step, torch.Tensor) else step))
+    if len(steps) != 1:
+        raise GteError(f"optimizer.load_state_dict: the parameters have different step counts {sorted(steps)}; the "
+                       "trainer keeps one")
+    step = steps.pop()
+    if not (step >= 0 and step == int(step)):
+        raise GteError(f"optimizer.load_state_dict: step {step} is not a count")
+    return int(step)
+
+
+class TrainerAdam(torch.optim.Adam):
+    """``SageTrainer.optimizer``: a ``torch.optim.Adam`` over the model's parameters, in flat-buffer order, whose state
+    lives in the trainer's device buffers.  Its one param group holds the hyper-parameters every update path of the
+    trainer reads -- torch's schedulers change them through it -- and ``state_dict()`` / ``load_state_dict()`` speak
+    torch's format, so checkpoints move between the trainer and a plain ``torch.optim.Adam`` over the same model.
+    ``step()`` and ``zero_grad()`` are refused: the trainer's own steps update the parameters."""
+
+    def __init__(self, trainer: "SageTrainer", params, lr, betas, eps, weight_decay):
+        super().__init__(params, lr=lr, betas=betas, eps=eps, weight_decay=weight_decay)
+        self._trainer = trainer
+        self._loaded_step = 0
+        self.register_state_dict_pre_hook(TrainerAdam._state_from_device)
+        self.register_load_state_dict_pre_hook(TrainerAdam._check_load)
+        self.register_load_state_dict_post_hook(TrainerAdam._state_to_device)
+
+    def step(self, closure=None):
+        raise GteError("SageTrainer.optimizer.step(): the trainer applies Adam in its own steps (train_step / replay); "
+                       "drive only the learning-rate schedule through the optimizer")
+
+    def zero_grad(self, set_to_none: bool = True):
+        raise GteError("SageTrainer.optimizer.zero_grad(): the trainer's backward overwrites its gradient buffer every "
+                       "step (and set_to_none would detach the parameters' gradient views)")
+
+    def add_param_group(self, param_group):
+        if self.param_groups:
+            raise GteError("SageTrainer.optimizer: one param group only (the trainer's flat parameter buffer)")
+        super().add_param_group(param_group)
+
+    def _views(self):
+        tr = self._trainer
+        return [(p, tr.exp_avg[o:o + p.numel()].view_as(p), tr.exp_avg_sq[o:o + p.numel()].view_as(p))
+                for p, o in zip(self.param_groups[0]["params"], tr._offs)]
+
+    def _set_state(self, step: int):
+        """per-parameter state as torch.optim.Adam keeps it: empty before the first step, else a float32 CPU ``step``
+        and views of the flat moment buffers"""
+        self.state.clear()
+        if step > 0:
+            for p, m, v in self._views():
+                self.state[p] = {"step": torch.tensor(float(step), dtype=torch.float32), "exp_avg": m, "exp_avg_sq": v}
+
+    def _state_from_device(self):
+        self._set_state(int(self._trainer.step_dev.item()))
+
+    def _check_load(self, state_dict):
+        self._loaded_step = loaded_adam_step(state_dict, [p.shape for p in self.param_groups[0]["params"]])
+
+    def _state_to_device(self):
+        # torch has cast the loaded moments to the parameters' device; copy them into the buffers captured graphs read
+        tr, step = self._trainer, self._loaded_step
+        with torch.no_grad():
+            if step == 0:
+                tr.exp_avg.zero_()
+                tr.exp_avg_sq.zero_()
+            else:
+                for p, m, v in self._views():
+                    m.copy_(self.state[p]["exp_avg"])
+                    v.copy_(self.state[p]["exp_avg_sq"])
+            tr.step_dev.fill_(step)
+        self._set_state(step)
+
+
 class SageTrainer:
     def __init__(self, model: GcnSAGE, lr: float = 0.01, weight_decay: float = 5e-4, betas=(0.9, 0.999),
                  eps: float = 1e-8, class_weights: Optional[torch.Tensor] = None, process_group=None):
@@ -218,7 +346,6 @@ class SageTrainer:
         for layer in model.layers:
             if layer.activation is not None and not _is_relu(layer.activation):
                 raise GteError("SageTrainer: only activation=F.relu/None is fused; use the nn.Module path otherwise")
-        self.lr, self.wd, self.betas, self.eps = lr, weight_decay, betas, eps
         self.class_w = None if class_weights is None else class_weights.to(self.device, torch.float32).contiguous()
         self.pg = process_group
         self.world = 1
@@ -259,6 +386,7 @@ class SageTrainer:
         self.exp_avg_sq = torch.zeros(o, dtype=torch.float32, device=self.device)
         self.step_dev = torch.zeros(1, dtype=torch.int64, device=self.device)
         self.num_params = total
+        self._offs = offs
         self._grad_views: Dict[int, torch.Tensor] = {}
         with torch.no_grad():
             for p, off in zip(params, offs):
@@ -281,6 +409,50 @@ class SageTrainer:
         self.num_classes = int(model.layers[-1].linear.weight.shape[0])
         self._train: Optional[_CapturedPass] = None  # the captured train or predict step
         self._mode = "train"
+        # Adam's hyper-parameters [lr, beta1, beta2, eps, weight_decay] in device memory: every update path reads them
+        # when it runs, so a learning-rate schedule reaches captured replays (a graph freezes by-value kernel
+        # arguments).  optimizer.param_groups[0] is where they are set; _sync_hparams writes them here when they change.
+        # Data parallel: every rank holds its own copy, so every rank must apply the same schedule.
+        self.hparams = torch.zeros(5, dtype=torch.float32, device=self.device)
+        self._hp_key = None
+        self.optimizer = TrainerAdam(self, model.parameters(), lr, betas, eps, weight_decay)
+        self._sync_hparams()
+
+    # ------------------------------------------------------- optimiser -----
+    @property
+    def lr(self):
+        """the learning rate of ``optimizer.param_groups[0]`` (the next step uses what is assigned here)"""
+        return self.optimizer.param_groups[0]["lr"]
+
+    @lr.setter
+    def lr(self, value):
+        self.optimizer.param_groups[0]["lr"] = value
+
+    def _sync_hparams(self):
+        """Called before every path that can run an update (train_step, replay, replay_set, replay_prefetched and the
+        capture warm-up; the split tail runs inside the replays).  When the param group changed since the last call,
+        validate it and write ``hparams`` with one copy, ordered on the current stream before the update; else this
+        is one tuple comparison."""
+        groups = self.optimizer.param_groups
+        g = groups[0]
+        key = (len(groups), g["lr"], g["betas"], g["eps"], g["weight_decay"], g["amsgrad"], g["maximize"],
+               g.get("decoupled_weight_decay", False))
+        if key != self._hp_key or isinstance(key[1], torch.Tensor):  # a tensor equal to the number compares equal
+            if len(groups) != 1:
+                raise GteError("SageTrainer.optimizer: one param group only (the trainer's flat parameter buffer)")
+            vals = check_adam_group(g, "SageTrainer.optimizer")
+            with torch.cuda.device(self.device):
+                if torch.cuda.is_current_stream_capturing():
+                    raise GteError("SageTrainer: Adam's hyper-parameters changed while a CUDA graph is being captured; "
+                                   "the copy would be replayed with the graph.  Change them before or after the capture")
+                # a fresh pinned staging tensor per write: the caching host allocator keeps it until the copy has run
+                staging = torch.tensor(vals, dtype=torch.float32).pin_memory()
+                self.hparams.copy_(staging, non_blocking=True)
+            self._hp_key = key
+        # LR schedulers warn about `scheduler.step()` before `optimizer.step()` unless the optimizer's `_opt_called`
+        # (torch's private flag, set by the wrapper a scheduler puts around optimizer.step) is true.  optimizer.step()
+        # is refused here, so the trainer's own updates count as the optimizer's steps.
+        self.optimizer._opt_called = True
 
     # ----------------------------------------------------------- pieces ----
     def _layer_args(self, layer):
@@ -365,9 +537,8 @@ class SageTrainer:
             ops.rng_advance(self.rng_dev, self._rng_used)  # the next step (or graph replay) draws new masks
 
     def _stage_update(self):
-        ops.adam_step(self.flat_param, self.flat_grad, self.exp_avg, self.exp_avg_sq, lr=self.lr, beta1=self.betas[0],
-                      beta2=self.betas[1], eps=self.eps, weight_decay=self.wd, step_dev=self.step_dev,
-                      grad_den=self.stats[1:2] if self.dp_fused else None, count=self._flat_len)
+        ops.adam_step(self.flat_param, self.flat_grad, self.exp_avg, self.exp_avg_sq, hparams=self.hparams,
+                      step_dev=self.step_dev, grad_den=self.stats[1:2] if self.dp_fused else None, count=self._flat_len)
 
     def _setup_peer_exchange(self, numel: int):
         """Flat gradient buffer in symmetric memory (every rank can load every other rank's buffer over NVLink) for the
@@ -400,9 +571,8 @@ class SageTrainer:
         if self._dp_peer is not None:
             d = self._dp_peer
             ops.dp_allreduce_adam(d["grad_ptrs"], d["pads"].data_ptr(), d["rank"], self.world, self._flat_len, self._flat_len,
-                                  self.flat_param, self.exp_avg, self.exp_avg_sq, self.stats_global, lr=self.lr,
-                                  beta1=self.betas[0], beta2=self.betas[1], eps=self.eps, weight_decay=self.wd,
-                                  step_dev=self.step_dev, local_words=d["local"])
+                                  self.flat_param, self.exp_avg, self.exp_avg_sq, self.stats_global,
+                                  hparams=self.hparams, step_dev=self.step_dev, local_words=d["local"])
         else:
             self._all_reduce(self.flat_grad)  # dp_fused: gradients + [sum w*nll, sum w, #correct] in one collective
             self._stage_update()
@@ -433,6 +603,7 @@ class SageTrainer:
         if labels is None:
             labels = g.ndata["label"]
         with torch.cuda.device(self.device):
+            self._sync_hparams()
             self._step_impl(g, labels)
         return self._result()
 
@@ -567,6 +738,8 @@ class SageTrainer:
             body, tail = self._stage_local, self._stage_exchange_update
         else:
             body, tail = self._step_impl, None
+        if mode == "train":
+            self._sync_hparams()  # the warm-up steps run with the current hyper-parameters
         # the warm-up steps train: restore the optimiser state afterwards
         snap = (self.flat_param.clone(), self.exp_avg.clone(), self.exp_avg_sq.clone(), self.step_dev.clone())
         self._train = _CapturedPass(self.device, host_batch, capacity, body, tail)
@@ -581,6 +754,10 @@ class SageTrainer:
         if self._train is None:
             raise GteError(f"{what}: call capture() first")
         return self._train
+
+    def _before_replay(self):
+        if self._mode == "train":
+            self._sync_hparams()
 
     def fits(self, host_batch: Dict[str, torch.Tensor]) -> bool:
         """True when ``host_batch`` can run through the captured step (``load_batch`` / ``prefetch_batch`` accept it).
@@ -614,7 +791,9 @@ class SageTrainer:
     def replay(self):
         """Run the captured step on input set 0 -- on a ``PagePool``: on the next planned batch that fits --; returns
         the statistics (train) or ``(preds, page_correct)`` of the batch (predict)."""
-        self._captured("replay").replay_next()
+        self._captured("replay")
+        self._before_replay()
+        self._train.replay_next()
         return self._outputs(0)
 
     def prefetch_batch(self, host_batch: Dict[str, torch.Tensor]):
@@ -626,13 +805,16 @@ class SageTrainer:
     def replay_set(self, which: int) -> torch.Tensor:
         """Run one captured step on static input set ``which`` (0 or 1) as it is: inputs resident in HBM, no copy.
         The sets are filled by ``prefetch_batch`` / ``load_batch``; the caller keeps track of what is in them."""
-        self._captured("replay_set").replay_set(which)
+        self._captured("replay_set")
+        self._before_replay()
+        self._train.replay_set(which)
         return self._outputs(which)
 
     def replay_prefetched(self):
         """Run one captured step on the oldest prefetched batch."""
         if self._train is None:
             raise GteError("replay_prefetched: no prefetched batch")
+        self._before_replay()
         return self._outputs(self._train.replay_prefetched())
 
 

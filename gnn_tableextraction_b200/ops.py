@@ -887,14 +887,36 @@ def cross_entropy_bwd(logits, labels, class_w, denominator, out=None):
     return out
 
 
-def adam_step(param, grad, exp_avg, exp_avg_sq, *, lr, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=0.0,
+def _hparams_or_values(where: str, hparams, values):
+    """``hparams`` (device float32 [5]: lr, beta1, beta2, eps, weight_decay) or the five values, not both"""
+    given = [v is not None for v in values]
+    if hparams is not None:
+        if any(given):
+            raise GteError(f"{where}: pass the hyper-parameters either as values or as an hparams tensor, not both")
+        return _vec(hparams, "hparams", n=5)
+    if not all(given):
+        raise GteError(f"{where}: the hyper-parameters are required, as values or as an hparams tensor")
+    return None
+
+
+def adam_step(param, grad, exp_avg, exp_avg_sq, *, lr=None, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=0.0,
               step: int = 0, step_dev: Optional[torch.Tensor] = None, grad_scale: float = 1.0,
-              grad_den: Optional[torch.Tensor] = None, count: Optional[int] = None):
+              grad_den: Optional[torch.Tensor] = None, count: Optional[int] = None,
+              hparams: Optional[torch.Tensor] = None):
+    """Adam over flat buffers (gte.h).  ``hparams`` (device float32 [5] = [lr, beta1, beta2, eps, weight_decay]) takes
+    the place of the five values: the kernel reads them when it runs, so a captured step follows later writes."""
     count = param.numel() if count is None else int(count)
     for t, nm in ((param, "param"), (grad, "grad"), (exp_avg, "exp_avg"), (exp_avg_sq, "exp_avg_sq")):
         _vec(t, nm, n=count)
     if step_dev is not None:
         _vec(step_dev, "step_dev", torch.int64, 1)
+    hp = _hparams_or_values("adam_step", hparams, (lr,))
+    if hp is not None:
+        check(lib().gte_adam_step_dev(param.data_ptr(), grad.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(),
+                                      count, hp, int(step), _ptr(step_dev), float(grad_scale),
+                                      _vec(grad_den, "grad_den", n=1), _stream()),
+              "gte_adam_step_dev")
+        return
     check(
         lib().gte_adam_step(param.data_ptr(), grad.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(), count,
                             float(lr), float(beta1), float(beta2), float(eps), float(weight_decay), int(step),
@@ -904,16 +926,21 @@ def adam_step(param, grad, exp_avg, exp_avg_sq, *, lr, beta1=0.9, beta2=0.999, e
 
 
 def dp_allreduce_adam(peer_grad_ptrs_dev: int, peer_signal_ptrs_dev: int, rank: int, world: int, count: int, stats_off: int,
-                      param, exp_avg, exp_avg_sq, stats_out, *, lr, beta1, beta2, eps, weight_decay, step_dev, local_words):
-    """One-shot all-reduce of the ranks' flat gradient buffers over NVLink peer memory fused with Adam (gte.h)."""
+                      param, exp_avg, exp_avg_sq, stats_out, *, lr=None, beta1=None, beta2=None, eps=None,
+                      weight_decay=None, step_dev, local_words, hparams: Optional[torch.Tensor] = None):
+    """One-shot all-reduce of the ranks' flat gradient buffers over NVLink peer memory fused with Adam (gte.h); the
+    hyper-parameters as five values or as a device ``hparams`` tensor (see ``adam_step``)."""
     for t, nm in ((param, "param"), (exp_avg, "exp_avg"), (exp_avg_sq, "exp_avg_sq")):
         _vec(t, nm, n=count)
-    check(lib().gte_dp_allreduce_adam(int(peer_grad_ptrs_dev), int(peer_signal_ptrs_dev), int(rank), int(world), int(count),
-                                      int(stats_off), param.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(),
-                                      _vec(stats_out, "stats_out", n=3), float(lr), float(beta1), float(beta2), float(eps),
-                                      float(weight_decay), _vec(step_dev, "step_dev", torch.int64, 1),
-                                      _vec(local_words, "local_words", torch.int32, 4), _stream()),
-          "gte_dp_allreduce_adam")
+    hp = _hparams_or_values("dp_allreduce_adam", hparams, (lr, beta1, beta2, eps, weight_decay))
+    head = (int(peer_grad_ptrs_dev), int(peer_signal_ptrs_dev), int(rank), int(world), int(count), int(stats_off),
+            param.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(), _vec(stats_out, "stats_out", n=3))
+    tail = (_vec(step_dev, "step_dev", torch.int64, 1), _vec(local_words, "local_words", torch.int32, 4), _stream())
+    if hp is not None:
+        check(lib().gte_dp_allreduce_adam_dev(*head, hp, *tail), "gte_dp_allreduce_adam_dev")
+    else:
+        check(lib().gte_dp_allreduce_adam(*head, float(lr), float(beta1), float(beta2), float(eps), float(weight_decay),
+                                          *tail), "gte_dp_allreduce_adam")
 
 
 # ------------------------------------------- either side of the layers ----

@@ -492,6 +492,16 @@ int gte_adam_step(float* param, const float* grad, float* exp_avg, float* exp_av
                   int64_t count, float lr, float beta1, float beta2, float eps,
                   float weight_decay, int64_t step_host, int64_t* step_dev, float grad_scale,
                   const float* grad_den, gte_stream_t stream);
+/*
+ * gte_adam_step with the hyper-parameters read from the device: `hparams` = float [5] = [lr, beta1, beta2, eps,
+ * weight_decay], loaded once per CTA; bit-identical to gte_adam_step given the same values.  The reference steps an
+ * optimizer built at model_train.py:168 every batch (:332) and lowers its learning rate from the validation loss once
+ * per epoch (:369).  A CUDA graph freezes by-value kernel arguments at capture, so a captured step that reads the
+ * values from device memory follows a schedule that rewrites that memory between replays.
+ */
+int gte_adam_step_dev(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t count,
+                      const float* hparams, int64_t step_host, int64_t* step_dev, float grad_scale,
+                      const float* grad_den, gte_stream_t stream);
 
 /*
  * Data-parallel step tail in ONE kernel: one-shot all-reduce of the flat gradient buffers over NVLink peer memory
@@ -510,6 +520,12 @@ int gte_dp_allreduce_adam(const void* peer_grad_ptrs_dev, const void* peer_signa
                           int64_t count, int64_t stats_off, float* param, float* exp_avg, float* exp_avg_sq,
                           float* stats_out, float lr, float beta1, float beta2, float eps, float weight_decay,
                           int64_t* step_dev, uint32_t* local_words, gte_stream_t stream);
+/* gte_dp_allreduce_adam with the hyper-parameters read from the device (`hparams`, as for gte_adam_step_dev);
+ * bit-identical to it given the same values. */
+int gte_dp_allreduce_adam_dev(const void* peer_grad_ptrs_dev, const void* peer_signal_ptrs_dev, int32_t rank,
+                              int32_t world, int64_t count, int64_t stats_off, float* param, float* exp_avg,
+                              float* exp_avg_sq, float* stats_out, const float* hparams, int64_t* step_dev,
+                              uint32_t* local_words, gte_stream_t stream);
 
 /* ---------------------------------------- either side of the layers ---- */
 /*
