@@ -11,9 +11,9 @@ import os
 from typing import Optional
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# GTE_LIB: load another in-tree build of the same ABI (the -DGTE_EXPERIMENTS build used by scripts/); never a fallback
+# GTE_LIB: load another build of the same ABI; never a fallback
 LIB_PATH = os.environ.get("GTE_LIB") or os.path.join(_HERE, "libgte_b200.so")
-ABI_VERSION = 2
+ABI_VERSION = 3
 HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "gte.h")
 
 _lib: Optional[C.CDLL] = None
@@ -54,7 +54,6 @@ SIGNATURES = {
     "gte_umma_pack_weights": (ci, [vp, i64, i32, i32, i32, vp, vp]),
     "gte_umma_linear_fwd": (ci, [vp, i64, vp, i64, i32, vp, vp, vp, vp, f32, ci, ci, vp, i64, vp, i64, vp, vp, i32, i32, vp]),
     "gte_umma_linear_bwd_data": (ci, [vp, i64, i32, vp, i32, vp, i64, vp, i64, i32, i32, vp]),
-    "gte_umma_debug_times": (ci, [i32, vp, i32]),
     "gte_umma_linear_fwd_stacked": (ci, [vp, i64, i32, vp, vp, i32, vp, i64, i32, vp]),
     "gte_umma_linear_bwd_data2": (ci, [vp, i64, vp, i64, i32, vp, vp, i64, i32, i32, vp]),
     "gte_umma_bwd_weight_supported": (ci, [i32, i32, i32]),
@@ -105,7 +104,7 @@ class PackDesc(C.Structure):
                 ("pack", C.c_void_p)]
 
 
-GTE_TUNE_UMMA_PAIR, GTE_TUNE_DW_PAIR, GTE_TUNE_EPI_STORE, GTE_TUNE_UMMA_SPLIT = 0, 1, 2, 3
+GTE_TUNE_UMMA_PAIR = 0
 GTE_AGG_SUM, GTE_AGG_SUM_NORM, GTE_AGG_MEAN = 0, 1, 2
 GTE_NORM_INV_DEG_ZERO, GTE_NORM_INV_DEG_CLAMP = 0, 1
 GTE_LABEL_I64, GTE_LABEL_I32, GTE_LABEL_F32 = 0, 1, 2

@@ -1,20 +1,11 @@
 #!/usr/bin/env bash
 # Builds libgte_b200.so (sm_100a only) in-tree next to the Python package.
-# Usage: csrc/build.sh [--exp] [extra nvcc flags]
-#   --exp   build libgte_b200_exp.so with -DGTE_EXPERIMENTS (role timestamps for scripts/umma_trace.py; load it with
-#           GTE_LIB=.../libgte_b200_exp.so); the product library never contains experiment code
+# Usage: csrc/build.sh [extra nvcc flags]
 set -euo pipefail
 here="$(cd "$(dirname "${BASH_SOURCE[0]}")" && pwd)"
 root="$(cd "$here/../.." && pwd)"
 out="$here/../libgte_b200.so"
 bdir="$here/build"
-extra=()
-if [[ "${1:-}" == "--exp" ]]; then
-  shift
-  out="$here/../libgte_b200_exp.so"
-  bdir="$here/build/exp"
-  extra+=(-DGTE_EXPERIMENTS)
-fi
 NVCC="${NVCC:-/usr/local/cuda/bin/nvcc}"
 srcs=("$here"/gte_*.cu)
 mkdir -p "$bdir"
@@ -25,7 +16,7 @@ for s in "${srcs[@]}"; do
   objs+=("$o")
   if [[ ! -f "$o" || "$s" -nt "$o" || -n "$(find "$here" "$root/include" \( -name '*.cuh' -o -name '*.h' \) -newer "$o" -print -quit)" ]]; then
     "$NVCC" -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 \
-      -Xcompiler -fPIC -I"$root/include" -I"$here" "${extra[@]}" "$@" -c "$s" -o "$o" &
+      -Xcompiler -fPIC -I"$root/include" -I"$here" "$@" -c "$s" -o "$o" &
     pids+=($!)
   fi
 done

@@ -49,8 +49,8 @@ int ensure_dynamic_smem(const void* func, size_t bytes, const char* name) {
   return GTE_OK;
 }
 
-// process-wide A/B switches (gte_set_tuning); defaults = the product path
-static std::atomic<int> g_tuning[GTE_TUNE_COUNT] = {{1}, {1}, {0}, {1}};
+// process-wide switches (gte_set_tuning); defaults = the product path
+static std::atomic<int> g_tuning[GTE_TUNE_COUNT] = {{1}};
 int tuning(int key) { return (key >= 0 && key < GTE_TUNE_COUNT) ? g_tuning[key].load(std::memory_order_relaxed) : 0; }
 
 int sm_count() {

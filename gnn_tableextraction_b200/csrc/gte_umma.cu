@@ -28,14 +28,8 @@
 #include "gte_umma_args.cuh"
 
 #include <cuda.h>
-#include <stdlib.h>
 
 namespace gte {
-
-#ifdef GTE_EXPERIMENTS
-// diagnostic: per-CTA, per-tile role timestamps (clock64) when UmmaArgs::dbg != 0; read with gte_umma_debug_times()
-__device__ long long g_umma_dbg[148 * 16 * 8];
-#endif
 
 constexpr int PK_PLANES = 2;  // packed weight tiles: tf32 hi, tf32 lo
 constexpr int UM_THREADS = 384;
@@ -78,16 +72,6 @@ __global__ void __launch_bounds__(UM_THREADS, 1) k_umma_gemm(const __grid_consta
   const int m_tiles = (P.M + UM_BM - 1) / UM_BM;
   const int total_tiles = m_tiles * P.ngroups;
   const int kb_total = P.kblocks[0] + (P.nseg > 1 ? P.kblocks[1] : 0);
-#ifdef GTE_EXPERIMENTS
-  auto stamp = [&](int tile, int slot) {
-    if (P.dbg && blockIdx.x < 148) {
-      const int t = (tile - blockIdx.x) / gridDim.x;
-      if (t < 16) g_umma_dbg[(blockIdx.x * 16 + t) * 8 + slot] = clock64();
-    }
-  };
-#else
-  auto stamp = [](int, int) {};
-#endif
 
   for (int i = threadIdx.x; i < UM_MAX_BN; i += UM_THREADS) {
     s_bias[i] = (P.bias && i < P.bias_n) ? P.bias[i] : 0.f;
@@ -136,13 +120,9 @@ __global__ void __launch_bounds__(UM_THREADS, 1) k_umma_gemm(const __grid_consta
           }
         }
       };
-#ifdef GTE_EXPERIMENTS
-      if (P.dbg & 32) pf_tile = total_tiles;  // timing experiment: no L2 prefetch
-#endif
       for (int i = 0; i < UM_PREFETCH; ++i) pf_step();
       for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
         const int mt = tile / P.ngroups, grp = tile % P.ngroups;
-        stamp(tile, 7);
         for (int seg = 0; seg < P.nseg; ++seg) {
           for (int kb = 0; kb < P.kblocks[seg]; ++kb) {
             pf_step();
@@ -169,10 +149,8 @@ __global__ void __launch_bounds__(UM_THREADS, 1) k_umma_gemm(const __grid_consta
       constexpr bool split_acc = SPLIT;
       constexpr int nacc = SPLIT ? 1 : 2;
       for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-        stamp(tile, 4);
         mbar_wait_backoff(smem_u32(&bar_tempty[acc]), acc_phase ^ 1);
         tc_fence_after();
-        stamp(tile, 5);
         const uint32_t d_tmem = tmem_base + (uint32_t)(acc * UM_ACC_STRIDE);
         const uint32_t d_cross = split_acc ? tmem_base + UM_ACC_STRIDE : d_tmem;
         for (int kb = 0; kb < kb_total; ++kb) {
@@ -193,7 +171,6 @@ __global__ void __launch_bounds__(UM_THREADS, 1) k_umma_gemm(const __grid_consta
           umma_commit(smem_u32(&bar_empty[stage]));
           if (++stage == UM_STAGES) { stage = 0; phase ^= 1; }
         }
-        stamp(tile, 6);
         umma_commit(smem_u32(&bar_tfull[acc]));
         if (++acc == nacc) { acc = 0; acc_phase ^= 1; }
       }
@@ -238,10 +215,8 @@ __global__ void __launch_bounds__(UM_THREADS, 1) k_umma_gemm(const __grid_consta
     const float inv_n = 1.0f / (float)P.N;
     for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
       const int mt = tile / P.ngroups, grp = tile % P.ngroups;
-      if (warp == 8 && lane == 0) stamp(tile, 0);
       mbar_wait(smem_u32(&bar_tfull[acc]), acc_phase);
       tc_fence_after();
-      if (warp == 8 && lane == 0) stamp(tile, 1);
       const uint32_t t_base = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * UM_ACC_STRIDE);
       const int64_t row0 = (int64_t)mt * UM_BM + q * 32;  // first global row of this warp
       float* outp = P.out[grp];
@@ -291,7 +266,6 @@ __global__ void __launch_bounds__(UM_THREADS, 1) k_umma_gemm(const __grid_consta
           P.rstd[grow] = rstd;
         }
       }
-      if (warp == 8 && lane == 0) stamp(tile, 2);
       const int rows_valid = (int)min((int64_t)32, (int64_t)P.M - row0);
       for (int c = 0; c < nchunks; ++c) {
         load_chunk(c);
@@ -310,7 +284,6 @@ __global__ void __launch_bounds__(UM_THREADS, 1) k_umma_gemm(const __grid_consta
         }
       }
 #undef load_chunk
-      if (warp == 8 && lane == 0) stamp(tile, 3);
       tc_fence_before();
       mbar_arrive(smem_u32(&bar_tempty[acc]));
       if (++acc == nacc) { acc = 0; acc_phase ^= 1; }
@@ -509,9 +482,6 @@ int launch_umma_single(UmmaArgs& a, cudaStream_t st) {
 // bounds the 3xTF32 contraction (see gte_umma2.cu); gte_set_tuning(GTE_TUNE_UMMA_PAIR, 0) forces the single-CTA kernel.
 static int launch_umma(UmmaArgs& a, cudaStream_t st) {
   if (int rc = setup_output_maps(a)) return rc;
-#ifdef GTE_EXPERIMENTS
-  a.dbg = getenv("GTE_UMMA_DBG") ? atoi(getenv("GTE_UMMA_DBG")) : 0;  // role timestamps
-#endif
   if (tuning(GTE_TUNE_UMMA_PAIR) != 0 && umma_pair_supported(a)) return launch_umma_pair(a, st);
   return launch_umma_single(a, st);
 }
@@ -797,21 +767,6 @@ int gte_umma_linear_bwd_data_comb(const float* dc, int64_t lddc, int32_t fo, con
   a.out[0] = dx;
   a.ldo[0] = lddx;
   return launch_umma(a, as_stream(stream));
-}
-
-// diagnostic only (-DGTE_EXPERIMENTS builds): copy the role timestamps of the last tensor-core projection launched with
-// GTE_UMMA_DBG=1 (148 x 16 x 8 int64); `which` 0 = single-CTA kernel, 1 = CTA-pair kernel
-int gte_umma_debug_times(int32_t which, int64_t* out_host, int32_t count) {
-  if (!out_host || count <= 0 || count > 148 * 16 * 8) return fail(GTE_ERR_INVALID, "gte_umma_debug_times: bad argument");
-#ifdef GTE_EXPERIMENTS
-  if (which == 1) return umma_pair_debug_times(out_host, count);
-  if (which == 2) return umma_dw_debug_times(out_host, count);
-  GTE_CHECK_CUDA(cudaMemcpyFromSymbol(out_host, g_umma_dbg, (size_t)count * 8), "gte_umma_debug_times");
-  return GTE_OK;
-#else
-  (void)which;
-  return fail(GTE_ERR_UNSUPPORTED, "gte_umma_debug_times: library built without -DGTE_EXPERIMENTS");
-#endif
 }
 
 }  // extern "C"

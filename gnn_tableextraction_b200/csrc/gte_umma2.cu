@@ -4,7 +4,7 @@
 // Why pairs: each SM stages only HALF of the weight tile (the hardware shares the halves of a cta_group::2 MMA), and the
 // operand split writes only the low part (the tensor core truncates the raw fp32 word to tf32 by itself).
 //
-// What bounds it (role timestamps, scripts/umma_trace.py, profiles/r02_umma_pair_experiments.md): NOT the tensor pipe
+// What bounds it (role timestamps, profiles/r02_umma_pair_experiments.md): NOT the tensor pipe
 // (issuing one of the three MMAs changes nothing; the 3x pattern alone runs at 1350-1500 clocks per k-block) but the
 // SM <-> L2 traffic: per 128-row tile 616 KB of operand tiles come in (224 KB activations + 392 KB weight tiles, which do
 // not fit in shared memory next to the operand ring and are re-read per tile) and 229 KB of z / y go out, ~1 GB per
@@ -35,21 +35,6 @@
 #include <cuda.h>
 
 namespace gte {
-
-#ifdef GTE_EXPERIMENTS
-__device__ long long g_umma2_dbg[148 * 16 * 8];
-// per-CTA role accounting (clock64 cycles): 0 span (producer), 1 producer waits on empty, 2 split waits on full,
-// 3 split work, 4 MMA waits on tempty, 5 MMA waits on ready, 6 MMA loop span, 7 epilogue waits on tfull,
-// 8 epilogue work, 9 k-blocks
-__device__ long long g_umma2_acc[148 * 16];
-#define U2_T0() const long long t0__ = clock64()
-#define U2_ACC(var) var += clock64() - t0__
-#define U2_PUT(slot, v) do { if (blockIdx.x < 148) g_umma2_acc[blockIdx.x * 16 + (slot)] = (v); } while (0)
-#else
-#define U2_T0()
-#define U2_ACC(var)
-#define U2_PUT(slot, v)
-#endif
 
 constexpr int U2_THREADS = 448;
 constexpr int U2_EPI_WARP0 = 4;   // epilogue warps 4..11
@@ -111,16 +96,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
   const int total = m_pairs * P.ngroups;
   const int cluster_id = blockIdx.x >> 1, nclusters = gridDim.x >> 1;
   const int kb_total = P.kblocks[0] + (P.nseg > 1 ? P.kblocks[1] : 0);
-#ifdef GTE_EXPERIMENTS
-  auto stamp = [&](int t, int slot) {
-    if (P.dbg && blockIdx.x < 148) {
-      const int i = (t - cluster_id) / nclusters;
-      if (i < 16) g_umma2_dbg[(blockIdx.x * 16 + i) * 8 + slot] = clock64();
-    }
-  };
-#else
-  auto stamp = [](int, int) {};
-#endif
 
   for (int i = threadIdx.x; i < UM_MAX_BN; i += U2_THREADS) {
     s_bias[i] = (P.bias && i < P.bias_n) ? P.bias[i] : 0.f;
@@ -173,25 +148,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
           }
         }
       };
-#ifdef GTE_EXPERIMENTS
-      if (P.dbg & 32) pf_t = total;  // timing experiment: no L2 prefetch
-#endif
       for (int i = 0; i < U2_PREFETCH; ++i) pf_step();
-      long long w_pe = 0, n_kb = 0;
-      const long long t_begin = clock64();
-      (void)w_pe; (void)n_kb; (void)t_begin;
       for (int t = cluster_id; t < total; t += nclusters) {
         const int mt = 2 * (t / P.ngroups) + (int)rank, grp = t % P.ngroups;
-        stamp(t, 7);
         for (int seg = 0; seg < P.nseg; ++seg) {
           for (int kb = 0; kb < P.kblocks[seg]; ++kb) {
             pf_step();
-            ++n_kb;
-            {
-              U2_T0();
-              mbar_wait_cluster_backoff(smem_u32(&bar_empty[stage]), phase ^ 1);
-              U2_ACC(w_pe);
-            }
+            mbar_wait_cluster_backoff(smem_u32(&bar_empty[stage]), phase ^ 1);
             const uint32_t fb = smem_u32(&bar_full[stage]);
             mbar_expect_tx(fb, (uint32_t)UM_A_BYTES + 2u * L.bh_bytes);
             tma_load_2d(smem_u32(sA_hi_p(stage)), &P.tmA[seg], fb, kb * UM_BK, mt * UM_BM);
@@ -201,9 +164,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
           }
         }
       }
-      U2_PUT(0, clock64() - t_begin);
-      U2_PUT(1, w_pe);
-      U2_PUT(9, n_kb);
     }
   } else if (warp == 1) {
     // ================================ MMA issuer (leader CTA) =================================
@@ -215,26 +175,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
       int acc = 0;
       uint32_t acc_phase = 0;
       constexpr int nacc = SPLIT ? 1 : 2;
-      long long w_mt = 0, w_mr = 0;
-      const long long t_begin = clock64();
-      (void)w_mt; (void)w_mr; (void)t_begin;
       for (int t = cluster_id; t < total; t += nclusters) {
-        stamp(t, 4);
-        {
-          U2_T0();
-          mbar_wait_cluster(smem_u32(&bar_tempty[acc]), acc_phase ^ 1);
-          U2_ACC(w_mt);
-        }
+        mbar_wait_cluster(smem_u32(&bar_tempty[acc]), acc_phase ^ 1);
         tc_fence_after();
-        stamp(t, 5);
         const uint32_t d_tmem = tmem_base + (uint32_t)(acc * UM_ACC_STRIDE);
         const uint32_t d_cross = SPLIT ? tmem_base + UM_ACC_STRIDE : d_tmem;
         for (int kb = 0; kb < kb_total; ++kb) {
-          {
-            U2_T0();
-            mbar_wait_cluster(smem_u32(&bar_ready[stage]), phase);
-            U2_ACC(w_mr);
-          }
+          mbar_wait_cluster(smem_u32(&bar_ready[stage]), phase);
           tc_fence_after();
           const uint64_t dah = make_desc_k_sw128(smem_u32(sA_hi_p(stage)));
           const uint64_t dal = make_desc_k_sw128(smem_u32(sA_lo_p(stage)));
@@ -250,13 +197,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
           umma_commit_pair(smem_u32(&bar_empty[stage]));
           if (++stage == S) { stage = 0; phase ^= 1; }
         }
-        stamp(t, 6);
         umma_commit_pair(smem_u32(&bar_tfull[acc]));
         if (++acc == nacc) { acc = 0; acc_phase ^= 1; }
       }
-      U2_PUT(4, w_mt);
-      U2_PUT(5, w_mr);
-      U2_PUT(6, clock64() - t_begin);
     }
   } else if (warp < U2_EPI_WARP0 || warp >= U2_EPI_WARP0 + U2_EPI_WARPS) {
     // ================================ operand split (warps 2, 3, 12, 13) ======================
@@ -264,16 +207,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
     const uint32_t ready_leader = mapa_shared(smem_u32(&bar_ready[0]), 0);
     int stage = 0;
     uint32_t phase = 0;
-    long long w_sf = 0, w_sw = 0;
-    (void)w_sf; (void)w_sw;
     for (int tile = cluster_id; tile < total; tile += nclusters) {
       for (int kb = 0; kb < kb_total; ++kb) {
-        {
-          U2_T0();
-          mbar_wait_backoff(smem_u32(&bar_full[stage]), phase);
-          U2_ACC(w_sf);
-        }
-        U2_T0();
+        mbar_wait_backoff(smem_u32(&bar_full[stage]), phase);
         const float4* hi = reinterpret_cast<const float4*>(sA_hi_p(stage));
         float4* lo = reinterpret_cast<float4*>(sA_lo_p(stage));
         // hi stays as TMA wrote it: kind::tf32 reads the top 19 bits of the fp32 word, i.e. a_hi = trunc(a); only the
@@ -290,13 +226,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
         fence_proxy_async();  // generic-proxy writes -> visible to the tensor-core (async) proxy
         __syncwarp();
         if (lane == 0) mbar_arrive_cluster(ready_leader + (uint32_t)stage * 8u);
-        U2_ACC(w_sw);
         if (++stage == S) { stage = 0; phase ^= 1; }
       }
-    }
-    if (t == 0) {
-      U2_PUT(2, w_sf);
-      U2_PUT(3, w_sw);
     }
   } else {
     // ================================ epilogue (warps 4..11) ===================================
@@ -322,8 +253,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
     const int cols_a = min(P.N, c_split * 32);
     const float n_a = (float)cols_a, n_b = (float)(P.N - cols_a), n_all = (float)P.N;
     const float my_n = (SPLIT && half) ? n_b : n_a;
-    long long w_et = 0, w_ew = 0;
-    (void)w_et; (void)w_ew;
     int it = 0;
     for (int t = cluster_id; t < total; t += nclusters, ++it) {
       const int mt = 2 * (t / P.ngroups) + (int)rank, grp = t % P.ngroups;
@@ -332,32 +261,17 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
         acc = half;
         acc_phase = (uint32_t)(it >> 1) & 1u;
       }
-      if (ew == 0 && lane == 0) stamp(t, 0);
-      {
-        U2_T0();
-        mbar_wait_cluster_backoff(smem_u32(&bar_tfull[acc]), acc_phase);
-        U2_ACC(w_et);
-      }
-      U2_T0();
+      mbar_wait_cluster_backoff(smem_u32(&bar_tfull[acc]), acc_phase);
       tc_fence_after();
-      if (ew == 0 && lane == 0) stamp(t, 1);
       const uint32_t t_base = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * UM_ACC_STRIDE);
       const int64_t row0 = (int64_t)mt * UM_BM + q * 32;  // first global row of this warp
       const bool rows_live = row0 < (int64_t)P.M;           // the odd tail tile of the peer CTA has no rows at all
       const bool store_z = P.out[grp] != nullptr && rows_live;
       const bool store_y = P.y != nullptr && rows_live;
       float x[32];
-      const int rows_valid = rows_live ? (int)min((int64_t)32, (int64_t)P.M - row0) : 0;
-      // one 32 x 32 chunk of this warp's rows to `dst` (z / dx or y): a TMA store of the swizzled tile, or the warp's
-      // own row-contiguous global stores (P.tma_store == 2)
-      auto put_chunk = [&](const CUtensorMap* map, float* dst, int64_t ld, int c) {
-#ifdef GTE_EXPERIMENTS
-        if (P.dbg & 2) return;  // timing experiment: no output stores
-#endif
-        if (P.tma_store == 2)
-          epi_store_chunk_lsu(stb, x, dst + row0 * ld + c * 32, ld, rows_valid, P.N - c * 32);
-        else
-          epi_store_chunk_tma(stb, nbuf, store_seq, x, map, c * 32, (int32_t)row0);
+      // one 32 x 32 chunk of this warp's rows (z / dx or y) leaves as a TMA store of the swizzled tile
+      auto put_chunk = [&](const CUtensorMap* map, int c) {
+        epi_store_chunk_tma(stb, nbuf, store_seq, x, map, c * 32, (int32_t)row0);
       };
 #define load_chunk(c) epi_load_chunk<SPLIT>(t_base + (c) * 32, s_bias + (c) * 32, x)
       if (P.fuse_ln) {
@@ -373,9 +287,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
             for (int j = 0; j < 32; ++j) s0 += (j < nv) ? x[j] : 0.f;
             shift = s0 / (float)nv;
           }
-#ifdef GTE_EXPERIMENTS
-          if (P.dbg & 8) { s1 += x[0]; s2 += x[1]; } else  // timing experiment: no statistics math
-#endif
           if (nv == 32) {
 #pragma unroll
             for (int j = 0; j < 32; ++j) {
@@ -391,7 +302,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
               s2 = fmaf(d, d, s2);
             }
           }
-          if (store_z) put_chunk(&P.tmOut[grp], P.out[grp], P.ldo[grp], c);
+          if (store_z) put_chunk(&P.tmOut[grp], c);
         }
         float mh = 0.f, m2h = 0.f;
         if (my_n > 0.f) {
@@ -422,40 +333,29 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
             P.rstd[grow] = rstd;
           }
         }
-        if (ew == 0 && lane == 0) stamp(t, 2);
         // pass 2: normalise + activation
         for (int c = c_beg; c < c_end; ++c) {
           load_chunk(c);
-#ifdef GTE_EXPERIMENTS
-          if (!(P.dbg & 4))  // timing experiment: no normalisation math
-#endif
           epi_norm_act(x, s_gamma + c * 32, s_beta + c * 32, true, P.relu != 0, mean, rstd);
-          if (store_y) put_chunk(&P.tmY, P.y, P.ldy, c);
+          if (store_y) put_chunk(&P.tmY, c);
         }
       } else {
-        if (ew == 0 && lane == 0) stamp(t, 2);
         for (int c = c_beg; c < c_end; ++c) {
           load_chunk(c);
-          if (store_z) put_chunk(&P.tmOut[grp], P.out[grp], P.ldo[grp], c);
+          if (store_z) put_chunk(&P.tmOut[grp], c);
           if (P.y != nullptr) {
             epi_norm_act(x, s_gamma + c * 32, s_beta + c * 32, false, P.relu != 0, 0.f, 1.f);
-            if (store_y) put_chunk(&P.tmY, P.y, P.ldy, c);
+            if (store_y) put_chunk(&P.tmY, c);
           }
         }
       }
 #undef load_chunk
-      if (ew == 0 && lane == 0) stamp(t, 3);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(tempty_leader + (uint32_t)acc * 8u);
       if constexpr (SPLIT) {
         if (++acc == nacc) { acc = 0; acc_phase ^= 1; }
       }
-      U2_ACC(w_ew);
-    }
-    if (ew == 0 && lane == 0) {
-      U2_PUT(7, w_et);
-      U2_PUT(8, w_ew);
     }
     if (lane == 0) tma_store_wait_all();  // shared store tiles must outlive their TMA reads
   }
@@ -508,7 +408,6 @@ int launch_umma_pair(UmmaArgs& a, cudaStream_t st) {
   if (stages < 2) return fail(GTE_ERR_UNSUPPORTED, "k_umma_gemm_pair: BN=%d does not fit shared memory", a.BN);
   a.stages = stages;
   a.epi_bufs = epi_bufs;
-  if (tuning(GTE_TUNE_EPI_STORE) == 1) a.tma_store = 2;
   const size_t smem = 1024 + (size_t)u2_layout(a.BN, a.stages, a.epi_bufs).total;
   if (int rc = ensure_dynamic_smem(reinterpret_cast<const void*>(&k_umma_gemm_pair<true>), smem, "k_umma_gemm_pair")) return rc;
   if (int rc = ensure_dynamic_smem(reinterpret_cast<const void*>(&k_umma_gemm_pair<false>), smem, "k_umma_gemm_pair")) return rc;
@@ -519,27 +418,12 @@ int launch_umma_pair(UmmaArgs& a, cudaStream_t st) {
   if (clusters < 1) return GTE_OK;
   // same SPLIT rule as the single-CTA kernel: contractions of one or two k-blocks keep one accumulator per TMEM stage
   // (two stages: the epilogue of tile i overlaps the MMAs of tile i+1)
-  if (kb_total > 2 && tuning(GTE_TUNE_UMMA_SPLIT) != 0)
+  if (kb_total > 2)
     k_umma_gemm_pair<true><<<2 * clusters, U2_THREADS, smem, st>>>(a);
   else
     k_umma_gemm_pair<false><<<2 * clusters, U2_THREADS, smem, st>>>(a);
   GTE_CHECK_LAUNCH("k_umma_gemm_pair");
   return GTE_OK;
-}
-
-int umma_pair_debug_times(int64_t* out_host, int32_t count) {
-#ifdef GTE_EXPERIMENTS
-  if (count == 148 * 16) {  // role accounting
-    GTE_CHECK_CUDA(cudaMemcpyFromSymbol(out_host, g_umma2_acc, (size_t)count * 8), "gte_umma_debug_times");
-    return GTE_OK;
-  }
-  GTE_CHECK_CUDA(cudaMemcpyFromSymbol(out_host, g_umma2_dbg, (size_t)count * 8), "gte_umma_debug_times");
-  return GTE_OK;
-#else
-  (void)out_host;
-  (void)count;
-  return fail(GTE_ERR_UNSUPPORTED, "built without -DGTE_EXPERIMENTS");
-#endif
 }
 
 }  // namespace gte

@@ -40,7 +40,6 @@ struct UmmaArgs {
   int32_t epi_bufs;   // store tiles per epilogue warp (single-CTA kernel: 2 unless shared memory is tight)
   int32_t bias_n;     // number of valid bias entries (the stacked class-layer output is wider than its bias)
   int32_t stages;     // operand ring depth (pair kernel)
-  int32_t dbg;        // GTE_EXPERIMENTS builds only: role timestamps
 };
 
 // launchers (host): return GTE_OK or a recorded failure
@@ -48,11 +47,6 @@ int launch_umma_single(UmmaArgs& a, cudaStream_t st);
 int launch_umma_pair(UmmaArgs& a, cudaStream_t st);
 bool umma_pair_supported(const UmmaArgs& a);
 int setup_weight_maps(UmmaArgs& a, int box_rows);  // tmBhi / tmBlo with the box the chosen kernel stages
-int umma_pair_debug_times(int64_t* out_host, int32_t count);  // GTE_EXPERIMENTS builds
-int umma_dw_debug_times(int64_t* out_host, int32_t count);    // GTE_EXPERIMENTS builds (gte_umma_dw.cu)
-
-// process-wide A/B switches behind gte_set_tuning() (gte_graph.cu)
-int tuning(int key);
 
 // x[j] = accumulator (main [+ cross-term accumulator]) + bias for the 32 columns of one chunk of this thread's row.
 // Everything is compile-time indexed so the 32-register TMEM load windows stay in registers (no local memory).

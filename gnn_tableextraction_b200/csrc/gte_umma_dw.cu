@@ -24,14 +24,12 @@
 // of a stage ran almost back to back); every operand tile arrives as ONE TMA request through a 3-D blocked view of the
 // row-major matrix (r01: one request per 32-column box, 11 per stage -- the TMA unit's request rate was a bound); the
 // operand split writes only the low parts (hi = the raw fp32 word, which kind::tf32 truncates by itself) with batched
-// shared-memory loads, on twelve worker warps that also run the per-chunk epilogue (role accounting,
-// scripts/dw_trace.py: with six split warps the MMA issuer waited 40 % of the time for split operands).
+// shared-memory loads, on twelve worker warps that also run the per-chunk epilogue (role accounting of an instrumented
+// build: with six split warps the MMA issuer waited 40 % of the time for split operands).
 //
 // Roofline: HBM (each activation byte is read once per use) -- the MMA work is 3*2*n*M*N flops.
 #include "gte_common.cuh"
 #include "gte_umma_ptx.cuh"
-
-#include <stdlib.h>
 
 namespace gte {
 
@@ -42,17 +40,6 @@ constexpr int DW_MAX_STAGES = 8;
 constexpr int DW_WORKERS = 12;                 // warps 2..13: operand split per stage + epilogue per chunk
 constexpr int DW_SPLIT_THREADS = DW_WORKERS * 32;
 constexpr int DW_MAX_BOXES = 8;
-
-#ifdef GTE_EXPERIMENTS
-// per-CTA role accounting (clock64 cycles): 0 span, 1 producer waits on empty, 2 split waits on full, 3 split work,
-// 4 MMA waits on ready, 5 MMA waits on tempty, 6 epilogue waits on tfull, 7 epilogue work, 8 stages
-__device__ long long g_dw_dbg[148 * 16];
-#define DW_T0() const long long t0__ = clock64()
-#define DW_ACC(var) var += clock64() - t0__
-#else
-#define DW_T0()
-#define DW_ACC(var)
-#endif
 
 struct DwRun {      // consecutive 32-column blocks of one B tensor, consecutive boxes of the shared-memory tile
   int32_t map;      // index into tmB
@@ -80,7 +67,6 @@ struct DwArgs {
   int32_t a_blocked[2];  // tmA[i] is a 3-D blocked map (box = 4 blocks = one m-tile)
   int32_t a_real_boxes;  // 4, or fewer when A is a narrow operand: boxes [a_real_boxes, 4) of the A tile stay zero
   int32_t stages;        // operand ring depth (as many stages as fit: narrow operands get a deeper ring)
-  int32_t dbg;           // GTE_EXPERIMENTS builds
   float* partial;        // [gridDim.x] tiles of [32 * max_boxes columns][128 rows] floats (column-major: row fastest)
   int64_t tile_stride;   // floats per partial tile
 };
@@ -165,19 +151,11 @@ __global__ void __launch_bounds__(DW_THREADS, 1) k_umma_dw(const __grid_constant
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      long long w_acc = 0, n_st = 0;
-      const long long t_begin = clock64();
-      (void)w_acc; (void)n_st; (void)t_begin;
       for (int chunk = first_chunk; chunk < P.nchunks; chunk += peers) {
         const int r0 = chunk * P.chunk_rows;
         const int nkb = chunk_kblocks(chunk);
         for (int kb = 0; kb < nkb; ++kb) {
-          ++n_st;
-          {
-            DW_T0();
-            mbar_wait(smem_u32(&bar_empty[stage]), phase ^ 1);
-            DW_ACC(w_acc);
-          }
+          mbar_wait(smem_u32(&bar_empty[stage]), phase ^ 1);
           const uint32_t fb = smem_u32(&bar_full[stage]);
           mbar_expect_tx(fb, (uint32_t)((AREAL + G.nboxes) * DW_BOX_BYTES));
           const int row = r0 + kb * DW_KB;
@@ -195,13 +173,6 @@ __global__ void __launch_bounds__(DW_THREADS, 1) k_umma_dw(const __grid_constant
           if (++stage == DW_STAGES) { stage = 0; phase ^= 1; }
         }
       }
-#ifdef GTE_EXPERIMENTS
-      if (blockIdx.x < 148) {
-        g_dw_dbg[blockIdx.x * 16 + 0] = clock64() - t_begin;
-        g_dw_dbg[blockIdx.x * 16 + 1] = w_acc;
-        g_dw_dbg[blockIdx.x * 16 + 8] = n_st;
-      }
-#endif
     }
   } else if (warp == 1) {
     // ================================ MMA issuer ==================================
@@ -213,22 +184,12 @@ __global__ void __launch_bounds__(DW_THREADS, 1) k_umma_dw(const __grid_constant
       const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(BN >> 3) << 17) |
                              ((uint32_t)(128 >> 4) << 24);
       const uint32_t d_main = tmem_base, d_cross = tmem_base + 256;
-      long long w_ready = 0, w_tempty = 0;
-      (void)w_ready; (void)w_tempty;
       for (int chunk = first_chunk; chunk < P.nchunks; chunk += peers) {
-        {
-          DW_T0();
-          mbar_wait_backoff(smem_u32(bar_tempty), acc_phase ^ 1);
-          DW_ACC(w_tempty);
-        }
+        mbar_wait_backoff(smem_u32(bar_tempty), acc_phase ^ 1);
         tc_fence_after();
         const int nkb = chunk_kblocks(chunk);
         for (int kb = 0; kb < nkb; ++kb) {
-          {
-            DW_T0();
-            mbar_wait(smem_u32(&bar_ready[stage]), phase);
-            DW_ACC(w_ready);
-          }
+          mbar_wait(smem_u32(&bar_ready[stage]), phase);
           tc_fence_after();
           const uint64_t dah = make_desc_mn_sw128_32b(smem_u32(sA_hi(stage)), DW_BOX_BYTES);
           const uint64_t dal = make_desc_mn_sw128_32b(smem_u32(sA_lo(stage)), DW_BOX_BYTES);
@@ -248,12 +209,6 @@ __global__ void __launch_bounds__(DW_THREADS, 1) k_umma_dw(const __grid_constant
         umma_commit(smem_u32(bar_tfull));
         acc_phase ^= 1;
       }
-#ifdef GTE_EXPERIMENTS
-      if (blockIdx.x < 148) {
-        g_dw_dbg[blockIdx.x * 16 + 4] = w_ready;
-        g_dw_dbg[blockIdx.x * 16 + 5] = w_tempty;
-      }
-#endif
     }
   } else {
     // ================================ worker warps (2..13) ========================
@@ -274,18 +229,11 @@ __global__ void __launch_bounds__(DW_THREADS, 1) k_umma_dw(const __grid_constant
     const int ones_col = G.ones_b_col >= 0 ? G.ones_b_col : ((G.ones_a_col >= 0 && G.ones_a_col / 128 == mt) ? G.ones_a_col % 128 : -1);
     float* const ptile = P.partial + (int64_t)blockIdx.x * P.tile_stride + q * 32 + lane;
     bool first = true;
-    long long w_full = 0, w_work = 0, w_tfull = 0, w_epi = 0;
-    (void)w_full; (void)w_work; (void)w_tfull; (void)w_epi;
     for (int chunk = first_chunk; chunk < P.nchunks; chunk += peers) {
       const int r0 = chunk * P.chunk_rows;
       const int nkb = chunk_kblocks(chunk);
       for (int kb = 0; kb < nkb; ++kb) {
-        {
-          DW_T0();
-          mbar_wait(smem_u32(&bar_full[stage]), phase);
-          DW_ACC(w_full);
-        }
-        DW_T0();
+        mbar_wait(smem_u32(&bar_full[stage]), phase);
         constexpr int PER = ((4 + DW_MAX_BOXES) * DW_BOX_BYTES / 16 + DW_SPLIT_THREADS - 1) / DW_SPLIT_THREADS;  // 4
         float4 v[PER];
         const float4* a_hi = reinterpret_cast<const float4*>(sA_hi(stage));
@@ -326,16 +274,10 @@ __global__ void __launch_bounds__(DW_THREADS, 1) k_umma_dw(const __grid_constant
         fence_proxy_async();
         __syncwarp();
         if (lane == 0) mbar_arrive(smem_u32(&bar_ready[stage]));
-        DW_ACC(w_work);
         if (++stage == DW_STAGES) { stage = 0; phase ^= 1; }
       }
       // ---- epilogue of this chunk
-      {
-        DW_T0();
-        mbar_wait(smem_u32(bar_tfull), acc_phase);
-        DW_ACC(w_tfull);
-      }
-      DW_T0();
+      mbar_wait(smem_u32(bar_tfull), acc_phase);
       tc_fence_after();
       const uint32_t t_base = tmem_base + ((uint32_t)(q * 32) << 16);
       for (int c = third; c < G.nboxes && epi_rows; c += 3) {
@@ -360,16 +302,7 @@ __global__ void __launch_bounds__(DW_THREADS, 1) k_umma_dw(const __grid_constant
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_u32(bar_tempty));
       acc_phase ^= 1;
-      DW_ACC(w_epi);
     }
-#ifdef GTE_EXPERIMENTS
-    if (blockIdx.x < 148 && threadIdx.x == 64) {
-      g_dw_dbg[blockIdx.x * 16 + 2] = w_full;
-      g_dw_dbg[blockIdx.x * 16 + 3] = w_work;
-      g_dw_dbg[blockIdx.x * 16 + 6] = w_tfull;
-      g_dw_dbg[blockIdx.x * 16 + 7] = w_epi;
-    }
-#endif
     if (first) {  // a CTA without any chunk still owns a partial tile: it must read as zero
       for (int c = third; c < G.nboxes && epi_rows; c += 3)
         for (int j = 0; j < 32; ++j) ptile[(int64_t)(c * 32 + j) * 128] = 0.f;
@@ -500,9 +433,6 @@ static int dw_launch(DwArgs& a, DwReduceArgs& r, cudaStream_t st) {
     a.nchunks = 0;
     grid = 0;
   }
-#ifdef GTE_EXPERIMENTS
-  if (const char* e = getenv("GTE_DW_DBG")) a.dbg = atoi(e);
-#endif
   a.tile_stride = (int64_t)32 * a.max_boxes * 128;
   r.tile_stride = a.tile_stride;
   r.grid = grid;
@@ -529,27 +459,12 @@ static int dw_launch(DwArgs& a, DwReduceArgs& r, cudaStream_t st) {
   return GTE_OK;
 }
 
-int umma_dw_debug_times(int64_t* out_host, int32_t count) {
-#ifdef GTE_EXPERIMENTS
-  if (count > 148 * 16) count = 148 * 16;
-  GTE_CHECK_CUDA(cudaMemcpyFromSymbol(out_host, g_dw_dbg, (size_t)count * 8), "gte_umma_debug_times");
-  return GTE_OK;
-#else
-  (void)out_host;
-  (void)count;
-  return fail(GTE_ERR_UNSUPPORTED, "built without -DGTE_EXPERIMENTS");
-#endif
-}
-
 static int boxes_of(int k) { return (k + 31) / 32; }
 
 // Operand map: the 3-D blocked view (one TMA request per run of 32-column blocks) when every block lies inside the row's
 // leading dimension, 2-D boxes (one request per block, columns past `cols` zero filled) otherwise.
 static int dw_make_map(CUtensorMap* m, int32_t* blocked, const float* p, int64_t rows, int64_t cols, int64_t ld, int box_blocks) {
   *blocked = (box_blocks > 1 && ld >= 32 * ((cols + 31) / 32)) ? 1 : 0;
-#ifdef GTE_EXPERIMENTS
-  if (const char* e = getenv("GTE_DW_DBG")) if (atoi(e) & 2) *blocked = 0;
-#endif
   if (*blocked) {
     if (make_tmap_3d_blocks(m, p, rows, cols, ld, DW_KB, box_blocks, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B) == GTE_OK) return GTE_OK;
     *blocked = 0;  // a driver that refuses the overlapping strides: plain boxes

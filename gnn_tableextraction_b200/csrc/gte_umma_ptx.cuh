@@ -333,38 +333,6 @@ __device__ __forceinline__ void epi_store_chunk(float* st, const float (&v)[32],
   }
 }
 
-// Same transpose through a warp-private 4096-byte tile in the swizzled layout of epi_store_chunk_tma, drained by the
-// warp itself with row-contiguous 128-bit global stores (4 rows x 128 bytes per instruction) instead of a TMA store:
-// no asynchronous reader, so ONE tile per warp suffices.  `out` points at (first row of the warp, first column of the
-// chunk); rows 16-byte aligned (ld % 4 == 0).  Columns at or past cols_valid are never written.
-__device__ __forceinline__ void epi_store_chunk_lsu(uint8_t* buf, const float (&v)[32], float* out, int64_t ld,
-                                                    int rows_valid, int cols_valid) {
-  const int lane = threadIdx.x & 31;
-  __syncwarp();  // the previous chunk's reads of this tile are done
-  float* rowp = reinterpret_cast<float*>(buf) + lane * 32;
-#pragma unroll
-  for (int q = 0; q < 8; ++q)
-    *reinterpret_cast<float4*>(rowp + ((q ^ (lane & 7)) << 2)) = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
-  __syncwarp();
-  const int r_in = lane >> 3, cq = lane & 7, c4 = cq * 4;
-  if (c4 >= cols_valid) return;
-  const bool full = c4 + 4 <= cols_valid;
-#pragma unroll
-  for (int it = 0; it < 8; ++it) {
-    const int row = it * 4 + r_in;
-    if (row >= rows_valid) break;
-    const float4 val = *reinterpret_cast<const float4*>(reinterpret_cast<const float*>(buf) + row * 32 + ((cq ^ (row & 7)) << 2));
-    float* p = out + (int64_t)row * ld + c4;
-    if (full) {
-      *reinterpret_cast<float4*>(p) = val;
-    } else {
-      p[0] = val.x;
-      if (c4 + 1 < cols_valid) p[1] = val.y;
-      if (c4 + 2 < cols_valid) p[2] = val.z;
-    }
-  }
-}
-
 // ------------------------------------------------------------ host: TMA descriptors ----
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,

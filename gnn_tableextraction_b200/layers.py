@@ -17,7 +17,6 @@ SpMM on the CSR (deterministic, no atomics).  Nothing here runs on the CPU.
 """
 from __future__ import annotations
 
-import os
 from dataclasses import dataclass, field
 from typing import Optional
 
@@ -26,10 +25,8 @@ import torch
 from . import _lib, ops
 from .graph import PageGraphBatch
 
-# Dense-contraction route: "auto" sends wide hidden layers (a real dense contraction, SURVEY 8a)
-# to the tcgen05 3xTF32 kernels and everything else to the exact-fp32 FFMA kernels;
-# "ffma" forces the CUDA-core path everywhere, "umma" forces tensor cores wherever supported.
-GEMM_MODE = os.environ.get("GTE_GEMM", "auto")
+# Dense-contraction route: wide hidden layers (a real dense contraction, SURVEY 8a) of batches of at least
+# UMMA_MIN_ROWS nodes go to the tcgen05 3xTF32 kernels and everything else to the exact-fp32 FFMA kernels.
 UMMA_MIN_ROWS = 1024
 UMMA_MIN_WIDTH = 64
 SKINNY_MIN_ROWS = 256  # below this the generic kernels are launch-latency bound anyway
@@ -79,36 +76,28 @@ def pick_strategy(fin: int, fout: int, use_pp: bool) -> str:
 def use_umma(n: int, fin: int, fout: int, *mats) -> bool:
     """Tensor-core projection.  Also used for narrow K (input layer, K = 2*13): the kernel then is an
     output-bandwidth-bound fused bias+LayerNorm+ReLU epilogue, still far ahead of GEMM + separate LayerNorm."""
-    if GEMM_MODE == "ffma" or not ops.umma_supported(fout, fin):
+    if not ops.umma_supported(fout, fin):
         return False
     if not all(ops._aligned_mat(m) for m in mats if m is not None):
         return False
-    if GEMM_MODE == "umma":
-        return True
     return n >= UMMA_MIN_ROWS and max(fin, fout) >= UMMA_MIN_WIDTH
 
 
 def use_umma_dw(n: int, fo: int, k1: int, k2: int, db_needed: bool, *mats) -> bool:
     """Tensor-core weight gradient: any width up to 256 (the reduction over all nodes is the long axis)."""
-    if GEMM_MODE == "ffma" or not ops.umma_bwd_weight_supported(fo, k1, k2):
+    if not ops.umma_bwd_weight_supported(fo, k1, k2):
         return False
     if not all(ops._aligned_mat(m) for m in mats if m is not None):
         return False
     if db_needed and k1 % 32 == 0:
         return False
-    return GEMM_MODE == "umma" or n >= UMMA_MIN_ROWS
-
-
-PAGE_FORMATS = os.environ.get("GTE_PAGE_FORMATS", "1") != "0"  # one-kernel batch assembly (0: individual builders)
-SPMM_MODE = os.environ.get("GTE_SPMM", "auto")  # auto | packed | paged | rows (diagnostics / A-B runs)
+    return n >= UMMA_MIN_ROWS
 
 
 def _use_packed(g: PageGraphBatch, x: torch.Tensor, addend: Optional[torch.Tensor]) -> bool:
     """The persistent page kernel needs a page table, 16-byte aligned rows and two stages of the
     largest page in shared memory; everything else goes to gte_spmm_paged / gte_spmm."""
-    if SPMM_MODE in ("paged", "rows"):
-        return False
-    if 16 < x.shape[1] <= 32 and SPMM_MODE != "packed":
+    if 16 < x.shape[1] <= 32:
         return False  # 5..8 chunks per row: the one-CTA-per-(page, slice) kernel measures faster (conv sweep, F = 32)
     return (ops.paged_packed_supported(g.pages(), x.shape[1]) and ops._aligned_mat(x)
             and (addend is None or ops._aligned_mat(addend)))
@@ -121,8 +110,7 @@ def _agg_mode(agg: str) -> int:
 def aggregate_forward(g: PageGraphBatch, h: torch.Tensor, w_edge: torch.Tensor, agg: str = GCN,
                       addend: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """``update_all(u_mul_e, sum|mean)`` (+ ``* norm``): models.py:53-54,69-71,149."""
-    if PAGE_FORMATS:
-        g.prepare(w_edge)  # first call per batch: CSC + CSR + norm + packed edges in one kernel
+    g.prepare(w_edge)  # first call per batch: CSC + CSR + norm + packed edges in one kernel
     indptr, indices, _ = g.csc()
     if _use_packed(g, h, addend):
         return ops.spmm_packed(indptr, g.packed_edges("csc", w_edge), h, g.pages(), mode=_agg_mode(agg),
@@ -134,8 +122,7 @@ def aggregate_forward(g: PageGraphBatch, h: torch.Tensor, w_edge: torch.Tensor, 
 def aggregate_backward(g: PageGraphBatch, d_out: torch.Tensor, w_edge: torch.Tensor,
                        addend: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """d h[u] = sum_{u->v} w_e * norm[v] * d_out[v] (+ addend[u]) on the CSR (reverse graph)."""
-    if PAGE_FORMATS:
-        g.prepare(w_edge)
+    g.prepare(w_edge)
     indptr, indices, _ = g.csr()
     if _use_packed(g, d_out, addend):
         return ops.spmm_packed(indptr, g.packed_edges("csr", w_edge), d_out, g.pages(), mode=_lib.GTE_AGG_SUM,
@@ -144,19 +131,14 @@ def aggregate_backward(g: PageGraphBatch, d_out: torch.Tensor, w_edge: torch.Ten
                     addend=addend, pages=g.pages(), out=out)
 
 
-COMB = os.environ.get("GTE_COMB", "1") != "0"  # combined [n, 32] operands for the narrow layers (0: two operands, A/B runs)
-# input gradient of an aggregate-first layer when the caller allows it: "agg" = (A_hat^T dz) first, then one projection
-# [dz | A_hat^T dz] W; "layer" = [dz Ws | dz Wn] first, then A_hat^T (dz Wn) + dz Ws (A/B runs)
-DH_ORDER = os.environ.get("GTE_DH_ORDER", "agg")
-
-
 def _comb_rows(n: int) -> bool:
-    return COMB and GEMM_MODE != "ffma" and (GEMM_MODE == "umma" or n >= UMMA_MIN_ROWS)
+    """Combined [n, 32] operands for the narrow layers: a tensor-core batch."""
+    return n >= UMMA_MIN_ROWS
 
 
 def wants_pack(n: int, fin: int, fout: int, use_pp: bool) -> bool:
     """Could sage_layer_forward take a tensor-core branch for this layer (so a caller may pre-pack W for it)?"""
-    return (not use_pp) and GEMM_MODE != "ffma" and (GEMM_MODE == "umma" or n >= UMMA_MIN_ROWS) and ops.umma_supported(fout, fin)
+    return (not use_pp) and n >= UMMA_MIN_ROWS and ops.umma_supported(fout, fin)
 
 
 def wants_class_grad_comb(ctx: "LayerCtx", n: int) -> bool:
@@ -193,7 +175,7 @@ def sage_layer_forward(g: Optional[PageGraphBatch], h: torch.Tensor, w_edge: Opt
         xc = ops.comb_from(h)
         hs, ahs = ops.comb_views(xc, fin)
         h = hs
-    elif GEMM_MODE != "ffma" and h.shape[0] >= UMMA_MIN_ROWS and not ops._aligned_mat(h):
+    elif h.shape[0] >= UMMA_MIN_ROWS and not ops._aligned_mat(h):
         # unaligned rows: one padded copy gives 16-byte aligned rows for TMA / 128-bit loads
         hp = ops.empty_padded(h.shape[0], h.shape[1], h.device)
         hp.copy_(h)
@@ -300,8 +282,7 @@ def sage_layer_backward(g: Optional[PageGraphBatch], ctx: LayerCtx, dy: torch.Te
             ops.linear_bwd_weight(dz, ctx.h, ctx.ah, dW, db, accumulate)
         if not need_dh:
             return None
-        if (dh_agg_first and DH_ORDER == "agg" and drop is None and fout <= fin and ctx.pack is not None
-                and ops._aligned_mat(dz)):
+        if dh_agg_first and drop is None and fout <= fin and ctx.pack is not None and ops._aligned_mat(dz):
             # dh = dz Ws + A_hat^T (dz Wn) = [dz | A_hat^T dz] W: 5 instead of 6 passes over an [n, fin] matrix
             # (the mask of [h | ah] sits between the projection and A_hat^T, hence no dropout)
             return ops.umma_linear_bwd_data2(dz, aggregate_backward(g, dz, ctx.w_edge), ctx.pack, fin)
@@ -325,12 +306,11 @@ def sage_layer_backward(g: Optional[PageGraphBatch], ctx: LayerCtx, dy: torch.Te
         ops.umma_linear_bwd_weight2_comb(dc, fout, ctx.h, dW, 0, fin, db, accumulate)
         return ops.umma_linear_bwd_data_comb(dc, fout, ctx.pack, fin) if need_dh else None
     gq = aggregate_backward(g, dz, ctx.w_edge)
-    if (2 * fout <= 32 and dz.shape[0] >= SKINNY_MIN_ROWS and dW.stride(1) == 1 and GEMM_MODE != "umma"
+    if (2 * fout <= 32 and dz.shape[0] >= SKINNY_MIN_ROWS and dW.stride(1) == 1
             and ops.gram_stream_supported(fin, 2 * fout, ctx.h, dz, gq)):
         # class layer: stream the wide input once against [dz | A^T dz]; the column sums of dz are the bias gradient
         ops.gram_stream(ctx.h, dz, gq, dW, 1, dW.stride(0), dW[:, fin:], 1, dW.stride(0), qsum=db, accumulate=accumulate)
-    elif (GEMM_MODE != "ffma" and fout <= 32 and fin <= 256 and (db is None or fin % 128 != 0) and
-            (GEMM_MODE == "umma" or dz.shape[0] >= UMMA_MIN_ROWS) and
+    elif (fout <= 32 and fin <= 256 and (db is None or fin % 128 != 0) and dz.shape[0] >= UMMA_MIN_ROWS and
             all(ops._aligned_mat(m) for m in (dz, gq, ctx.h))):
         ops.umma_linear_bwd_weight2(dz, gq, ctx.h, dW, 0, fin, db, accumulate)
     else:

@@ -8,7 +8,6 @@ is passed as the leading dimension, so padded / sliced views work unchanged.
 """
 from __future__ import annotations
 
-import os
 from typing import Optional, Tuple
 
 import ctypes as C
@@ -19,7 +18,6 @@ from . import _lib
 from ._lib import GteError, check, lib
 
 _WS = {}
-_LD_ALIGN = max(4, int(os.environ.get("GTE_LD_ALIGN", "32")) // 4 * 4)
 
 
 def _stream() -> int:
@@ -81,9 +79,9 @@ def workspace(nbytes: int, device: torch.device) -> torch.Tensor:
 
 def padded_cols(f: int) -> int:
     """Leading dimension used for internally allocated feature matrices: rows 16-byte aligned (128-bit
-    accesses, TMA); wide rows start on 128-byte lines (``GTE_LD_ALIGN`` floats, default 32) so that a warp's
-    row segments never straddle cache lines -- 218 columns live in 224."""
-    a = _LD_ALIGN if f > _LD_ALIGN else 4
+    accesses, TMA); wide rows start on 128-byte lines (32 floats) so that a warp's row segments never straddle
+    cache lines -- 218 columns live in 224."""
+    a = 32 if f > 32 else 4
     return (f + a - 1) // a * a
 
 

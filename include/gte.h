@@ -40,7 +40,7 @@ extern "C" {
 
 typedef void* gte_stream_t; /* cudaStream_t */
 
-#define GTE_ABI_VERSION 2
+#define GTE_ABI_VERSION 3
 
 #define GTE_OK 0
 #define GTE_ERR_INVALID (-1)     /* bad argument (null pointer, negative size, bad enum) */
@@ -69,22 +69,13 @@ const char* gte_last_error_string(void);
 int64_t gte_launch_count(void);
 
 /*
- * Process-wide A/B switches for tests and measurements (NOT a configuration surface: the defaults are the product
- * path; every value computes the same results through a different kernel).
+ * Process-wide switch for tests (NOT a configuration surface: the default is the product path; either value computes
+ * the same results through a different kernel).
  *   GTE_TUNE_UMMA_PAIR   1 (default): tensor-core projections run on CTA pairs (tcgen05 cta_group::2) when the shape
  *                        allows it; 0: always the single-CTA kernel
- *   GTE_TUNE_DW_PAIR     reserved, no effect (the weight-gradient kernel has one form: a CTA-pair variant would not raise
- *                        its MMA rate and was not built -- DESIGN.md section d)
- *   GTE_TUNE_UMMA_SPLIT  1 (default): contractions of more than two k-blocks keep the 3xTF32 cross terms in their own
- *                        TMEM accumulator; 0: one accumulator (and two accumulator stages) for every shape
- *   GTE_TUNE_EPI_STORE   0 (default): the pair kernel's epilogue leaves through TMA stores; 1: through the epilogue
- *                        warps' own row-contiguous 128-bit global stores
  */
 #define GTE_TUNE_UMMA_PAIR 0
-#define GTE_TUNE_DW_PAIR 1
-#define GTE_TUNE_EPI_STORE 2
-#define GTE_TUNE_UMMA_SPLIT 3
-#define GTE_TUNE_COUNT 4
+#define GTE_TUNE_COUNT 1
 int gte_set_tuning(int key, int value);
 int gte_get_tuning(int key);
 /* SM count and compute capability of the current device. */
@@ -323,10 +314,6 @@ int gte_umma_linear_fwd(const float* x1, int64_t ldx1, const float* x2, int64_t 
 int gte_umma_linear_bwd_data(const float* dz, int64_t lddz, int32_t fo, const float* pack, int32_t nseg,
                              float* dx1, int64_t lddx1, float* dx2, int64_t lddx2, int32_t n, int32_t fin,
                              gte_stream_t stream);
-
-/* Diagnostic (-DGTE_EXPERIMENTS builds; GTE_ERR_UNSUPPORTED otherwise): role timestamps (clock64) of the last tensor-core
- * projection launched with GTE_UMMA_DBG=1; which: 0 = single-CTA kernel, 1 = CTA-pair kernel. */
-int gte_umma_debug_times(int32_t which, int64_t* out_host, int32_t count);
 
 /*
  * Class-layer (fo <= 16) forms of the project-then-aggregate strategy.  `pack` from

@@ -5,7 +5,6 @@ from gnn_tableextraction_b200 import ops
 DEV="cuda"
 def padded(t):
     o = ops.empty_padded(t.shape[0], t.shape[1], DEV); o.copy_(t); return o
-print("GTE_DW_DESC", os.environ.get("GTE_DW_DESC","0"))
 for (n,fo,k) in [(32,128,32),(64,128,32),(512,128,64),(1000,218,218)]:
     g=torch.Generator().manual_seed(1)
     dz=torch.randn(n,fo,generator=g); x=torch.randn(n,k,generator=g)

@@ -14,4 +14,4 @@ e0.record()
 for _ in range(20): fn()
 e1.record(); torch.cuda.synchronize()
 ms=e0.elapsed_time(e1)/20
-print("grid cap", os.environ.get("GTE_LNBWD_GRID","592"), "ln bwd us", ms*1e3, "GB/s", 12*n*f/ms/1e6)
+print("ln bwd us", ms*1e3, "GB/s", 12*n*f/ms/1e6)

@@ -1,4 +1,4 @@
-"""Times the packed page kernel at config-2 conv size under the GTE_SPMM_DBG experiment switches (set per process)."""
+"""Times the packed page kernel at config-2 conv size (DEG, PAGES and F from the environment)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -29,4 +29,4 @@ def t(fn, it=20):
 a = t(lambda: ops.spmm_packed(indptr, pk, x, pg, mode=_lib.GTE_AGG_SUM_NORM, row_norm=norm, out=y))
 b = t(lambda: ops.spmm_packed(indptr, pk, x, pg, mode=_lib.GTE_AGG_SUM, addend=add, out=y))
 c = t(lambda: y.copy_(x))
-print(f"dbg={os.environ.get('GTE_SPMM_DBG','0')} pages={pages} deg={deg} f={f}: fwd {a*1e3:.1f} us, with addend {b*1e3:.1f} us, torch copy x->y {c*1e3:.1f} us")
+print(f"pages={pages} deg={deg} f={f}: fwd {a*1e3:.1f} us, with addend {b*1e3:.1f} us, torch copy x->y {c*1e3:.1f} us")

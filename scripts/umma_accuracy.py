@@ -1,5 +1,4 @@
-"""Experiment (GPU): error of the tcgen05 3xTF32 projection vs fp64, by variant and K.
-Usage: GTE_UMMA_VARIANT={0,1,2,3} python scripts/umma_accuracy.py"""
+"""Experiment (GPU): error of the tcgen05 3xTF32 projection vs fp64, by K."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -14,7 +13,6 @@ def rel(a, b):
 def mask(t):
     return (t.view(torch.int32) & -8192).view(torch.float32)
 
-print("variant", os.environ.get("GTE_UMMA_VARIANT", "0"))
 for fin in (32, 64, 128, 218, 256):
     for exact in (False, True):
         g = torch.Generator().manual_seed(fin)

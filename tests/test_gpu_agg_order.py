@@ -42,6 +42,17 @@ def _spy(monkeypatch, names):
     return calls
 
 
+def _layer_order(monkeypatch):
+    """the trainer's backward with the per-layer input-gradient order: [dz Ws | dz Wn] first, then A_hat^T"""
+    backward = L.sage_layer_backward
+
+    def per_layer(*a, **kw):
+        kw["dh_agg_first"] = False
+        return backward(*a, **kw)
+
+    monkeypatch.setattr(L, "sage_layer_backward", per_layer)
+
+
 def test_umma_bwd_data2_hidden_shape(umma_kernel):
     """dh = dz Ws + G Wn at fo = fin = 218 (K = 2 x 7 k-blocks: the split-accumulator path) against fp64"""
     n, fin, fo = 3001, 218, 218
@@ -60,10 +71,12 @@ def test_config2_step_agg_first_matches_layer_order_and_replays(monkeypatch):
     hb = batch_pages_host(synth.make_pages(512, distinct=48))
     res = {}
     for order in ("layer", "agg"):
-        monkeypatch.setattr(L, "DH_ORDER", order)
-        cm = _models(31)
-        tr = gte.SageTrainer(cm)
-        st = tr.train_step(gte.PageGraphBatch.from_host(hb, DEV)).clone()
+        with monkeypatch.context() as mp:
+            if order == "layer":
+                _layer_order(mp)
+            cm = _models(31)
+            tr = gte.SageTrainer(cm)
+            st = tr.train_step(gte.PageGraphBatch.from_host(hb, DEV)).clone()
         res[order] = (st, {k: p.grad.clone() for k, p in cm.named_parameters()}, tr.flat_param.clone())
     assert rel_err(res["agg"][0], res["layer"][0]) < 1e-6
     for k, gl in res["layer"][1].items():
@@ -85,7 +98,7 @@ def test_trainer_step_launch_count_and_order(monkeypatch):
     tr.train_step(gte.PageGraphBatch.from_host(hb, DEV))
     assert lib.gte_launch_count() - c0 == 28
     assert calls == {"umma_linear_bwd_data": 0, "umma_linear_bwd_data2": 1}
-    monkeypatch.setattr(L, "DH_ORDER", "layer")
+    _layer_order(monkeypatch)
     c0 = lib.gte_launch_count()
     tr.train_step(gte.PageGraphBatch.from_host(hb, DEV))
     assert lib.gte_launch_count() - c0 == 28

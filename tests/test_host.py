@@ -34,7 +34,7 @@ def test_library_exports_every_header_symbol():
 
 def test_abi_version_and_error_string():
     l = gte.lib()
-    assert l.gte_abi_version() == _lib.ABI_VERSION == 2
+    assert l.gte_abi_version() == _lib.ABI_VERSION == 3
     assert isinstance(l.gte_last_error_string(), bytes)
     # argument validation happens before any CUDA call: usable without a GPU
     assert l.gte_spmm(None, None, None, None, None, 7, None, 0, None, 0, None, 0, 4, 4, None) == -1
