@@ -277,7 +277,9 @@ def test_relu_l2norm_and_relu(n, f):
 
 
 @pytest.mark.parametrize("n,c,weighted,ldt", [(1000, 9, False, torch.float32), (333, 9, True, torch.int64),
-                                              (50, 5, True, torch.int32), (1, 3, False, torch.float32)])
+                                              (50, 5, True, torch.int32), (1, 3, False, torch.float32),
+                                              (1000, 16, False, torch.float32), (777, 17, True, torch.int64),
+                                              (1025, 33, False, torch.int32), (300, 64, True, torch.float32)])
 def test_cross_entropy(n, c, weighted, ldt):
     gen = torch.Generator().manual_seed(n)
     logits = (torch.randn(n, c, generator=gen) * 3).requires_grad_(True)
@@ -322,7 +324,11 @@ def _log_err(tag, err):
 
 @pytest.mark.parametrize("n,fin,fo,ln,relu,two", [(1000, 218, 218, True, True, True), (129, 64, 64, False, False, True),
                                                   (5000, 100, 130, True, False, True), (128, 32, 16, False, True, False),
-                                                  (3001, 256, 256, True, True, True), (40000, 218, 218, True, True, True)])
+                                                  (3001, 256, 256, True, True, True), (40000, 218, 218, True, True, True)] + [
+    # both sides of the split-accumulator threshold (more than two 32-float k-blocks in all) for one and two segments,
+    # at one full row tile of 128, an odd last tile of the CTA pair and a one-row last tile
+    (n, fin, fo, fo == 250, n != 1153, two) for two, fin in ((False, 64), (False, 65), (True, 32), (True, 33))
+    for fo in (17, 250) for n in (1024, 1153, 1279)])
 def test_umma_linear_fwd_3xtf32(n, fin, fo, ln, relu, two, umma_kernel):
     gen = torch.Generator().manual_seed(n)
     x1 = torch.randn(n, fin, generator=gen)
@@ -354,7 +360,7 @@ def test_umma_linear_fwd_3xtf32(n, fin, fo, ln, relu, two, umma_kernel):
         assert rel_err(rstd, 1.0 / torch.sqrt(z64.var(1, unbiased=False) + 1e-5)) < 3e-6
 
 
-@pytest.mark.parametrize("n,fin,fo", [(1000, 218, 218), (4097, 64, 96), (257, 256, 16)])
+@pytest.mark.parametrize("n,fin,fo", [(1000, 218, 218), (4097, 64, 96), (257, 256, 16), (1279, 33, 17), (1024, 255, 250)])
 def test_umma_linear_bwd_data_3xtf32(n, fin, fo, umma_kernel):
     gen = torch.Generator().manual_seed(n + 1)
     dz = torch.randn(n, fo, generator=gen)
@@ -502,7 +508,8 @@ def test_spmm_paged_packed_wrong_page_table_and_small_capacity():
 
 
 @pytest.mark.parametrize("n,fo,k1,k2,with_db", [(5000, 218, 218, 218, False), (2000, 218, 13, 13, True), (1000, 64, 100, 0, True),
-                                                (513, 256, 256, 256, False), (40000, 218, 218, 218, False), (7, 9, 20, 0, True)])
+                                                (513, 256, 256, 256, False), (40000, 218, 218, 218, False), (7, 9, 20, 0, True),
+                                                (1153, 17, 31, 31, True), (1279, 17, 33, 33, True)])
 def test_umma_linear_bwd_weight_3xtf32(n, fo, k1, k2, with_db, umma_kernel):
     gen = torch.Generator().manual_seed(n + fo)
     dz = torch.randn(n, fo, generator=gen)
