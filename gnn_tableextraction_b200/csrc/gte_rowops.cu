@@ -395,23 +395,19 @@ __global__ void __launch_bounds__(CE_THREADS)
   for (int64_t i = (int64_t)blockIdx.x * CE_THREADS + threadIdx.x; i < n; i += (int64_t)gridDim.x * CE_THREADS) {
     const float* lr = logits + i * ld;
     const int64_t yv = load_label(labels, label_dtype, i);
-    float mx = -INFINITY;
-    int arg = 0;
-    for (int j = 0; j < c; ++j) {
-      const float v = lr[j];
-      if (v > mx) {
-        mx = v;
-        arg = j;
-      }
-    }
+    // torch.argmax and the row maximum in one pass: a NaN row picks a NaN maximum, its se and nll are NaN either way
+    const int arg = row_argmax(lr, c);
+    const float mx = lr[arg];
     float se = 0.f;
     for (int j = 0; j < c; ++j) se += expf(lr[j] - mx);
     if (yv >= 0 && yv < c) {
       const float wv = class_w ? __ldg(class_w + yv) : 1.0f;
-      const float nll = (mx + logf(se)) - lr[yv];
+      // log-sum-exp minus the label's distance below the maximum: both terms are independent of a common offset of the
+      // row (the form mx + logf(se) - lr[y] rounds at the scale of |mx|)
+      const float nll = logf(se) - (lr[yv] - mx);
       loss = fmaf(wv, nll, loss);
       wsum += wv;
-      if constexpr (EVAL) atomicAdd(&hist[(int)yv * c + row_argmax(lr, c)], 1);
+      if constexpr (EVAL) atomicAdd(&hist[(int)yv * c + arg], 1);
     }
     if constexpr (!EVAL) correct += (arg == (int)yv) ? 1.f : 0.f;
   }

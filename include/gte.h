@@ -429,8 +429,10 @@ int gte_relu_bwd(const float* dy, int64_t lddy, const float* z, int64_t ldz, flo
 /* ------------------------------------------------ loss and optimiser ---- */
 /*
  * nn.CrossEntropyLoss(weight=class_w) forward statistics (model_train.py:171,327-328):
- * stats[0] = sum_i w[y_i] * nll_i, stats[1] = sum_i w[y_i], stats[2] = #(argmax == y).
- * The loss is stats[0]/stats[1].  class_w NULL = all ones.  Deterministic.
+ * stats[0] = sum_i w[y_i] * nll_i, stats[1] = sum_i w[y_i], stats[2] = #(argmax == y), argmax as torch.argmax:
+ * the first maximal index, NaN counting as maximal (as gte_eval_accumulate and gte_page_predictions).
+ * nll_i = log(sum_j exp(x_ij - m_i)) - (x_iy - m_i) with m_i the row maximum: its rounding error does not grow
+ * with a common offset of the row.  The loss is stats[0]/stats[1].  class_w NULL = all ones.  Deterministic.
  */
 size_t gte_cross_entropy_workspace_bytes(int32_t n);
 int gte_cross_entropy_fwd(const float* logits, int64_t ld, const void* labels, int label_dtype,
