@@ -319,29 +319,35 @@ __global__ void __launch_bounds__(ROW_THREADS)
   const float* zr = z + row * ldz;
   const float* gr = dy + row * lddy;
   float r[MAXC], g[MAXC];
-  float q = 0.f, dot = 0.f;
+  float q = 0.f;
 #pragma unroll
   for (int c = 0; c < MAXC; ++c) {
     const int col = lane + 32 * c;
     r[c] = col < f ? fmaxf(zr[col], 0.f) : 0.f;
     g[c] = col < f ? gr[col] : 0.f;
     q = fmaf(r[c], r[c], q);
-    dot = fmaf(r[c], g[c], dot);
   }
   const float nrm_raw = sqrtf(warp_sum(q));
-  dot = warp_sum(dot);
-  const bool clamped = !(nrm_raw > eps);
+  // F.normalize divides by norm.clamp_min(eps), whose gradient passes where norm >= eps: only a norm strictly below
+  // eps drops the second term
+  const bool clamped = nrm_raw < eps;
   const float nrm = clamped ? eps : nrm_raw;
+  // d r = (g - y (y.g)) / nrm with y = r / nrm: no power of the norm is formed, so neither overflows nor underflows
+  // where the norm itself is finite and normal
+  float y[MAXC];
+  float dot_y = 0.f;
+#pragma unroll
+  for (int c = 0; c < MAXC; ++c) {
+    y[c] = r[c] / nrm;
+    dot_y = fmaf(y[c], g[c], dot_y);
+  }
+  dot_y = warp_sum(dot_y);
+  if (clamped) dot_y = 0.f;
   float* dr = dz + row * lddz;
 #pragma unroll
   for (int c = 0; c < MAXC; ++c) {
     const int col = lane + 32 * c;
-    if (col < f) {
-      // y = r/nrm ; d r = g/nrm - r * (r.g)/nrm^3   (no second term while the norm is clamped)
-      float d = g[c] / nrm;
-      if (!clamped) d -= r[c] * dot / (nrm * nrm * nrm);
-      dr[col] = r[c] > 0.f ? d : 0.f;
-    }
+    if (col < f) dr[col] = r[c] > 0.f ? (g[c] - y[c] * dot_y) / nrm : 0.f;
   }
 }
 

@@ -399,7 +399,9 @@ int gte_layernorm_act_bwd(const float* dy, int64_t lddy, const float* z, int64_t
                           float* dgamma, float* dbeta, float* dz_colsum, int accumulate,
                           int32_t n, int32_t f, void* ws, size_t ws_bytes, gte_stream_t stream);
 
-/* y = normalize(relu(z)) : F.relu + F.normalize(p=2, dim=1, eps) (models.py:168-169) */
+/* y = normalize(relu(z)) : F.relu + F.normalize(p=2, dim=1, eps) (models.py:168-169).  The backward follows
+ * torch's clamp_min rule: a row norm >= eps is differentiated as a norm, one < eps as the constant eps.  It forms no
+ * power of the norm, so it stays accurate for every row whose sum of squares fits fp32 (|z| below about 1.8e19). */
 int gte_relu_l2norm_fwd(const float* z, int64_t ldz, float eps, float* y, int64_t ldy,
                         int32_t n, int32_t f, gte_stream_t stream);
 int gte_relu_l2norm_bwd(const float* dy, int64_t lddy, const float* z, int64_t ldz, float eps,
