@@ -71,6 +71,8 @@ SIGNATURES = {
     "gte_layernorm_act_bwd": (ci, [vp, i64, vp, i64, vp, vp, vp, vp, ci, vp, i64, vp, vp, vp, ci, i32, i32, vp, sz, vp]),
     "gte_relu_l2norm_fwd": (ci, [vp, i64, f32, vp, i64, i32, i32, vp]),
     "gte_relu_l2norm_bwd": (ci, [vp, i64, vp, i64, f32, vp, i64, i32, i32, vp]),
+    "gte_relu_l2norm_bwd_colsum_workspace_bytes": (sz, [i32, i32]),
+    "gte_relu_l2norm_bwd_colsum": (ci, [vp, i64, vp, i64, f32, vp, i64, vp, ci, i32, i32, vp, sz, vp]),
     "gte_relu_fwd": (ci, [vp, i64, vp, i64, i32, i32, vp]),
     "gte_dropout_concat": (ci, [vp, i64, i32, vp, i64, i32, i32, f32, C.c_uint64, C.c_uint64, vp, vp, i64, vp, i64, vp]),
     "gte_rng_advance": (ci, [vp, i64, vp]),
@@ -108,6 +110,7 @@ GTE_TUNE_UMMA_PAIR = 0
 GTE_AGG_SUM, GTE_AGG_SUM_NORM, GTE_AGG_MEAN = 0, 1, 2
 GTE_NORM_INV_DEG_ZERO, GTE_NORM_INV_DEG_CLAMP = 0, 1
 GTE_LABEL_I64, GTE_LABEL_I32, GTE_LABEL_F32 = 0, 1, 2
+GTE_EPI_NONE, GTE_EPI_LN, GTE_EPI_L2 = 0, 1, 2  # the fuse_ln selector of gte_umma_linear_fwd(_comb)
 
 
 class GteError(RuntimeError):

@@ -309,13 +309,11 @@ __global__ void __launch_bounds__(ROW_THREADS)
   }
 }
 
-template <int MAXC>
-__global__ void __launch_bounds__(ROW_THREADS)
-    k_relu_l2norm_bwd(const float* __restrict__ dy, int64_t lddy, const float* __restrict__ z, int64_t ldz, float eps,
-                      float* __restrict__ dz, int64_t lddz, int32_t n, int32_t f) {
-  const int lane = threadIdx.x & 31;
-  const int64_t row = (int64_t)blockIdx.x * ROW_WARPS + (threadIdx.x >> 5);
-  if (row >= n) return;
+// One warp per row: dz of row `row`; returns nothing, adds dz to cs[] when COLSUM
+template <int MAXC, bool COLSUM>
+__device__ __forceinline__ void relu_l2norm_bwd_row(const float* __restrict__ dy, int64_t lddy, const float* __restrict__ z,
+                                                    int64_t ldz, float eps, float* __restrict__ dz, int64_t lddz,
+                                                    int64_t row, int32_t f, int lane, float (&cs)[MAXC]) {
   const float* zr = z + row * ldz;
   const float* gr = dy + row * lddy;
   float r[MAXC], g[MAXC];
@@ -347,7 +345,51 @@ __global__ void __launch_bounds__(ROW_THREADS)
 #pragma unroll
   for (int c = 0; c < MAXC; ++c) {
     const int col = lane + 32 * c;
-    if (col < f) dr[col] = r[c] > 0.f ? (g[c] - y[c] * dot_y) / nrm : 0.f;
+    if (col < f) {
+      const float o = r[c] > 0.f ? (g[c] - y[c] * dot_y) / nrm : 0.f;
+      dr[col] = o;
+      if constexpr (COLSUM) cs[c] += o;
+    }
+  }
+}
+
+template <int MAXC>
+__global__ void __launch_bounds__(ROW_THREADS)
+    k_relu_l2norm_bwd(const float* __restrict__ dy, int64_t lddy, const float* __restrict__ z, int64_t ldz, float eps,
+                      float* __restrict__ dz, int64_t lddz, int32_t n, int32_t f) {
+  const int lane = threadIdx.x & 31;
+  const int64_t row = (int64_t)blockIdx.x * ROW_WARPS + (threadIdx.x >> 5);
+  if (row >= n) return;
+  float unused[MAXC];
+  relu_l2norm_bwd_row<MAXC, false>(dy, lddy, z, ldz, eps, dz, lddz, row, f, lane, unused);
+}
+
+// the same rows, grid-stride, plus the column sums of dz (the linear-bias gradient): every lane keeps the sums of its
+// columns, the block writes partial[block][f] (warps added in fixed order) for k_reduce_partials
+template <int MAXC>
+__global__ void __launch_bounds__(ROW_THREADS)
+    k_relu_l2norm_bwd_colsum(const float* __restrict__ dy, int64_t lddy, const float* __restrict__ z, int64_t ldz,
+                             float eps, float* __restrict__ dz, int64_t lddz, float* __restrict__ partial, int32_t n,
+                             int32_t f) {
+  extern __shared__ float sm[];  // [ROW_WARPS][f]
+  const int lane = threadIdx.x & 31;
+  const int warp = threadIdx.x >> 5;
+  float cs[MAXC];
+#pragma unroll
+  for (int c = 0; c < MAXC; ++c) cs[c] = 0.f;
+#pragma unroll 1
+  for (int64_t row = (int64_t)blockIdx.x * ROW_WARPS + warp; row < n; row += (int64_t)gridDim.x * ROW_WARPS)
+    relu_l2norm_bwd_row<MAXC, true>(dy, lddy, z, ldz, eps, dz, lddz, row, f, lane, cs);
+#pragma unroll
+  for (int c = 0; c < MAXC; ++c) {
+    const int col = lane + 32 * c;
+    if (col < f) sm[warp * f + col] = cs[c];
+  }
+  __syncthreads();
+  for (int col = threadIdx.x; col < f; col += ROW_THREADS) {
+    float s = 0.f;
+    for (int w = 0; w < ROW_WARPS; ++w) s += sm[w * f + col];
+    partial[(int64_t)blockIdx.x * f + col] = s;
   }
 }
 
@@ -683,7 +725,6 @@ using namespace gte;
     else if ((F) <= 512) KERNEL<16> __VA_ARGS__;                                                    \
     else KERNEL<32> __VA_ARGS__;                                                                    \
   } while (0)
-
 extern "C" {
 
 int gte_layernorm_act_fwd(const float* z, int64_t ldz, const float* gamma, const float* beta, float eps, int relu,
@@ -775,6 +816,38 @@ int gte_relu_l2norm_bwd(const float* dy, int64_t lddy, const float* z, int64_t l
   cudaStream_t st = as_stream(stream);
   GTE_ROW_DISPATCH(k_relu_l2norm_bwd, f, <<<grid, ROW_THREADS, 0, st>>>(dy, lddy, z, ldz, eps, dz, lddz, n, f));
   GTE_CHECK_LAUNCH("k_relu_l2norm_bwd");
+  return GTE_OK;
+}
+
+size_t gte_relu_l2norm_bwd_colsum_workspace_bytes(int32_t n, int32_t f) {
+  if (n < 0 || f <= 0) return 0;
+  return (size_t)ln_bwd_grid(n) * (size_t)f * 4 + 256;
+}
+
+int gte_relu_l2norm_bwd_colsum(const float* dy, int64_t lddy, const float* z, int64_t ldz, float eps, float* dz,
+                               int64_t lddz, float* dz_colsum, int accumulate, int32_t n, int32_t f, void* ws,
+                               size_t ws_bytes, gte_stream_t stream) {
+  GTE_CHECK_ARG(n >= 0 && f > 0, "gte_relu_l2norm_bwd_colsum: bad size");
+  if (f > 1024) return fail(GTE_ERR_UNSUPPORTED, "gte_relu_l2norm_bwd_colsum: f=%d > 1024 not supported", f);
+  GTE_CHECK_ARG(dz_colsum, "gte_relu_l2norm_bwd_colsum: null dz_colsum");
+  GTE_CHECK_ARG(n == 0 || (dy && z && dz), "gte_relu_l2norm_bwd_colsum: null argument");
+  GTE_CHECK_ARG(lddy >= f && ldz >= f && lddz >= f, "gte_relu_l2norm_bwd_colsum: leading dimension < f");
+  const size_t need = gte_relu_l2norm_bwd_colsum_workspace_bytes(n, f);
+  if (ws == nullptr || ws_bytes < need)
+    return fail(GTE_ERR_WORKSPACE, "gte_relu_l2norm_bwd_colsum: workspace %zu < required %zu", ws_bytes, need);
+  cudaStream_t st = as_stream(stream);
+  float* partial = static_cast<float*>(ws);
+  const int grid = ln_bwd_grid(n);
+  if (n > 0) {
+    const size_t smem = (size_t)ROW_WARPS * f * 4;  // 32 KB at f = 1024
+    GTE_ROW_DISPATCH(k_relu_l2norm_bwd_colsum, f,
+                     <<<grid, ROW_THREADS, smem, st>>>(dy, lddy, z, ldz, eps, dz, lddz, partial, n, f));
+    GTE_CHECK_LAUNCH("k_relu_l2norm_bwd_colsum");
+  }
+  // fixed-order second stage over the per-block partials (none when n == 0: zeros, or dz_colsum unchanged)
+  k_reduce_partials<float><<<(unsigned)ceil_div64(f, 32), RED_THREADS, 0, st>>>(partial, n > 0 ? grid : 0, f, f,
+                                                                               dz_colsum, accumulate);
+  GTE_CHECK_LAUNCH("k_reduce_partials");
   return GTE_OK;
 }
 

@@ -225,8 +225,16 @@ __global__ void __launch_bounds__(UM_THREADS, 1) k_umma_gemm(const __grid_consta
       const bool vec_y = P.y != nullptr && ((reinterpret_cast<uintptr_t>(P.y) & 15) == 0) && (P.ldy % 4 == 0);
       float x[32];
 #define load_chunk(c) epi_load_chunk<SPLIT>(t_base + (c) * 32, s_bias + (c) * 32, x)
-      float mean = 0.f, rstd = 1.f;
-      if (P.fuse_ln) {
+      float mean = 0.f, rstd = 1.f, nrm = 1.f;
+      if (P.fuse_ln == UM_EPI_L2) {
+        // one pass over TMEM for ||relu(z)||^2 (column order), y below divides by max(||relu(z)||, eps)
+        float ss = 0.f;
+        for (int c = 0; c < nchunks; ++c) {
+          load_chunk(c);
+          ss = epi_relu_sq_sum(x, min(32, P.N - c * 32), ss);
+        }
+        nrm = fmaxf(sqrtf(ss), P.eps);
+      } else if (P.fuse_ln == UM_EPI_LN) {
         // two passes over TMEM (mean, then centred second moment): exact like nn.LayerNorm; the last chunk
         // is the only one that needs per-column predicates
         const int nfull = P.N / 32, ntail = P.N % 32;
@@ -276,7 +284,10 @@ __global__ void __launch_bounds__(UM_THREADS, 1) k_umma_gemm(const __grid_consta
             epi_store_chunk(st, x, outp + row0 * ldo + c * 32, ldo, rows_valid, P.N - c * 32, vec_out);
         }
         if (P.y != nullptr) {
-          epi_norm_act(x, s_gamma + c * 32, s_beta + c * 32, P.fuse_ln != 0, P.relu != 0, mean, rstd);
+          if (P.fuse_ln == UM_EPI_L2)
+            epi_relu_div(x, nrm);
+          else
+            epi_norm_act(x, s_gamma + c * 32, s_beta + c * 32, P.fuse_ln == UM_EPI_LN, P.relu != 0, mean, rstd);
           if (P.tma_store)
             epi_store_chunk_tma(stb, P.epi_bufs, store_seq, x, &P.tmY, c * 32, (int32_t)row0);
           else if (rows_valid > 0)
@@ -556,7 +567,9 @@ int gte_umma_linear_fwd(const float* x1, int64_t ldx1, const float* x2, int64_t 
   if (!gte_umma_supported(fo, fin)) return fail(GTE_ERR_UNSUPPORTED, "gte_umma_linear_fwd: fo=%d fin=%d unsupported", fo, fin);
   if (n == 0) return GTE_OK;
   GTE_CHECK_ARG(x1 && pack && (z || y), "gte_umma_linear_fwd: null argument (z may be NULL only when y is given)");
-  GTE_CHECK_ARG(!fuse_ln || (gamma && beta && mean && rstd && y), "gte_umma_linear_fwd: fused LayerNorm needs gamma/beta/mean/rstd/y");
+  GTE_CHECK_ARG(fuse_ln >= UM_EPI_NONE && fuse_ln <= UM_EPI_L2, "gte_umma_linear_fwd: fuse_ln must be 0 (none), 1 (LayerNorm) or 2 (ReLU + L2-normalise)");
+  GTE_CHECK_ARG(fuse_ln != UM_EPI_LN || (gamma && beta && mean && rstd && y), "gte_umma_linear_fwd: fused LayerNorm needs gamma/beta/mean/rstd/y");
+  GTE_CHECK_ARG(fuse_ln != UM_EPI_L2 || y, "gte_umma_linear_fwd: fused ReLU + L2-normalise needs y");
   GTE_CHECK_ARG(aligned16(x1) && ldx1 % 4 == 0 && ldx1 >= fin, "gte_umma_linear_fwd: x1 must be 16-byte aligned with ld %% 4 == 0");
   GTE_CHECK_ARG(!x2 || (aligned16(x2) && ldx2 % 4 == 0 && ldx2 >= fin), "gte_umma_linear_fwd: x2 must be 16-byte aligned with ld %% 4 == 0");
   GTE_CHECK_ARG((!z || ldz >= fo) && (!y || ldy >= fo), "gte_umma_linear_fwd: output leading dimension < fo");
@@ -590,8 +603,8 @@ int gte_umma_linear_fwd(const float* x1, int64_t ldx1, const float* x2, int64_t 
   a.mean = mean;
   a.rstd = rstd;
   a.eps = eps;
-  a.fuse_ln = fuse_ln ? 1 : 0;
-  a.relu = relu ? 1 : 0;
+  a.fuse_ln = fuse_ln;
+  a.relu = (relu && fuse_ln != UM_EPI_L2) ? 1 : 0;  // the L2 mode applies its own ReLU
   return launch_umma(a, as_stream(stream));
 }
 
@@ -705,7 +718,9 @@ int gte_umma_linear_fwd_comb(const float* xc, int64_t ldx, int32_t fin, const fl
     return fail(GTE_ERR_UNSUPPORTED, "gte_umma_linear_fwd_comb: fo=%d fin=%d unsupported (fin <= 16)", fo, fin);
   if (n == 0) return GTE_OK;
   GTE_CHECK_ARG(xc && pack && (z || y), "gte_umma_linear_fwd_comb: null argument (z may be NULL only when y is given)");
-  GTE_CHECK_ARG(!fuse_ln || (gamma && beta && mean && rstd && y), "gte_umma_linear_fwd_comb: fused LayerNorm needs gamma/beta/mean/rstd/y");
+  GTE_CHECK_ARG(fuse_ln >= UM_EPI_NONE && fuse_ln <= UM_EPI_L2, "gte_umma_linear_fwd_comb: fuse_ln must be 0 (none), 1 (LayerNorm) or 2 (ReLU + L2-normalise)");
+  GTE_CHECK_ARG(fuse_ln != UM_EPI_LN || (gamma && beta && mean && rstd && y), "gte_umma_linear_fwd_comb: fused LayerNorm needs gamma/beta/mean/rstd/y");
+  GTE_CHECK_ARG(fuse_ln != UM_EPI_L2 || y, "gte_umma_linear_fwd_comb: fused ReLU + L2-normalise needs y");
   GTE_CHECK_ARG(aligned16(xc) && ldx % 4 == 0 && ldx >= 32, "gte_umma_linear_fwd_comb: xc must be 16-byte aligned with ld %% 4 == 0, ld >= 32");
   GTE_CHECK_ARG((!z || ldz >= fo) && (!y || ldy >= fo), "gte_umma_linear_fwd_comb: output leading dimension < fo");
   PackDims d = pack_dims(fo, fin, 2);
@@ -733,8 +748,8 @@ int gte_umma_linear_fwd_comb(const float* xc, int64_t ldx, int32_t fin, const fl
   a.mean = mean;
   a.rstd = rstd;
   a.eps = eps;
-  a.fuse_ln = fuse_ln ? 1 : 0;
-  a.relu = relu ? 1 : 0;
+  a.fuse_ln = fuse_ln;
+  a.relu = (relu && fuse_ln != UM_EPI_L2) ? 1 : 0;  // the L2 mode applies its own ReLU
   return launch_umma(a, as_stream(stream));
 }
 

@@ -25,7 +25,8 @@
 //   warps 4-11      epilogue, TWO warps per TMEM lane quarter.  Split accumulator (long k loops, one TMEM stage): the two
 //                   share a tile, each takes half of the column chunks -- bias, LayerNorm statistics in ONE TMEM pass
 //                   (shifted sums per half, merged with the parallel-variance formula through shared memory), second
-//                   pass normalises + ReLU.  One accumulator (k loops of one or two k-blocks, two TMEM stages): each
+//                   pass normalises + ReLU (the ReLU + L2-normalise epilogue merges the halves' sums of relu(z)^2 the
+//                   same way).  One accumulator (k loops of one or two k-blocks, two TMEM stages): each
 //                   group of four warps owns a stage and takes every second tile, whole rows, no exchange.  z and y
 //                   leave through swizzled shared tiles and TMA stores; one arrive per warp on the leader's tempty
 //
@@ -274,7 +275,30 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(U2_THREADS, 1)
         epi_store_chunk_tma(stb, nbuf, store_seq, x, map, c * 32, (int32_t)row0);
       };
 #define load_chunk(c) epi_load_chunk<SPLIT>(t_base + (c) * 32, s_bias + (c) * 32, x)
-      if (P.fuse_ln) {
+      if (P.fuse_ln == UM_EPI_L2) {
+        // pass 1: z leaves, and this warp's columns add relu(z)^2 in column order
+        float ss = 0.f;
+        for (int c = c_beg; c < c_end; ++c) {
+          load_chunk(c);
+          ss = epi_relu_sq_sum(x, min(32, P.N - c * 32), ss);
+          if (store_z) put_chunk(&P.tmOut[grp], c);
+        }
+        if constexpr (SPLIT) {
+          // the two halves meet through shared memory; both warps add them in the same order, so hold the same bits
+          float2* const st = s_stat + (par * 2) * 128 + q * 32 + lane;
+          st[half * 128] = make_float2(ss, 0.f);
+          asm volatile("bar.sync %0, 64;" ::"r"(1 + q) : "memory");  // the two warps of this lane quarter
+          ss = st[0].x + st[128].x;
+          par ^= 1;
+        }
+        const float nrm = fmaxf(sqrtf(ss), P.eps);
+        // pass 2: y = relu(z) / max(||relu(z)||, eps)
+        for (int c = c_beg; c < c_end; ++c) {
+          load_chunk(c);
+          epi_relu_div(x, nrm);
+          if (store_y) put_chunk(&P.tmY, c);
+        }
+      } else if (P.fuse_ln == UM_EPI_LN) {
         // pass 1: z leaves, and this warp's columns are summed around a shift (the mean of its first chunk), which
         // keeps the one-pass variance as accurate as the two-pass form
         float shift = 0.f, s1 = 0.f, s2 = 0.f;

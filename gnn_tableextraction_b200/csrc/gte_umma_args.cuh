@@ -13,6 +13,11 @@ constexpr int UM_A_BYTES = UM_BM * 128;  // 16 KB
 constexpr int UM_MAX_BN = 256;
 constexpr int UM_ACC_STRIDE = 256;       // TMEM columns per accumulator stage
 
+// UmmaArgs::fuse_ln: the forward epilogue that turns z into y
+constexpr int UM_EPI_NONE = 0;  // y = act(z)
+constexpr int UM_EPI_LN = 1;    // y = act(LayerNorm(z)), mean / rstd per row
+constexpr int UM_EPI_L2 = 2;    // y = relu(z) / max(||relu(z)||_2, eps), nothing saved per row
+
 struct UmmaArgs {
   CUtensorMap tmA[2];       // per K segment: activations [M, K_s], box 32 x 128
   CUtensorMap tmBhi[2][2];  // [group][segment]: packed weights hi [BN, Kpad], box 32 x BN (pair kernel: 32 x BN/2)
@@ -35,7 +40,7 @@ struct UmmaArgs {
   float* mean;
   float* rstd;
   float eps;
-  int32_t fuse_ln, relu;
+  int32_t fuse_ln, relu;    // fuse_ln: UM_EPI_NONE / UM_EPI_LN / UM_EPI_L2
   int32_t tma_store;  // outputs are TMA-store compatible (16-byte aligned, ld % 4 == 0)
   int32_t epi_bufs;   // store tiles per epilogue warp (single-CTA kernel: 2 unless shared memory is tight)
   int32_t bias_n;     // number of valid bias entries (the stacked class-layer output is wider than its bias)
@@ -90,6 +95,22 @@ __device__ __forceinline__ void epi_norm_act(float (&x)[32], const float* gamma_
       x[4 * qd + e] = o;
     }
   }
+}
+
+// sum of relu(x)^2 over the first nv columns of one chunk, added to q in column order
+__device__ __forceinline__ float epi_relu_sq_sum(const float (&x)[32], int nv, float q) {
+#pragma unroll
+  for (int j = 0; j < 32; ++j) {
+    const float r = (j < nv) ? fmaxf(x[j], 0.f) : 0.f;
+    q = fmaf(r, r, q);
+  }
+  return q;
+}
+
+// y = relu(x) / nrm for one chunk (nrm = max(||relu(z)||_2, eps): a division, as k_relu_l2norm_fwd and F.normalize)
+__device__ __forceinline__ void epi_relu_div(float (&x)[32], float nrm) {
+#pragma unroll
+  for (int j = 0; j < 32; ++j) x[j] = fmaxf(x[j], 0.f) / nrm;
 }
 
 }  // namespace gte

@@ -1,4 +1,4 @@
-"""Train / inference step engine for ``GcnSAGE`` on the sm_100a kernels.
+"""Train / inference step engine for ``GcnSAGE`` and ``MeanSAGE`` on the sm_100a kernels.
 
 Restates the train-step envelope of the reference
 (/root/reference/src/models/model_train.py:297,320-332):
@@ -35,13 +35,60 @@ from . import layers as L
 from . import ops
 from ._lib import GteError
 from .graph import PageGraphBatch, page_table
-from .nn import GcnSAGE, _is_relu
+from .nn import GcnSAGE, MeanSAGE, _is_relu
 from .pool import PagePool
 
 
 def _dropout_p(d) -> float:
     """dropout attribute of the reference modules: nn.Dropout or the float 0. (models.py:30-33)"""
     return float(d.p) if isinstance(d, nn.Dropout) else float(d or 0.0)
+
+
+L2_MAX_WIDTH = 1024  # gte_relu_l2norm_fwd / _bwd(_colsum): one warp holds a row
+
+
+@dataclass(frozen=True)
+class LayerSpec:
+    """What one layer of the model computes, read once from its module: the aggregation (``L.GCN`` / ``L.MEAN``),
+    LayerNorm (with its eps), ReLU, ReLU + L2-normalise after the layer (with the normalise eps), the dropout
+    probability on [h | ah] and whether the input is pre-propagated."""
+
+    agg: str
+    ln: bool
+    relu: bool
+    l2: bool
+    eps: float
+    drop_p: float
+    use_pp: bool
+
+
+def model_spec(model) -> Tuple[float, List[LayerSpec]]:
+    """(dropout p on the input features, one LayerSpec per layer) of a ``GcnSAGE`` (models.py:80-116) or a
+    ``MeanSAGE`` (models.py:154-170); a GteError for any other model or for one the kernels cannot run."""
+    if isinstance(model, GcnSAGE):
+        specs = []
+        for layer in model.layers:
+            if layer.activation is not None and not _is_relu(layer.activation):
+                raise GteError("SageTrainer: only activation=F.relu/None is fused; use the nn.Module path otherwise")
+            has_ln = isinstance(layer.lynorm, nn.LayerNorm)
+            specs.append(LayerSpec(agg=L.GCN, ln=has_ln, relu=_is_relu(layer.activation), l2=False,
+                                   eps=float(layer.lynorm.eps) if has_ln else 1e-5, drop_p=_dropout_p(layer.dropout),
+                                   use_pp=bool(layer.use_pp)))
+        return _dropout_p(model.dropout), specs
+    if isinstance(model, MeanSAGE):
+        # every layer but the last is followed by F.relu + F.normalize (eps 1e-12); no dropout, no LayerNorm
+        last = len(model.layers) - 1
+        specs = []
+        for i, layer in enumerate(model.layers):
+            fo = int(layer.linear.weight.shape[0])
+            if i != last and fo > L2_MAX_WIDTH:
+                raise GteError(f"SageTrainer: MeanSAGE hidden width {fo} > {L2_MAX_WIDTH}, the widest row the ReLU + "
+                               "L2-normalise kernels hold")
+            specs.append(LayerSpec(agg=L.MEAN, ln=False, relu=False, l2=i != last, eps=1e-12, drop_p=0.0,
+                                   use_pp=False))
+        return 0.0, specs
+    raise GteError(f"SageTrainer: {type(model).__name__} is not supported; the trainer runs GcnSAGE and MeanSAGE "
+                   "(gnn_tableextraction_b200.nn)")
 
 
 @dataclass(frozen=True)
@@ -336,16 +383,18 @@ class TrainerAdam(torch.optim.Adam):
 
 
 class SageTrainer:
-    def __init__(self, model: GcnSAGE, lr: float = 0.01, weight_decay: float = 5e-4, betas=(0.9, 0.999),
+    """Fused train, validate and predict passes of a ``GcnSAGE`` or a ``MeanSAGE``.  The passes read their inputs
+    from the batch: node features ``g.ndata["feat"]`` and edge weights ``g.edata["feat"]`` -- for a MeanSAGE that is
+    ``model(g, g.ndata["feat"], g.edata["feat"])``."""
+
+    def __init__(self, model, lr: float = 0.01, weight_decay: float = 5e-4, betas=(0.9, 0.999),
                  eps: float = 1e-8, class_weights: Optional[torch.Tensor] = None, process_group=None):
+        in_drop, self._spec = model_spec(model)
         self.model = model
         params = list(model.parameters())
         if not params or not params[0].is_cuda:
             raise GteError("SageTrainer: move the model to a CUDA device first (no CPU path)")
         self.device = params[0].device
-        for layer in model.layers:
-            if layer.activation is not None and not _is_relu(layer.activation):
-                raise GteError("SageTrainer: only activation=F.relu/None is fused; use the nn.Module path otherwise")
         self.class_w = None if class_weights is None else class_weights.to(self.device, torch.float32).contiguous()
         self.pg = process_group
         self.world = 1
@@ -355,7 +404,7 @@ class SageTrainer:
         # Dropout (models.py:30-33,60-61,113): masks come from Philox keyed by (seed, offset) held on the DEVICE, so a
         # captured step draws fresh masks on every replay: every call site of a step uses base offset + its own share,
         # and the base advances once per step (gte_rng_advance, captured with the step).
-        self._drop_p = [_dropout_p(model.dropout)] + [_dropout_p(layer.dropout) for layer in model.layers]
+        self._drop_p = [in_drop] + [sp.drop_p for sp in self._spec]
         self.has_dropout = any(p > 0 for p in self._drop_p)
         gen = torch.cuda.default_generators[self.device.index if self.device.index is not None else torch.cuda.current_device()]
         rank = torch.distributed.get_rank(process_group) if self.world > 1 else 0
@@ -455,16 +504,20 @@ class SageTrainer:
         self.optimizer._opt_called = True
 
     # ----------------------------------------------------------- pieces ----
-    def _layer_args(self, layer):
-        has_ln = isinstance(layer.lynorm, nn.LayerNorm)
-        return (layer.linear.weight.data, None if layer.linear.bias is None else layer.linear.bias.data,
-                layer.lynorm.weight.data if has_ln else None, layer.lynorm.bias.data if has_ln else None, has_ln,
-                layer.lynorm.eps if has_ln else 1e-5, _is_relu(layer.activation))
+    def _layer_params(self, li: int):
+        """(W, b, gamma, beta) parameters of layer ``li`` (gamma / beta None without LayerNorm)"""
+        layer, sp = self.model.layers[li], self._spec[li]
+        return (layer.linear.weight, layer.linear.bias, layer.lynorm.weight if sp.ln else None,
+                layer.lynorm.bias if sp.ln else None)
+
+    def _layer_args(self, li: int):
+        return tuple(None if p is None else p.data for p in self._layer_params(li))
 
     def forward(self, g: PageGraphBatch, keep_ctx: bool = True, layer_outputs: Optional[list] = None,
                 training: bool = False):
-        """Layer loop of ``GcnSAGE.forward`` (models.py:105-116).  ``layer_outputs`` (tests): a list that receives every
-        layer's output tensor (the parity tests read the ReLU on/off patterns from it).  ``training``: dropout active."""
+        """Layer loop of ``GcnSAGE.forward`` (models.py:105-116) or ``MeanSAGE.forward`` (models.py:164-170) on
+        ``g.ndata["feat"]`` / ``g.edata["feat"]``.  ``layer_outputs`` (tests): a list that receives every layer's output
+        tensor (the parity tests read the ReLU on/off patterns from it).  ``training``: dropout active."""
         h = g.ndata["feat"]
         w_edge = g.edata["feat"]
         ctxs: List[L.LayerCtx] = []
@@ -478,19 +531,20 @@ class SageTrainer:
         n_rows = h.shape[0]
         todo = [(li, layer.linear.weight.data, layer.linear.weight.shape[1] // 2)
                 for li, layer in enumerate(self.model.layers)
-                if L.wants_pack(n_rows, layer.linear.weight.shape[1] // 2, layer.linear.weight.shape[0], layer.use_pp)]
+                if L.wants_pack(n_rows, layer.linear.weight.shape[1] // 2, layer.linear.weight.shape[0],
+                                self._spec[li].use_pp)]
         if len(todo) > 1:
             for (li, _, _), pk in zip(todo, ops.umma_pack_weights_batch([(W, fin, 2) for _, W, fin in todo])):
                 packs[li] = pk
-        for li, layer in enumerate(self.model.layers):
-            W, b, gamma, beta, has_ln, eps, relu = self._layer_args(layer)
+        for li, sp in enumerate(self._spec):
+            W, b, gamma, beta = self._layer_args(li)
             drop = None
             if drop_on and self._drop_p[1 + li] > 0:
                 drop = L.DropoutSpec(self._drop_p[1 + li], 0, used, self.rng_dev)
                 used += ops.dropout_counters(h.shape[0], W.shape[1])
-            h, ctx = L.sage_layer_forward(g, h, w_edge, W, b, gamma, beta, ln=has_ln, relu=relu, eps=eps, agg=L.GCN,
-                                          use_pp=layer.use_pp, save_for_backward=keep_ctx, dropout=drop,
-                                          pack=packs.get(li))
+            h, ctx = L.sage_layer_forward(g, h, w_edge, W, b, gamma, beta, ln=sp.ln, relu=sp.relu, eps=sp.eps,
+                                          agg=sp.agg, use_pp=sp.use_pp, save_for_backward=keep_ctx, dropout=drop,
+                                          pack=packs.get(li), l2=sp.l2)
             ctxs.append(ctx if keep_ctx else None)
             if layer_outputs is not None:
                 layer_outputs.append(h)
@@ -500,16 +554,14 @@ class SageTrainer:
     def backward(self, g: PageGraphBatch, ctxs: List[L.LayerCtx], dlogits: torch.Tensor,
                  dy_comb: Optional[torch.Tensor] = None):
         dy = dlogits
-        layers = list(self.model.layers)
-        for i in range(len(layers) - 1, -1, -1):
-            layer = layers[i]
-            W, b, gamma, beta, has_ln, eps, relu = self._layer_args(layer)
-            gv = self._grad_views
+        nl = len(self._spec)
+        gv = self._grad_views
+        for i in range(nl - 1, -1, -1):
+            W, b, gamma, beta = self._layer_params(i)
+            dW, db, dgamma, dbeta = (None if p is None else gv[id(p)] for p in (W, b, gamma, beta))
             dy = L.sage_layer_backward(
-                g, ctxs[i], dy, W, gamma, beta, gv[id(layer.linear.weight)],
-                None if layer.linear.bias is None else gv[id(layer.linear.bias)],
-                gv[id(layer.lynorm.weight)] if has_ln else None, gv[id(layer.lynorm.bias)] if has_ln else None,
-                need_dh=(i > 0), accumulate=False, dy_comb=dy_comb if i == len(layers) - 1 else None,
+                g, ctxs[i], dy, W.data, None if gamma is None else gamma.data, None if beta is None else beta.data,
+                dW, db, dgamma, dbeta, need_dh=(i > 0), accumulate=False, dy_comb=dy_comb if i == nl - 1 else None,
                 dh_agg_first=True)
 
     def _all_reduce(self, t: torch.Tensor):

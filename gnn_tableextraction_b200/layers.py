@@ -7,6 +7,9 @@ autograd derives from them, as explicit kernel sequences:
     ah  = post(v) * sum_{u->v} w_e h[u]           gte_spmm on the CSC
     z   = [h | ah] W^T + b                        gte_linear_fwd (no concat buffer)
     out = relu(LayerNorm(z))                      gte_layernorm_act_fwd
+    out = relu(z) / max(||relu(z)||, eps)         gte_relu_l2norm_fwd (``l2``: MeanSAGE's F.relu + F.normalize)
+
+The tensor-core projection fuses either epilogue (gte_umma_linear_fwd's fuse_ln selector).
 
 Two algebraically equal orders are used (A.(H W2^T) = (A.H) W2^T):
   * ``agg``  aggregate-then-project  (Fin <= Fout: aggregate the narrow input)
@@ -65,6 +68,8 @@ class LayerCtx:
     fout: int = 0
     drop: Optional[DropoutSpec] = None  # the mask of [h | ah] is recomputed from this in the backward pass
     comb: Optional[torch.Tensor] = None  # narrow input (fin <= 16): [h | ah] side by side in one [n, 32] operand
+    l2: bool = False  # out = relu(z) / max(||relu(z)||, l2_eps): the backward recomputes the norm from z
+    l2_eps: float = 1e-12
 
 
 def pick_strategy(fin: int, fout: int, use_pp: bool) -> str:
@@ -131,6 +136,20 @@ def aggregate_backward(g: PageGraphBatch, d_out: torch.Tensor, w_edge: torch.Ten
                     addend=addend, pages=g.pages(), out=out)
 
 
+def relu_l2norm_forward(z: torch.Tensor, eps: float) -> torch.Tensor:
+    """``F.normalize(F.relu(z))`` of a layer whose projection did not fuse it (models.py:167-169)."""
+    return ops.relu_l2norm_fwd(z, eps)
+
+
+def relu_l2norm_backward(dy: torch.Tensor, z: torch.Tensor, eps: float, db: Optional[torch.Tensor],
+                         accumulate: bool) -> torch.Tensor:
+    """dz of ``F.normalize(F.relu(z))`` (the norm recomputed from z); ``db`` (may be None) receives (accumulate: gains)
+    the column sums of dz, the linear-bias gradient, from the same pass."""
+    if db is None:
+        return ops.relu_l2norm_bwd(dy, z, eps)
+    return ops.relu_l2norm_bwd_colsum(dy, z, eps, dz_colsum=db, accumulate=accumulate)
+
+
 def _comb_rows(n: int) -> bool:
     """Combined [n, 32] operands for the narrow layers: a tensor-core batch."""
     return n >= UMMA_MIN_ROWS
@@ -145,7 +164,7 @@ def wants_class_grad_comb(ctx: "LayerCtx", n: int) -> bool:
     """The class layer's backward wants its incoming gradient as the self block of a combined [n, 32] operand
     (d logits | A_hat^T d logits): a caller that PRODUCES that gradient (the trainer's loss backward) builds it with
     ``ops.cross_entropy_bwd_comb`` (or ``ops.comb_from``) and passes the buffer as ``dy_comb``."""
-    return (ctx.strategy == "proj" and not ctx.ln and not ctx.relu and ctx.fout <= ops.COMB_W and ctx.pack is not None
+    return (ctx.strategy == "proj" and not ctx.ln and not ctx.relu and not ctx.l2 and ctx.fout <= ops.COMB_W and ctx.pack is not None
             and _comb_rows(n) and ctx.fin <= 256 and ctx.fin % 32 != 0 and ops._aligned_mat(ctx.h))
     # fin % 32 != 0: the bias gradient rides on a free padding column of the input operand
 
@@ -154,14 +173,19 @@ def sage_layer_forward(g: Optional[PageGraphBatch], h: torch.Tensor, w_edge: Opt
                        W: torch.Tensor, b: Optional[torch.Tensor], gamma: Optional[torch.Tensor],
                        beta: Optional[torch.Tensor], *, ln: bool, relu: bool, eps: float = 1e-5, agg: str = GCN,
                        use_pp: bool = False, strategy: Optional[str] = None, save_for_backward: bool = True,
-                       dropout: Optional[DropoutSpec] = None, pack: Optional[torch.Tensor] = None):
-    """Returns (out [N, Fout], LayerCtx).  ``save_for_backward=False`` (inference): the fused tensor-core epilogue does not
+                       dropout: Optional[DropoutSpec] = None, pack: Optional[torch.Tensor] = None,
+                       l2: bool = False):
+    """Returns (out [N, Fout], LayerCtx).  ``l2`` (MeanSAGE's hidden layers, models.py:167-169): out =
+    relu(z) / max(||relu(z)||_2, eps) with ``eps`` the normalise eps (ln and relu off); the narrow input layer's
+    tensor-core projection fuses it into its epilogue, the other routes run ``ops.relu_l2norm_fwd`` after the layer.  ``save_for_backward=False`` (inference): the fused tensor-core epilogue does not
     write the pre-activation z (it only exists for the backward pass).  ``dropout`` (training): nn.Dropout on the
     concatenation [h | ah * norm] before the linear (models.py:60-61), in-kernel Philox, never materialising the concat.
     ``pack``: ``ops.umma_pack_weights(W, fin, 2)`` of the CURRENT W when the caller already made it (the trainer packs all
     layers in one launch); otherwise the tensor-core branches pack W themselves."""
     fout = W.shape[0]
     fin = W.shape[1] if use_pp else W.shape[1] // 2
+    if l2 and (ln or relu):
+        raise _lib.GteError("sage_layer_forward: l2 is its own epilogue (ReLU included); pass ln=False, relu=False")
     if h.shape[1] != (W.shape[1] if use_pp else fin):
         raise _lib.GteError(f"layer expects {W.shape[1] if use_pp else fin} input features, got {h.shape[1]}")
     st = strategy or pick_strategy(fin, fout, use_pp)
@@ -180,7 +204,8 @@ def sage_layer_forward(g: Optional[PageGraphBatch], h: torch.Tensor, w_edge: Opt
         hp = ops.empty_padded(h.shape[0], h.shape[1], h.device)
         hp.copy_(h)
         h = hp
-    ctx = LayerCtx(strategy=st, agg=agg, h=h, ln=ln, relu=relu, fin=fin, fout=fout, w_edge=w_edge, drop=drop)
+    ctx = LayerCtx(strategy=st, agg=agg, h=h, ln=ln, relu=relu, fin=fin, fout=fout, w_edge=w_edge, drop=drop, l2=l2,
+                   l2_eps=eps if l2 else 1e-12)
     if st == "pp":  # pre-propagated input: plain linear (models.py:49)
         if drop is not None:
             h, _ = ops.dropout_concat(h, None, drop.p, drop.seed, drop.offset, drop.rng_dev)
@@ -201,23 +226,31 @@ def sage_layer_forward(g: Optional[PageGraphBatch], h: torch.Tensor, w_edge: Opt
             ctx.comb = xc
             ctx.pack = pack if pack is not None else ops.umma_pack_weights(W, fin, 2)
             z, y, ctx.mean, ctx.rstd = ops.umma_linear_fwd_comb(xc, fin, ctx.pack, b, fout, gamma=gamma, beta=beta,
-                                                                eps=eps, relu=relu, fuse_ln=ln, want_z=save_for_backward)
+                                                                eps=eps, relu=relu, fuse_ln=ln, want_z=save_for_backward,
+                                                                l2=l2)
             ctx.z = z
             return (y if y is not None else z), ctx
         if use_umma(h.shape[0], fin, fout, h, ah):
-            # tensor cores: projection + bias + LayerNorm + ReLU in one kernel
+            # tensor cores: projection + bias + LayerNorm + ReLU in one kernel.  ReLU + L2-normalise is not fused here:
+            # these k loops (more than two k-blocks) keep one TMEM accumulator stage, whose second epilogue pass holds
+            # up the next tile's MMAs -- at 218 -> 218 the projection followed by gte_relu_l2norm_fwd measured faster
+            # (profiles/meansage_bench.json)
             ctx.pack = pack if pack is not None else ops.umma_pack_weights(W, fin, 2)
             z, y, ctx.mean, ctx.rstd = ops.umma_linear_fwd(h, ah, fin, ctx.pack, b, fout, gamma=gamma, beta=beta,
-                                                           eps=eps, relu=relu, fuse_ln=ln, want_z=save_for_backward)
-            ctx.z = z
-            return (y if y is not None else z), ctx
-        if (ln or not relu) and ops.wide_out_supported(fin, fin, fout, h, ah) and h.shape[0] >= SKINNY_MIN_ROWS:
+                                                           eps=eps, relu=relu, fuse_ln=ln,
+                                                           want_z=save_for_backward or l2)
+            if not l2:
+                ctx.z = z
+                return (y if y is not None else z), ctx
+        elif (ln or not relu) and ops.wide_out_supported(fin, fin, fout, h, ah) and h.shape[0] >= SKINNY_MIN_ROWS:
             # exact-fp32 route for a narrow input (K = 2 * fin <= 32): one streaming pass, bias + LayerNorm + ReLU fused
             z, y, ctx.mean, ctx.rstd = ops.wide_out(h, ah, W.data_ptr(), W.data_ptr() + 4 * fin, 1, W.stride(0), fout, b,
                                                     gamma=gamma, beta=beta, eps=eps, relu=relu, fuse_ln=ln)
-            ctx.z = z
-            return (y if y is not None else z), ctx
-        z = ops.linear_fwd(h, ah, W, b)
+            if not l2:
+                ctx.z = z
+                return (y if y is not None else z), ctx
+        else:
+            z = ops.linear_fwd(h, ah, W, b)
     elif st == "proj":
         if fout <= 16 and use_umma(h.shape[0], fin, fout, h):
             # one tensor-core pass over h: [h Ws^T + b | h Wn^T] side by side, aggregated through column views
@@ -233,6 +266,8 @@ def sage_layer_forward(g: Optional[PageGraphBatch], h: torch.Tensor, w_edge: Opt
     ctx.z = z
     if ln:
         out, ctx.mean, ctx.rstd = ops.layernorm_act_fwd(z, gamma, beta, eps, relu)
+    elif l2:
+        out = relu_l2norm_forward(z, eps)
     elif relu:
         out = ops.relu_fwd(z)
     else:
@@ -255,6 +290,11 @@ def sage_layer_backward(g: Optional[PageGraphBatch], ctx: LayerCtx, dy: torch.Te
         # the linear-bias gradient (column sums of dz) falls out of the same pass
         dz = ops.layernorm_act_bwd(dy, ctx.z, ctx.mean, ctx.rstd, gamma, beta, ctx.relu, dgamma, dbeta, accumulate,
                                    dz_colsum=db)
+        db = None
+    elif ctx.l2:
+        # the same pass yields the linear-bias gradient, so the weight gradient below needs no bias column: every width
+        # <= 256 keeps the tensor-core dW (its bias column needs fin % 32 != 0)
+        dz = relu_l2norm_backward(dy, ctx.z, ctx.l2_eps, db, accumulate)
         db = None
     elif ctx.relu:
         dz = ops.relu_bwd(dy, ctx.z)

@@ -474,10 +474,19 @@ def get_tuning(key: int) -> int:
     return int(lib().gte_get_tuning(int(key)))
 
 
+def _epilogue(fuse_ln: bool, l2: bool) -> int:
+    if fuse_ln and l2:
+        raise GteError("umma_linear_fwd: fuse_ln and l2 are two different epilogues")
+    return _lib.GTE_EPI_L2 if l2 else (_lib.GTE_EPI_LN if fuse_ln else _lib.GTE_EPI_NONE)
+
+
 def umma_linear_fwd(x1, x2, fin: int, pack, bias, fo: int, *, gamma=None, beta=None, eps: float = 1e-5,
-                    relu: bool = False, fuse_ln: bool = False, want_y: bool = False, want_z: bool = True):
+                    relu: bool = False, fuse_ln: bool = False, want_y: bool = False, want_z: bool = True,
+                    l2: bool = False):
     """(z, y, mean, rstd): z = [x1 | x2] W^T + b ; y = act(LN(z)) / act(z) (None unless requested).
-    ``want_z=False`` (inference: nothing is saved for a backward pass) skips the z stores when y exists."""
+    ``l2``: y = relu(z) / max(||relu(z)||_2, eps) per row (F.relu + F.normalize; ``eps`` is the normalise eps, mean
+    and rstd are None).  ``want_z=False`` (inference: nothing is saved for a backward pass) skips the z stores when y
+    exists."""
     x1p, ld1, k1 = _mat(x1, "umma.x1")
     n = x1.shape[0]
     x2p, ld2 = None, 0
@@ -488,7 +497,8 @@ def umma_linear_fwd(x1, x2, fin: int, pack, bias, fo: int, *, gamma=None, beta=N
     if k1 != fin:
         raise GteError("umma_linear_fwd: x1 shape mismatch")
     dev = x1.device
-    need_y = fuse_ln or want_y or relu
+    mode = _epilogue(fuse_ln, l2)
+    need_y = fuse_ln or want_y or relu or l2
     z = empty_padded(n, fo, dev) if (want_z or not need_y) else None
     zp, ldz = (None, 0) if z is None else _mat(z, "umma.z")[:2]
     y = empty_padded(n, fo, dev) if need_y else None
@@ -498,7 +508,7 @@ def umma_linear_fwd(x1, x2, fin: int, pack, bias, fo: int, *, gamma=None, beta=N
     check(
         lib().gte_umma_linear_fwd(x1p, ld1, x2p, ld2, fin, _vec(pack, "pack"), _vec(bias, "bias", n=fo),
                                   _vec(gamma, "gamma", n=fo), _vec(beta, "beta", n=fo), float(eps), 1 if relu else 0,
-                                  1 if fuse_ln else 0, zp, ldz, yp, ldy, _ptr(mean), _ptr(rstd), n, fo, _stream()),
+                                  mode, zp, ldz, yp, ldy, _ptr(mean), _ptr(rstd), n, fo, _stream()),
         "gte_umma_linear_fwd",
     )
     return z, y, mean, rstd
@@ -621,12 +631,14 @@ def _comb(buf, what):
 
 
 def umma_linear_fwd_comb(xc, fin: int, pack, bias, fo: int, *, gamma=None, beta=None, eps: float = 1e-5,
-                         relu: bool = False, fuse_ln: bool = False, want_y: bool = False, want_z: bool = True):
+                         relu: bool = False, fuse_ln: bool = False, want_y: bool = False, want_z: bool = True,
+                         l2: bool = False):
     """umma_linear_fwd for a narrow input (fin <= 16) held as one combined operand xc = [h | A_hat h]."""
     xp, ldx = _comb(xc, "umma_linear_fwd_comb.xc")
     n = xc.shape[0]
     dev = xc.device
-    need_y = fuse_ln or want_y or relu
+    mode = _epilogue(fuse_ln, l2)
+    need_y = fuse_ln or want_y or relu or l2
     z = empty_padded(n, fo, dev) if (want_z or not need_y) else None
     zp, ldz = (None, 0) if z is None else _mat(z, "umma.z")[:2]
     y = empty_padded(n, fo, dev) if need_y else None
@@ -636,7 +648,7 @@ def umma_linear_fwd_comb(xc, fin: int, pack, bias, fo: int, *, gamma=None, beta=
     check(
         lib().gte_umma_linear_fwd_comb(xp, ldx, fin, _vec(pack, "pack"), _vec(bias, "bias", n=fo),
                                        _vec(gamma, "gamma", n=fo), _vec(beta, "beta", n=fo), float(eps),
-                                       1 if relu else 0, 1 if fuse_ln else 0, zp, ldz, yp, ldy, _ptr(mean), _ptr(rstd),
+                                       1 if relu else 0, mode, zp, ldz, yp, ldy, _ptr(mean), _ptr(rstd),
                                        n, fo, _stream()),
         "gte_umma_linear_fwd_comb",
     )
@@ -745,6 +757,23 @@ def relu_l2norm_bwd(dy, z, eps: float = 1e-12, out=None):
         out = empty_padded(n, f, dy.device)
     dzp, lddz, _ = _mat(out, "l2_bwd.dz")
     check(lib().gte_relu_l2norm_bwd(dyp, lddy, zp, ldz, float(eps), dzp, lddz, n, f, _stream()), "gte_relu_l2norm_bwd")
+    return out
+
+
+def relu_l2norm_bwd_colsum(dy, z, eps: float = 1e-12, dz_colsum=None, accumulate=False, out=None):
+    """``relu_l2norm_bwd`` (the same dz bits) that also writes ``dz_colsum`` [f] (+)= the column sums of dz: the bias
+    gradient of the linear before the normalisation, in a fixed-order two-stage reduction."""
+    dyp, lddy, f = _mat(dy, "l2_bwd.dy")
+    zp, ldz, _ = _mat(z, "l2_bwd.z")
+    n = dy.shape[0]
+    if out is None:
+        out = empty_padded(n, f, dy.device)
+    dzp, lddz, _ = _mat(out, "l2_bwd.dz")
+    l = lib()
+    ws = workspace(l.gte_relu_l2norm_bwd_colsum_workspace_bytes(n, f), dy.device)
+    check(l.gte_relu_l2norm_bwd_colsum(dyp, lddy, zp, ldz, float(eps), dzp, lddz, _vec(dz_colsum, "dz_colsum", n=f),
+                                       1 if accumulate else 0, n, f, ws.data_ptr(), ws.numel(), _stream()),
+          "gte_relu_l2norm_bwd_colsum")
     return out
 
 

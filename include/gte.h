@@ -303,8 +303,14 @@ int gte_umma_pack_weights_batch(const gte_pack_desc_t* descs, int32_t count, gte
 int gte_umma_pack_weights(const float* W, int64_t ldw, int32_t fo, int32_t fin, int32_t nseg,
                           float* pack, gte_stream_t stream);
 /*
- * z = x1 W[:, :fin]^T (+ x2 W[:, fin:]^T) + bias ; y = act(LayerNorm(z)) when
- * fuse_ln (mean/rstd [n] saved), else y = act(z) when y != NULL.  x2 may be NULL.
+ * z = x1 W[:, :fin]^T (+ x2 W[:, fin:]^T) + bias, then the epilogue `fuse_ln` selects:
+ *   0  y = act(z) when y != NULL
+ *   1  y = act(LayerNorm(z; gamma, beta, eps)), mean / rstd [n] saved
+ *   2  y = relu(z) / max(||relu(z)||_2, eps) per row (F.relu + F.normalize, models.py:167-169; a division by the
+ *      clamped norm, as gte_relu_l2norm_fwd).  `relu` is ignored, y is required, gamma / beta / mean / rstd may be
+ *      NULL and nothing is saved per row: gte_relu_l2norm_bwd(_colsum) recomputes the norm from z.
+ * z may be NULL when y is given (inference).  The z bits do not depend on the epilogue, and the y bits not on
+ * whether z is written.  x2 may be NULL.
  */
 int gte_umma_linear_fwd(const float* x1, int64_t ldx1, const float* x2, int64_t ldx2, int32_t fin,
                         const float* pack, const float* bias, const float* gamma, const float* beta,
@@ -355,7 +361,8 @@ int gte_umma_linear_bwd_weight2(const float* dz1, int64_t lddz1, const float* dz
  * [0, w) and [16, 16+w), every other column FINITE (zero): the narrow side of each contraction is then
  * a single k-block / a single full-row TMA box.  Same results contract as the two-operand forms they
  * replace (models.py:47-62 with `pool` aggregation; concat order self | neighbour):
- *   fwd_comb          (fin <= 16)  z = [xc[:, :fin] | xc[:, 16:16+fin]] W^T + b, epilogue as gte_umma_linear_fwd
+ *   fwd_comb          (fin <= 16)  z = [xc[:, :fin] | xc[:, 16:16+fin]] W^T + b, epilogue (all three fuse_ln
+ *                                  modes) as gte_umma_linear_fwd
  *   bwd_data_comb     (fo  <= 16)  dx = dc[:, :fo] W[:, :fin] + dc[:, 16:16+fo] W[:, fin:2 fin]
  *   bwd_weight_comb   (w   <= 16)  dW[:, :w] (+)= dz^T xc[:, :w] ; dW[:, w:2w] (+)= dz^T xc[:, 16:16+w] ;
  *                                  db (+)= colsum(dz) (needs w < 16)
@@ -406,6 +413,13 @@ int gte_relu_l2norm_fwd(const float* z, int64_t ldz, float eps, float* y, int64_
                         int32_t n, int32_t f, gte_stream_t stream);
 int gte_relu_l2norm_bwd(const float* dy, int64_t lddy, const float* z, int64_t ldz, float eps,
                         float* dz, int64_t lddz, int32_t n, int32_t f, gte_stream_t stream);
+/* gte_relu_l2norm_bwd (the same dz bits) that also writes dz_colsum[f] (+)= the column sums of dz, i.e. the bias
+ * gradient of the nn.Linear before the normalisation: per-block partials in fixed order, then a fixed-order reduction
+ * over the blocks (deterministic).  n == 0 writes zeros (accumulate: leaves dz_colsum unchanged).  f <= 1024. */
+size_t gte_relu_l2norm_bwd_colsum_workspace_bytes(int32_t n, int32_t f);
+int gte_relu_l2norm_bwd_colsum(const float* dy, int64_t lddy, const float* z, int64_t ldz, float eps,
+                               float* dz, int64_t lddz, float* dz_colsum, int accumulate, int32_t n,
+                               int32_t f, void* ws, size_t ws_bytes, gte_stream_t stream);
 /* elementwise relu helpers for activation=F.relu without LayerNorm */
 int gte_relu_fwd(const float* z, int64_t ldz, float* y, int64_t ldy, int32_t n, int32_t f, gte_stream_t stream);
 
